@@ -17,6 +17,7 @@ construction (valid -> 1, corrupted -> 0).
   python bench.py --gpus N --steps K --warmup W           our arm (torchrun for N > 1, one rank per GPU)
   python bench.py --workload proof|proof_l10|bn254|sign|rlc ...     one workload as the line itself (ad-hoc runs, profiling)
   python bench.py --impl reference ...                    CPU arm: the oracle port of the reference's path
+  python bench.py ... --dump-outputs DIR                  also write what the timed steps returned (rank 0) as DIR/<name>.npy
 
 Prints ONE JSON line (rank 0)."""
 import argparse
@@ -55,6 +56,7 @@ TOTALS = {"proof": 262144, "proof_l10": 524288, "bn254": 1 << 20, "sign": 1 << 2
 SIG_BYTES = 80
 MSG_BYTES = 32
 PROOF_FIXED = 3 * 48 + 128
+DUMP_VALUES = 1 << 20     # values kept per --dump-outputs array (4 MB of float32; 7 arrays at most in one run)
 
 
 def ptr(a):
@@ -218,6 +220,15 @@ class Env:
         self.n_sm = torch.cuda.get_device_properties(self.local).multi_processor_count
         self.sm_max_mhz = 1965
         self._flush_k = 0
+        self.outputs = {}
+
+    def keep(self, name, a, width=1):
+        """Records what the last timed step returned (rows of `width` values) for --dump-outputs, as float32.  An output
+        of more than DUMP_VALUES values keeps a fixed, seeded sample of its rows (the same rows for the same size)."""
+        a = np.asarray(a).reshape(-1, width)
+        if a.size > DUMP_VALUES:
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), DUMP_VALUES // width, replace=False))]
+        self.outputs[name] = a.astype(np.float32).squeeze(1) if width == 1 else a.astype(np.float32)
 
     def barrier(self):
         self.torch.cuda.synchronize()
@@ -348,12 +359,16 @@ def bench_verify(env, args):
     launches0 = ctx.launch_count()
     sampler = ClockSampler(env.local)
     sampler.start()
-    t_max = env.time_device(step_timed, args.steps)
-    clocks = sampler.stop()
+    try:
+        t_max = env.time_device(step_timed, args.steps)
+    finally:
+        clocks = sampler.stop()       # never leave nvidia-smi running
     env.sm_max_mhz = clocks.get("sm_max_mhz") or env.sm_max_mhz
     launches = (ctx.launch_count() - launches0) // max(args.steps, 1)
-    if not np.array_equal(d_status.cpu().numpy(), expect):
+    got = d_status.cpu().numpy()
+    if not np.array_equal(got, expect):
         raise RuntimeError("status vector mismatch after the timed region")
+    env.keep("verify_status", got)
     value = env.world * n * args.steps / t_max
 
     # ---- end-to-end arm: host (pinned) buffers through the reference-facing call, copies included ----
@@ -447,6 +462,7 @@ def bench_proof(env, n, steps, warmup, seed=77, L=32, R=16):
     launches0 = ctx.launch_count()
     t = env.time_device(step, steps)
     launches = (ctx.launch_count() - launches0) // max(steps, 1)
+    env.keep(f"proof_L{L}_R{R}_status", d_status.cpu().numpy())
     kt = env.kernel_times(ctx, 3)
     kt[0] = h2s_ev[0].elapsed_time(h2s_ev[1])
     lib.bbs_ctx_set_profiling(ctx.handle, 0)
@@ -546,6 +562,7 @@ def bench_bn254(env, n, steps, warmup, seed=5):
     launches0 = ctx.launch_count()
     t = env.time_device(step, steps)
     launches = (ctx.launch_count() - launches0) // max(steps, 1)
+    env.keep("bn254_status", d_status.cpu().numpy())
     kt = env.kernel_times(ctx, 3)
     lib.bbs_ctx_set_profiling(ctx.handle, 0)
     p_sigs, p_sc = env.pin(sigs), env.pin(sc)
@@ -611,14 +628,17 @@ def bench_sign(env, n, steps, warmup, L=10, seed=7):
     launches0 = ctx.launch_count()
     t = env.time_device(step, steps)
     launches = (ctx.launch_count() - launches0) // max(steps, 1)
+    sigs, st = d_sigs.cpu().numpy(), d_st.cpu().numpy()
+    env.keep("sign_signatures", sigs, SIG_BYTES)
+    env.keep("sign_status", st)
     kt = env.kernel_times(ctx, 2)
     kt[0] = h2s_ev[0].elapsed_time(h2s_ev[1])
     lib.bbs_ctx_set_profiling(ctx.handle, 0)
     e2e_step()
     te = env.time_host(e2e_step, steps)
-    if not (p_st.numpy() == 1).all() or not (d_st.cpu().numpy() == 1).all():
+    if not (p_st.numpy() == 1).all() or not (st == 1).all():
         raise RuntimeError("sign status vector is not all ACCEPT")
-    if not np.array_equal(d_sigs.cpu().numpy(), p_sigs.numpy()):
+    if not np.array_equal(sigs, p_sigs.numpy()):
         raise RuntimeError("device-resident and host-buffer signing disagree")
     seed32 = np.frombuffer(os.urandom(32), dtype=np.uint8).copy()
     verdict = np.zeros(1, dtype=np.uint8)
@@ -659,8 +679,8 @@ def bench_rlc(env, n, steps, warmup, L=10, seed=99):
     st = np.zeros(n, dtype=np.uint8)
     sk = np.frombuffer(IRTF_SK.to_bytes(32, "little"), dtype=np.uint8).copy()
     _check(lib, lib.bbs_sign_batch(ctx.handle, ptr(sk), n, ptr(p_msgs), ptr(p_offs), L, ptr(p_sigs), None, ptr(st)))
-    # the seed is drawn after the batch is fixed, by rank 0, and shared
-    seed_t = torch.from_numpy(np.frombuffer(os.urandom(32), dtype=np.uint8).copy()).to(env.dev)
+    # the seed is drawn after the batch is fixed, by rank 0, and shared; seeded, so that runs get the same inputs
+    seed_t = torch.from_numpy(rng.integers(0, 256, size=32, dtype=np.uint8)).to(env.dev)
     if world > 1:
         dist.broadcast(seed_t, 0)
     seed32 = seed_t.cpu().numpy()
@@ -697,6 +717,7 @@ def bench_rlc(env, n, steps, warmup, L=10, seed=99):
     launches0 = ctx.launch_count()
     t = env.time_host(step, steps)
     launches = (ctx.launch_count() - launches0) // max(steps, 1)
+    env.keep("rlc_verdict", verdict)
     # a corrupted batch must be rejected (one flipped bit of e in the last rank's shard)
     if rank == world - 1:
         p_sigs.numpy()[48] ^= 1
@@ -751,6 +772,10 @@ def run_ours(args):
             out = rec
         if out is not None and env.world == 1 and not args.no_cpu and args.workload == "verify":
             out["cpu_baseline"] = cpu_baseline(args, sample=args.cpu_sample)
+        if args.dump_outputs and env.rank == 0:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in env.outputs.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     finally:
         env.close()
     return out
@@ -816,7 +841,13 @@ def main():
     ap.add_argument("--extras", default="proof_l10,proof,bn254,sign,rlc", help="comma list of extra workloads of the default run ('' = none)")
     ap.add_argument("--extra-steps", type=int, default=3, help="timed steps per extra workload (at most --steps)")
     ap.add_argument("--extra-n", type=int, default=None, help="items per GPU for every extra workload (default: BASELINE total / N)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="our arm: write what the last timed step of each workload returned (status vectors, signatures, the "
+                         "RLC verdict) as DIR/<name>.npy in float32, at most 2^20 values each (a fixed seeded sample of "
+                         "larger outputs); the inputs are seeded, so runs with the same arguments compare output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     args.extras = [x for x in args.extras.split(",") if x]
     if args.impl == "reference":
