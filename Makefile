@@ -6,7 +6,7 @@ NVCCFLAGS := $(ARCH) -O3 -std=c++17 -lineinfo -Xcompiler -fPIC $(EXTRA_NVCCFLAGS
 SRC       := bbs_sign_b200/csrc
 BUILD     ?= build/obj
 OUT       ?= bbs_sign_b200/libbbs_b200.so
-GROUPS    := ctx h2s verify pairing sign proof rlc selftest
+GROUPS    := ctx h2s verify pairing sign signitem proof proofitem rlc selftest
 HDRS      := $(wildcard $(SRC)/*.cuh) $(wildcard $(SRC)/*.inc) include/bbs_b200.h
 OBJS      := $(BUILD)/capi.o $(foreach g,$(GROUPS),$(BUILD)/tu_$(g)_bls.o $(BUILD)/tu_$(g)_bn.o)
 

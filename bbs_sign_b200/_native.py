@@ -62,6 +62,19 @@ SYMBOLS = {
     "bbs_proof_gen_batch": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p,
                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p,
                                       C.c_void_p, C.c_void_p]),
+    "bbs_core_verify_batch_hdr": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p,
+                                            C.c_void_p, C.c_void_p]),
+    "bbs_verify_batch_hdr": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p,
+                                       C.c_void_p, C.c_void_p]),
+    "bbs_core_sign_batch_hdr": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_uint32] + [C.c_void_p] * 5),
+    "bbs_sign_batch_hdr": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_uint32] + [C.c_void_p] * 5),
+    "bbs_core_proof_verify_batch_hdr": (C.c_int, [C.c_void_p, C.c_size_t] + [C.c_void_p] * 11),
+    "bbs_proof_verify_batch_hdr": (C.c_int, [C.c_void_p, C.c_size_t] + [C.c_void_p] * 12),
+    "bbs_core_proof_gen_batch_hdr": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_uint32] + [C.c_void_p] * 12),
+    "bbs_proof_gen_batch_hdr": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32]
+                                + [C.c_void_p] * 12),
+    "bbs_core_verify_batch_hdr_dev": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_uint32] + [C.c_void_p] * 4),
+    "bbs_core_proof_verify_batch_hdr_dev": (C.c_int, [C.c_void_p, C.c_size_t] + [C.c_void_p] * 12),
     "bbs_rlc_partial_core": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint64,
                                        C.c_void_p, C.c_void_p]),
     "bbs_rlc_partial": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p,

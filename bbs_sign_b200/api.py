@@ -30,6 +30,7 @@ from . import _native
 ST_REJECT, ST_ACCEPT, ST_ERR_MSG_GEN_LEN, ST_ERR_DISCLOSED_INDEX, ST_ERR_IDX_MSG_LEN, ST_ERR_MALFORMED = range(6)
 ST_ERR_DISCLOSED_LEN, ST_ERR_RANDOM_LEN = 6, 7
 CTX_SMALL_TABLES = 1          # BBS_CTX_SMALL_TABLES (bbs_ctx_create_ex)
+CTX_PER_ITEM_HEADER = 2       # BBS_CTX_PER_ITEM_HEADER (bbs_ctx_create_ex)
 
 
 
@@ -96,12 +97,28 @@ def _pack_ragged(items: Sequence[bytes]):
     return flat, offs
 
 
+def _is_per_item(x) -> bool:
+    """a header / ph argument given as a list / tuple of byte strings, one per item, rather than one shared byte string
+    (bytes, bytearray, memoryview or a numpy uint8 array, as the calls have always accepted)"""
+    return x is not None and not isinstance(x, (bytes, bytearray, memoryview, np.ndarray))
+
+
+def _pack_items(items, n: int, what: str):
+    """one byte string per item -> (flat bytes, n + 1 uint64 offsets) as the *_hdr calls take them"""
+    items = [bytes(x) for x in items]
+    if len(items) != n:
+        raise BbsError(f"one {what} per item required ({len(items)} for {n} items)")
+    return _pack_ragged(items)
+
+
 class BatchContext:
-    """Per (GPU, issuer key, header, generators) state: `bbs_ctx_create` of include/bbs_b200.h."""
+    """Per (GPU, issuer key, header, generators) state: `bbs_ctx_create` of include/bbs_b200.h.  With
+    `per_item_headers=True` (BBS_CTX_PER_ITEM_HEADER) the batch methods also accept `headers=` (one header per item), so
+    one context serves every header of a key and L."""
 
     def __init__(self, suite: Ciphersuite, pk: bytes, header: bytes = b"", n_messages: Optional[int] = None,
                  generators: Optional[bytes] = None, api_id: Optional[bytes] = None, device: int = 0,
-                 lib_path: Optional[str] = None, small_tables: bool = False):
+                 lib_path: Optional[str] = None, small_tables: bool = False, per_item_headers: bool = False):
         self.suite = suite
         self.lib = _native.load(lib_path)
         if generators is None:
@@ -114,13 +131,15 @@ class BatchContext:
         self.L = self.n_generators - 1
         self.api_id = suite.api_id if api_id is None else api_id
         self.header = header
+        self.per_item_headers = per_item_headers
         self.pk = bytes(pk)
         if len(self.pk) != suite.g2_bytes:
             raise BbsError("public key has the wrong length")
         h = C.c_void_p()
         hdr = _buf(header) if header else None
         aid = _buf(self.api_id) if self.api_id else None
-        rc = self.lib.bbs_ctx_create_ex(suite.curve_id, device, CTX_SMALL_TABLES if small_tables else 0, _ptr(_buf(self.pk)),
+        flags = (CTX_SMALL_TABLES if small_tables else 0) | (CTX_PER_ITEM_HEADER if per_item_headers else 0)
+        rc = self.lib.bbs_ctx_create_ex(suite.curve_id, device, flags, _ptr(_buf(self.pk)),
                                         _ptr(_buf(generators)), self.n_generators, _ptr(hdr), len(header), _ptr(aid),
                                         len(self.api_id), C.byref(h))
         if rc != 0:
@@ -165,7 +184,8 @@ class BatchContext:
         return out
 
     # ---- verify.rs ----
-    def core_verify_batch(self, signatures, msg_scalars, n_msgs: int) -> np.ndarray:
+    def core_verify_batch(self, signatures, msg_scalars, n_msgs: int, *, headers: Optional[Sequence[bytes]] = None) -> np.ndarray:
+        """`headers`: one header per signature instead of the context's (needs `per_item_headers=True`)"""
         sigs = _buf(signatures)
         n = sigs.size // self.suite.signature_bytes
         sc = _buf(msg_scalars)
@@ -174,10 +194,17 @@ class BatchContext:
         if sc.size == 0:
             sc = np.zeros(1, dtype=np.uint8)
         st = np.full(n, 255, dtype=np.uint8)
+        if headers is not None:
+            hdr, hoff = _pack_items(headers, n, "header")
+            self._check(self.lib.bbs_core_verify_batch_hdr(self._h, n, _ptr(sigs), _ptr(sc), n_msgs, _ptr(hdr), _ptr(hoff), _ptr(st)),
+                        "bbs_core_verify_batch_hdr")
+            return st
         self._check(self.lib.bbs_core_verify_batch(self._h, n, _ptr(sigs), _ptr(sc), n_msgs, _ptr(st)), "bbs_core_verify_batch")
         return st
 
-    def verify_batch(self, signatures, messages: Sequence[Sequence[bytes]]) -> np.ndarray:
+    def verify_batch(self, signatures, messages: Sequence[Sequence[bytes]], *,
+                     headers: Optional[Sequence[bytes]] = None) -> np.ndarray:
+        """`headers`: one header per signature instead of the context's (needs `per_item_headers=True`)"""
         sigs = _buf(signatures)
         n = sigs.size // self.suite.signature_bytes
         if len(messages) != n:
@@ -187,6 +214,11 @@ class BatchContext:
             raise BbsError("all items of a batch must carry the same number of messages")
         flat, offs = _pack_ragged([m for item in messages for m in item])
         st = np.full(n, 255, dtype=np.uint8)
+        if headers is not None:
+            hdr, hoff = _pack_items(headers, n, "header")
+            self._check(self.lib.bbs_verify_batch_hdr(self._h, n, _ptr(sigs), _ptr(flat), _ptr(offs), n_msgs, _ptr(hdr), _ptr(hoff),
+                                                      _ptr(st)), "bbs_verify_batch_hdr")
+            return st
         self._check(self.lib.bbs_verify_batch(self._h, n, _ptr(sigs), _ptr(flat), _ptr(offs), n_msgs, _ptr(st)), "bbs_verify_batch")
         return st
 
@@ -238,7 +270,9 @@ class BatchContext:
         self._check(self.lib.bbs_ctx_set_rlc_windows(self._h, windows), "bbs_ctx_set_rlc_windows")
 
     # ---- sign.rs ----
-    def core_sign_batch(self, sk_le32: bytes, msg_scalars, n: int, n_msgs: int, want_b: bool = False):
+    def core_sign_batch(self, sk_le32: bytes, msg_scalars, n: int, n_msgs: int, want_b: bool = False, *,
+                        headers: Optional[Sequence[bytes]] = None):
+        """`headers`: one header per signature instead of the context's (needs `per_item_headers=True`)"""
         sc = _buf(msg_scalars)
         if sc.size != n * n_msgs * 32:
             raise BbsError("msg_scalars has the wrong size")
@@ -247,11 +281,18 @@ class BatchContext:
         sigs = np.zeros((n, self.suite.signature_bytes), dtype=np.uint8)
         b = np.zeros((n, self.suite.g1_bytes), dtype=np.uint8) if want_b else None
         st = np.full(n, 255, dtype=np.uint8)
+        if headers is not None:
+            hdr, hoff = _pack_items(headers, n, "header")
+            self._check(self.lib.bbs_core_sign_batch_hdr(self._h, _ptr(_buf(sk_le32)), n, _ptr(sc), n_msgs, _ptr(hdr), _ptr(hoff),
+                                                         _ptr(sigs), _ptr(b), _ptr(st)), "bbs_core_sign_batch_hdr")
+            return sigs, b, st
         self._check(self.lib.bbs_core_sign_batch(self._h, _ptr(_buf(sk_le32)), n, _ptr(sc), n_msgs, _ptr(sigs), _ptr(b), _ptr(st)),
                     "bbs_core_sign_batch")
         return sigs, b, st
 
-    def sign_batch(self, sk_le32: bytes, messages: Sequence[Sequence[bytes]], want_b: bool = False):
+    def sign_batch(self, sk_le32: bytes, messages: Sequence[Sequence[bytes]], want_b: bool = False, *,
+                   headers: Optional[Sequence[bytes]] = None):
+        """`headers`: one header per message list instead of the context's (needs `per_item_headers=True`)"""
         n = len(messages)
         n_msgs = len(messages[0]) if n else 0
         if any(len(m) != n_msgs for m in messages):
@@ -260,15 +301,21 @@ class BatchContext:
         sigs = np.zeros((n, self.suite.signature_bytes), dtype=np.uint8)
         b = np.zeros((n, self.suite.g1_bytes), dtype=np.uint8) if want_b else None
         st = np.full(n, 255, dtype=np.uint8)
+        if headers is not None:
+            hdr, hoff = _pack_items(headers, n, "header")
+            self._check(self.lib.bbs_sign_batch_hdr(self._h, _ptr(_buf(sk_le32)), n, _ptr(flat), _ptr(offs), n_msgs, _ptr(hdr),
+                                                    _ptr(hoff), _ptr(sigs), _ptr(b), _ptr(st)), "bbs_sign_batch_hdr")
+            return sigs, b, st
         self._check(self.lib.bbs_sign_batch(self._h, _ptr(_buf(sk_le32)), n, _ptr(flat), _ptr(offs), n_msgs, _ptr(sigs), _ptr(b), _ptr(st)),
                     "bbs_sign_batch")
         return sigs, b, st
 
     # ---- proof_verify.rs ----
     def proof_gen_batch(self, signatures, messages: Sequence[Sequence[bytes]], disclosed_indexes: Sequence[Sequence[int]],
-                        random_scalars: Sequence[Sequence[bytes]], ph: bytes = b""):
+                        random_scalars: Sequence[Sequence[bytes]], ph=b"", *, headers: Optional[Sequence[bytes]] = None):
         """Batch form of `proof_gen` (proof_gen.rs:78-113) with caller-supplied random scalars (LE32 each, 5 + U per
-        item).  Returns (list of ProofBytes or None, status array)."""
+        item).  `ph` is one presentation header for the batch or one per item; `headers` one header per item instead of the
+        context's (needs `per_item_headers=True`).  Returns (list of ProofBytes or None, status array)."""
         n = len(messages)
         n_msgs = len(messages[0]) if n else 0
         flat, offs = _pack_ragged([m for ms in messages for m in ms])
@@ -287,10 +334,18 @@ class BatchContext:
         fixed = np.zeros(max(n, 1) * self.suite.proof_fixed_bytes, dtype=np.uint8)
         commit = np.zeros(max(int(commit_off[n]), 1) * 32, dtype=np.uint8)
         st = np.full(n, 255, dtype=np.uint8)
-        phb = _buf(ph) if ph else None
-        self._check(self.lib.bbs_proof_gen_batch(self._h, n, _ptr(sigs), _ptr(flat), _ptr(offs), n_msgs, _ptr(idx),
-                                                 _ptr(dis_off), _ptr(rand), _ptr(rand_off), _ptr(commit_off), _ptr(phb),
-                                                 len(ph), _ptr(fixed), _ptr(commit), _ptr(st)), "bbs_proof_gen_batch")
+        if headers is not None or _is_per_item(ph):
+            phs, poff = _pack_items(ph if _is_per_item(ph) else [ph] * n, n, "ph")
+            hdr, hoff = _pack_items(headers, n, "header") if headers is not None else (None, None)
+            self._check(self.lib.bbs_proof_gen_batch_hdr(self._h, n, _ptr(sigs), _ptr(flat), _ptr(offs), n_msgs, _ptr(idx),
+                                                         _ptr(dis_off), _ptr(rand), _ptr(rand_off), _ptr(commit_off), _ptr(hdr),
+                                                         _ptr(hoff), _ptr(phs), _ptr(poff), _ptr(fixed), _ptr(commit), _ptr(st)),
+                        "bbs_proof_gen_batch_hdr")
+        else:
+            phb = _buf(ph) if len(ph) else None
+            self._check(self.lib.bbs_proof_gen_batch(self._h, n, _ptr(sigs), _ptr(flat), _ptr(offs), n_msgs, _ptr(idx),
+                                                     _ptr(dis_off), _ptr(rand), _ptr(rand_off), _ptr(commit_off), _ptr(phb),
+                                                     len(ph), _ptr(fixed), _ptr(commit), _ptr(st)), "bbs_proof_gen_batch")
         pf = self.suite.proof_fixed_bytes
         out = []
         for i in range(n):
@@ -317,8 +372,19 @@ class BatchContext:
             idx = np.zeros(1, np.uint32)
         return fixed, commit, commit_off, idx, dis_off
 
-    def core_proof_verify_batch(self, proofs, ph: bytes, disclosed_scalars: Sequence[Sequence[bytes]],
-                                disclosed_indexes: Sequence[Sequence[int]]) -> np.ndarray:
+    def _per_item_ph_args(self, keep, n, ph, headers):
+        """(headers, hdr_off, phs, ph_off) of the kept items for a *_proof_verify_batch_hdr call; headers None = the context's"""
+        phs = list(ph) if _is_per_item(ph) else [ph] * n
+        if len(phs) != n or (headers is not None and len(headers) != n):
+            raise BbsError("one ph (and header) per proof required")
+        pb, poff = _pack_items([phs[i] for i in keep], len(keep), "ph")
+        hb, hoff = _pack_items([headers[i] for i in keep], len(keep), "header") if headers is not None else (None, None)
+        return hb, hoff, pb, poff
+
+    def core_proof_verify_batch(self, proofs, ph, disclosed_scalars: Sequence[Sequence[bytes]],
+                                disclosed_indexes: Sequence[Sequence[int]], *, headers: Optional[Sequence[bytes]] = None) -> np.ndarray:
+        """`ph`: one presentation header for the batch or one per proof; `headers`: one header per proof instead of the
+        context's (needs `per_item_headers=True`)"""
         n = len(proofs)
         st = np.full(n, 255, dtype=np.uint8)
         # InvalidIndicesAndMessagesLength (proof_verify.rs:144-146) is a property of the host-side lists
@@ -329,11 +395,17 @@ class BatchContext:
             sc = np.frombuffer(b"".join(s for i in keep for s in disclosed_scalars[i]), dtype=np.uint8)
             if sc.size == 0:
                 sc = np.zeros(1, np.uint8)
-            phb = _buf(ph) if ph else None
             out = np.full(len(keep), 255, dtype=np.uint8)
-            self._check(self.lib.bbs_core_proof_verify_batch(self._h, len(keep), _ptr(fixed), _ptr(commit), _ptr(commit_off),
-                                                             _ptr(idx), _ptr(sc), _ptr(dis_off), _ptr(phb), len(ph), _ptr(out)),
-                        "bbs_core_proof_verify_batch")
+            if headers is not None or _is_per_item(ph):
+                hb, hoff, pb, poff = self._per_item_ph_args(keep, n, ph, headers)
+                self._check(self.lib.bbs_core_proof_verify_batch_hdr(self._h, len(keep), _ptr(fixed), _ptr(commit), _ptr(commit_off),
+                                                                     _ptr(idx), _ptr(sc), _ptr(dis_off), _ptr(hb), _ptr(hoff),
+                                                                     _ptr(pb), _ptr(poff), _ptr(out)), "bbs_core_proof_verify_batch_hdr")
+            else:
+                phb = _buf(ph) if len(ph) else None
+                self._check(self.lib.bbs_core_proof_verify_batch(self._h, len(keep), _ptr(fixed), _ptr(commit), _ptr(commit_off),
+                                                                 _ptr(idx), _ptr(sc), _ptr(dis_off), _ptr(phb), len(ph), _ptr(out)),
+                            "bbs_core_proof_verify_batch")
             st[keep] = out
         for i in range(n):
             if bad[i]:
@@ -345,8 +417,10 @@ class BatchContext:
         L = len(proof.commitments) // 32 + len(idxs)
         return ST_ERR_DISCLOSED_INDEX if any(i >= L for i in idxs) else ST_ERR_IDX_MSG_LEN
 
-    def proof_verify_batch(self, proofs, ph: bytes, disclosed_messages: Sequence[Sequence[bytes]],
-                           disclosed_indexes: Sequence[Sequence[int]]) -> np.ndarray:
+    def proof_verify_batch(self, proofs, ph, disclosed_messages: Sequence[Sequence[bytes]],
+                           disclosed_indexes: Sequence[Sequence[int]], *, headers: Optional[Sequence[bytes]] = None) -> np.ndarray:
+        """`ph`: one presentation header for the batch or one per proof; `headers`: one header per proof instead of the
+        context's (needs `per_item_headers=True`)"""
         n = len(proofs)
         st = np.full(n, 255, dtype=np.uint8)
         bad = [len(disclosed_messages[i]) != len(disclosed_indexes[i]) for i in range(n)]
@@ -354,11 +428,17 @@ class BatchContext:
         if keep:
             fixed, commit, commit_off, idx, dis_off = self._pack_proofs([proofs[i] for i in keep], [disclosed_indexes[i] for i in keep])
             flat, moffs = _pack_ragged([m for i in keep for m in disclosed_messages[i]])
-            phb = _buf(ph) if ph else None
             out = np.full(len(keep), 255, dtype=np.uint8)
-            self._check(self.lib.bbs_proof_verify_batch(self._h, len(keep), _ptr(fixed), _ptr(commit), _ptr(commit_off), _ptr(idx),
-                                                        _ptr(flat), _ptr(moffs), _ptr(dis_off), _ptr(phb), len(ph), _ptr(out)),
-                        "bbs_proof_verify_batch")
+            if headers is not None or _is_per_item(ph):
+                hb, hoff, pb, poff = self._per_item_ph_args(keep, n, ph, headers)
+                self._check(self.lib.bbs_proof_verify_batch_hdr(self._h, len(keep), _ptr(fixed), _ptr(commit), _ptr(commit_off),
+                                                                _ptr(idx), _ptr(flat), _ptr(moffs), _ptr(dis_off), _ptr(hb), _ptr(hoff),
+                                                                _ptr(pb), _ptr(poff), _ptr(out)), "bbs_proof_verify_batch_hdr")
+            else:
+                phb = _buf(ph) if len(ph) else None
+                self._check(self.lib.bbs_proof_verify_batch(self._h, len(keep), _ptr(fixed), _ptr(commit), _ptr(commit_off), _ptr(idx),
+                                                            _ptr(flat), _ptr(moffs), _ptr(dis_off), _ptr(phb), len(ph), _ptr(out)),
+                            "bbs_proof_verify_batch")
             st[keep] = out
         for i in range(n):
             if bad[i]:
@@ -463,7 +543,7 @@ class IssuerSet:
                                                                                 [disclosed_indexes[i] for i in keep])
             flat, moffs = _pack_ragged([m for i in keep for m in disclosed_messages[i]])
             iss = np.ascontiguousarray(np.asarray([item_issuer[i] for i in keep], dtype=np.uint32))
-            phb = _buf(ph) if ph else None
+            phb = _buf(ph) if len(ph) else None
             out = np.full(len(keep), 255, dtype=np.uint8)
             rc = self.lib.bbs_proof_verify_batch_multi(self._h, len(keep), _ptr(iss), _ptr(fixed), _ptr(commit), _ptr(commit_off),
                                                        _ptr(idx), _ptr(flat), _ptr(moffs), _ptr(dis_off), _ptr(phb), len(ph), _ptr(out))
@@ -488,7 +568,7 @@ class IssuerSet:
         if sc.size == 0:
             sc = np.zeros(1, np.uint8)
         iss = np.ascontiguousarray(np.asarray(item_issuer, dtype=np.uint32))
-        phb = _buf(ph) if ph else None
+        phb = _buf(ph) if len(ph) else None
         st = np.full(n, 255, dtype=np.uint8)
         rc = self.lib.bbs_core_proof_verify_batch_multi(self._h, n, _ptr(iss), _ptr(fixed), _ptr(commit), _ptr(commit_off), _ptr(idx),
                                                         _ptr(sc), _ptr(dis_off), _ptr(phb), len(ph), _ptr(st))
@@ -524,30 +604,39 @@ class PublicKey:
 
     def __init__(self, suite: Ciphersuite, pk: bytes, lib_path: Optional[str] = None):
         self.suite, self.pk, self.lib_path = suite, bytes(pk), lib_path
-        self._ctx = {}         # (header, L, device) -> BatchContext, least recently used first
+        self._ctx = {}         # (header, L, device) -> BatchContext, least recently used first; header None = per-item headers
 
-    def context(self, header: bytes, n_messages: int, device: int = 0) -> BatchContext:
+    def context(self, header: Optional[bytes], n_messages: int, device: int = 0) -> BatchContext:
+        """the context for `header`, or (header None) the one context serving every header of (L, device)"""
         key = (header, n_messages, device)
         ctx = self._ctx.pop(key, None)
         if ctx is None:
             while len(self._ctx) >= self.MAX_CONTEXTS:
                 self._ctx.pop(next(iter(self._ctx))).close()
-            ctx = BatchContext(self.suite, self.pk, header, n_messages, device=device, lib_path=self.lib_path)
+            ctx = BatchContext(self.suite, self.pk, header or b"", n_messages, device=device, lib_path=self.lib_path,
+                               per_item_headers=header is None)
         self._ctx[key] = ctx
         return ctx
 
-    def verify_batch(self, signatures, header: bytes, messages: Sequence[Sequence[bytes]], device: int = 0) -> np.ndarray:
-        """verify.rs:18-50 for a batch sharing `header`; messages[i] is the message list of signature i."""
+    def verify_batch(self, signatures, header, messages: Sequence[Sequence[bytes]], device: int = 0) -> np.ndarray:
+        """verify.rs:18-50; messages[i] is the message list of signature i, `header` one header for the batch or one per
+        signature."""
         n_msgs = len(messages[0]) if len(messages) else 0
+        if _is_per_item(header):
+            return self.context(None, n_msgs, device).verify_batch(signatures, messages, headers=header)
         return self.context(header, n_msgs, device).verify_batch(signatures, messages)
 
-    def proof_verify_batch(self, proofs: Sequence[ProofBytes], header: bytes, ph: bytes,
+    def proof_verify_batch(self, proofs: Sequence[ProofBytes], header, ph,
                            disclosed_messages: Sequence[Sequence[bytes]], disclosed_indexes: Sequence[Sequence[int]],
                            device: int = 0) -> np.ndarray:
-        """proof_verify.rs:19-61 for a batch sharing header / ph and the same total message count."""
+        """proof_verify.rs:19-61 for a batch with the same total message count; `header` and `ph` are each one byte string
+        for the batch or one per proof."""
         if not proofs:
             return np.zeros(0, dtype=np.uint8)
         L = len(proofs[0].commitments) // 32 + len(disclosed_indexes[0])
+        if _is_per_item(header):
+            return self.context(None, L, device).proof_verify_batch(proofs, ph, disclosed_messages, disclosed_indexes,
+                                                                    headers=header)
         return self.context(header, L, device).proof_verify_batch(proofs, ph, disclosed_messages, disclosed_indexes)
 
 
@@ -558,7 +647,9 @@ class SecretKey:
     def __init__(self, suite: Ciphersuite, sk_le32: bytes, pk: bytes):
         self.suite, self.sk, self.pk = suite, bytes(sk_le32), PublicKey(suite, pk)
 
-    def sign_batch(self, messages: Sequence[Sequence[bytes]], header: bytes, want_b: bool = False, device: int = 0):
-        """sign.rs:32-60 for a batch sharing `header`."""
+    def sign_batch(self, messages: Sequence[Sequence[bytes]], header, want_b: bool = False, device: int = 0):
+        """sign.rs:32-60; `header` is one header for the batch or one per message list."""
         n_msgs = len(messages[0]) if len(messages) else 0
+        if _is_per_item(header):
+            return self.pk.context(None, n_msgs, device).sign_batch(self.sk, messages, want_b, headers=header)
         return self.pk.context(header, n_msgs, device).sign_batch(self.sk, messages, want_b)

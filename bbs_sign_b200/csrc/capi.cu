@@ -5,6 +5,7 @@
 
 #include <algorithm>
 #include <new>
+#include <string>
 #include <vector>
 
 using namespace bbs;
@@ -20,8 +21,13 @@ struct ProfEvents {
 #ifndef BBS_HOSTSIM
     cudaEvent_t ev[MAX] = {};
     int used = 0;
+    // the per-item domain kernel of a bbs_*_hdr call is timed by its own pair of events and reported in slot xslot, after
+    // the call's other slots; every call's chain of marks starts at slot 0 or 1, which forgets the previous call's xslot
+    cudaEvent_t xev[2] = {};
+    int xslot = -1;
     int mark(int slot, rt_stream_t s) {
         if (slot >= MAX) return 0;
+        if (slot <= 1) xslot = -1;
         if (!ev[slot]) RT_CHECK(cudaEventCreate(&ev[slot]));
         RT_CHECK(cudaEventRecord(ev[slot], s));
         used = slot + 1;
@@ -34,11 +40,25 @@ struct ProfEvents {
             RT_CHECK(cudaEventSynchronize(ev[i + 1]));
             RT_CHECK(cudaEventElapsedTime(&ms[i], ev[i], ev[i + 1]));
         }
+        if (xslot >= 0 && xslot < n && xev[0] && xev[1]) {
+            RT_CHECK(cudaEventSynchronize(xev[1]));
+            RT_CHECK(cudaEventElapsedTime(&ms[xslot], xev[0], xev[1]));
+        }
         return 0;
     }
-    void release() { for (auto& e : ev) if (e) { cudaEventDestroy(e); e = nullptr; } }
+    int mark_extra(int k, rt_stream_t s) {
+        if (!xev[k]) RT_CHECK(cudaEventCreate(&xev[k]));
+        RT_CHECK(cudaEventRecord(xev[k], s));
+        return 0;
+    }
+    void release() {
+        for (auto& e : ev) if (e) { cudaEventDestroy(e); e = nullptr; }
+        for (auto& e : xev) if (e) { cudaEventDestroy(e); e = nullptr; }
+    }
 #else
+    int xslot = -1;
     int mark(int, rt_stream_t) { return 0; }
+    int mark_extra(int, rt_stream_t) { return 0; }
     int read(float* ms, int n) { for (int i = 0; i < n; i++) ms[i] = 0.f; return 0; }
     void release() {}
 #endif
@@ -59,9 +79,10 @@ struct Ctx {
     bool profile = false;            // bbs_ctx_set_profiling: CUDA events around each kernel of a batch call
     ProfEvents prof;
     DevBuf pk_comp, gens_comp, api_id, header, dst_h2s, dst_map;
-    DevBuf gens, W, K, domain, tab, wbase, lines, lines_coop, misc;
+    DevBuf gens, W, K, domain, tab, wbase, lines, lines_coop, misc, prefix;
     bool coop = false;               // cooperative pairing kernel usable (no degenerate line)
     bool force_per_thread = false;   // bbs_ctx_use_per_thread_pairing: the fallback kernel on request (tests)
+    bool per_item_header = false;    // BBS_CTX_PER_ITEM_HEADER: Q1 table in slot L + 1 and the domain prefix state in `prefix`
     uint32_t rlc_windows = 0;        // bbs_ctx_set_rlc_windows: digits per 128-bit value of the bucket MSM (0 = cost model)
     CtxView view{};
     // grow-only scratch for the batch calls
@@ -71,11 +92,12 @@ struct Ctx {
     DevBuf s_gscr, s_rlc_pt, s_rlc_sc, s_rlc_parts, s_rlc_bad, s_msm_pts, s_msm_kv, s_msm_idx, s_msm_entries, s_msm_buckets;
     DevBuf s_sigs, s_scalars, s_msgs, s_offsets, s_pair, s_flags, s_status, s_out, s_out2;
     DevBuf s_commit, s_commit_off, s_dis_idx, s_dis_scalars, s_dis_off, s_ph, s_dis_msgs, s_dis_msg_off;
+    DevBuf s_hdr, s_hdr_off, s_ph_off, s_ik, s_idom, s_ifl;     // per-item headers / phs and the ItemKeyView arrays
     template <class Fn> void each_buffer(Fn f) {
         DevBuf* all[] = {&pk_comp, &gens_comp, &api_id, &header, &dst_h2s, &dst_map, &gens, &W, &K, &domain, &tab, &wbase,
                          &lines, &lines_coop, &s_rand, &s_rand_off, &s_sk, &s_g1v, &s_g1f, &s_g1st, &s_g1t, &s_gscr, &s_rlc_pt, &s_rlc_sc, &s_rlc_parts, &s_rlc_bad, &s_msm_pts, &s_msm_kv, &s_msm_idx, &s_msm_entries, &s_msm_buckets, &misc, &s_sigs, &s_scalars, &s_msgs, &s_offsets, &s_pair, &s_flags, &s_status, &s_out,
                          &s_out2, &s_commit, &s_commit_off, &s_dis_idx, &s_dis_scalars, &s_dis_off, &s_ph, &s_dis_msgs,
-                         &s_dis_msg_off};
+                         &s_dis_msg_off, &prefix, &s_hdr, &s_hdr_off, &s_ph_off, &s_ik, &s_idom, &s_ifl};
         for (DevBuf* b : all) f(b);
     }
     void release_all() { each_buffer([](DevBuf* b) { b->release(); }); }
@@ -104,6 +126,20 @@ bool counts_fit(size_t n, size_t per_item) {
     if (n > 0xffffffffull) return false;
     return per_item == 0 || n <= 0xffffffffull / per_item;
 }
+// Per-item byte strings (headers, phs): n + 1 offsets that never decrease, each item shorter than 2^28 bytes so that every
+// hash input built from one stays below the 2^29 bytes that Sha256 counts.
+constexpr uint64_t MAX_ITEM_BYTES = 1ull << 28;
+int check_items(size_t n, const uint8_t* bytes, const uint64_t* off, const char* what) {
+    for (size_t i = 0; i < n; i++) {
+        if (off[i + 1] < off[i]) { rt_set_error("bad argument", (std::string(what) + " offsets decrease").c_str()); return BBS_E_ARG; }
+        if (off[i + 1] - off[i] >= MAX_ITEM_BYTES) {
+            rt_set_error("bad argument", (std::string(what) + " longer than 2^28 bytes").c_str());
+            return BBS_E_ARG;
+        }
+    }
+    if (off[n] != off[0] && !bytes) return arg_error("null per-item byte strings");
+    return BBS_OK;
+}
 #define CHECK_COUNTS(n, per_item) do { if (!counts_fit((n), (per_item))) return arg_error("batch too large: n and n * n_msgs must fit in 32 bits"); } while (0)
 
 template <class C>
@@ -115,6 +151,8 @@ struct Impl {
                       size_t header_len, const uint8_t* api_id, size_t api_id_len, uint32_t flags) {
         const TabGeom G((flags & BBS_CTX_SMALL_TABLES) ? (uint32_t)TAB_BITS_SMALL : (uint32_t)BBS_TAB_BITS_GLV);
         const uint32_t L = n_gens - 1;
+        const bool per_item = (flags & BBS_CTX_PER_ITEM_HEADER) != 0;
+        const uint32_t n_tabs = per_item ? L + 2 : L + 1;        // K, H_1..H_L (, Q1)
         c->L = L;
         c->api_id_len = api_id_len; c->header_len = header_len;
         rt_stream_t s = c->stream;
@@ -135,7 +173,8 @@ struct Impl {
         TRY(c->K.reserve(2 * C::Fp::N * 4));
         TRY(c->domain.reserve(32));
         TRY(c->misc.reserve((n_gens + 2) * 4));
-        const size_t tab_entries = (size_t)(L + 1) * G.windows * G.entries;
+        if (per_item) TRY(c->prefix.reserve(SHA_STATE_WORDS * 4));
+        const size_t tab_entries = (size_t)n_tabs * G.windows * G.entries;
         TRY(c->tab.reserve(tab_entries * 2 * C::Fp::N * 4));
         const int n_lines = ate_line_count<C>();
         TRY(c->lines.reserve((size_t)n_lines * 2 * 4 * C::Fp::N * 4));
@@ -163,16 +202,17 @@ struct Impl {
         CtxDomainArgs dom{(const uint8_t*)c->pk_comp.p, (const uint8_t*)c->gens_comp.p, L,
                           (const uint8_t*)c->api_id.p, (uint32_t)api_id_len, (const uint8_t*)c->header.p,
                           (uint32_t)header_len, (const uint8_t*)c->dst_h2s.p, (uint32_t)dsth.size(),
-                          (const uint32_t*)c->gens.p, (uint32_t*)c->domain.p, (uint32_t*)c->K.p, d_kinf};
+                          (const uint32_t*)c->gens.p, (uint32_t*)c->domain.p, (uint32_t*)c->K.p, d_kinf,
+                          per_item ? (uint32_t*)c->prefix.p : nullptr};
         TRY((launch_ctx_domain<C>(dom, 1, s)));
         uint32_t k_inf = 0;
         TRY(rt_d2h(&k_inf, d_kinf, 4, s));
         TRY(rt_sync(s));
         // 3. window tables, 4. line tables
-        TRY(c->wbase.reserve((size_t)(L + 1) * G.windows * 2 * C::Fp::N * 4));
+        TRY(c->wbase.reserve((size_t)n_tabs * G.windows * 2 * C::Fp::N * 4));
         CtxTableArgs ta{(const uint32_t*)c->K.p, (const uint32_t*)c->gens.p, (uint32_t*)c->tab.p, (uint32_t*)c->wbase.p,
-                        (uint32_t)G.bits};
-        TRY((launch_ctx_table<C>(ta, L + 1, s)));
+                        (uint32_t)G.bits, per_item ? L + 1 : 0u};
+        TRY((launch_ctx_table<C>(ta, n_tabs, s)));
         CtxLinesArgs la{(const uint32_t*)c->W.p, w_inf, (uint32_t*)c->lines.p};
         TRY((launch_ctx_lines<C>(la, 2, s)));
         TRY(rt_sync(s));
@@ -200,6 +240,7 @@ struct Impl {
         v.gens = (const uint32_t*)c->gens.p; v.W = (const uint32_t*)c->W.p; v.K = (const uint32_t*)c->K.p;
         v.domain = (const uint32_t*)c->domain.p; v.tab = (const uint32_t*)c->tab.p;
         v.lines = (const uint32_t*)c->lines.p;
+        c->per_item_header = per_item;
 #ifndef BBS_HOSTSIM
         c->split_max = (size_t)-1;       // the two-task G1 path is faster at every batch size measured (DESIGN 4.2)
 #endif
@@ -237,7 +278,7 @@ struct Impl {
     // G1 half of core_verify for items [first, first + n) of a batch whose pair records / flags / statuses are indexed by the
     // batch (scratch of the task split is per launch: reserve it for the largest launch BEFORE a chunked sequence starts)
     static int verify_g1_dev(Ctx* c, size_t n, size_t first, const uint8_t* d_sigs, const uint8_t* d_scalars, uint32_t n_msgs,
-                             uint8_t* d_status, rt_stream_t s, const IssuerSet* S = nullptr) {
+                             uint8_t* d_status, rt_stream_t s, const IssuerSet* S = nullptr, const ItemKeyView* item = nullptr) {
         VerifyG1Args a{c->view, d_sigs + first * SIG, d_scalars + first * n_msgs * 32, n_msgs,
                        (uint32_t*)c->s_pair.p + first * 6 * C::Fp::N, (uint32_t*)c->s_flags.p + first, d_status + first};
         if (n <= c->split_max) {
@@ -251,20 +292,93 @@ struct Impl {
             a.iss = IssuerSetView{(const uint32_t*)S->K.p, (const uint32_t*)S->flags.p, (const uint32_t*)S->lines.p,
                                   S->line_stride, (uint32_t)S->n_issuers, (const uint32_t*)S->domains.p};
         }
+        if (item) a.item = ItemKeyView{item->K + first * 2 * C::Fp::N, item->domains + first * 8, item->flags + first};
         TRY((launch_verify_g1<C>(a, (uint32_t)n, s)));
         c->launches += n ? (a.part_v ? 2 : 1) : 0;
         return BBS_OK;
     }
     static int core_verify_dev(Ctx* c, size_t n, const uint8_t* d_sigs, const uint8_t* d_scalars, uint32_t n_msgs,
-                               uint8_t* d_status, rt_stream_t s, const IssuerSet* S = nullptr) {
+                               uint8_t* d_status, rt_stream_t s, const IssuerSet* S = nullptr, const ItemKeyView* item = nullptr) {
         TRY(c->s_pair.reserve(n * 6 * C::Fp::N * 4));
         TRY(c->s_flags.reserve(n * 4));
         PROF(c, 1, s);
-        TRY(verify_g1_dev(c, n, 0, d_sigs, d_scalars, n_msgs, d_status, s, S));
+        TRY(verify_g1_dev(c, n, 0, d_sigs, d_scalars, n_msgs, d_status, s, S, item));
         PROF(c, 2, s);
         TRY(pairing_dev(c, n, d_status, s, S));
         PROF(c, 3, s);
+        if (item) c->prof.xslot = 3;
         return BBS_OK;
+    }
+
+    // ---- per-item headers (bbs_*_hdr) ----------------------------------------------------------------------
+    // domain_i, K_i and the K_i-is-identity flags of items [0, n) into the call's scratch; `item` is what the consumers read
+    static int item_keys_dev(Ctx* c, size_t n, const uint8_t* d_headers, const uint64_t* d_hdr_off, ItemKeyView& item,
+                             rt_stream_t s) {
+        TRY(c->s_ik.reserve(n * 2 * C::Fp::N * 4));
+        TRY(c->s_idom.reserve(n * 32));
+        TRY(c->s_ifl.reserve(n * 4));
+        ItemDomainArgs a{c->view, (const uint32_t*)c->prefix.p, d_headers, d_hdr_off, (uint32_t*)c->s_idom.p,
+                         (uint32_t*)c->s_ik.p, (uint32_t*)c->s_ifl.p};
+        if (c->profile) TRY(c->prof.mark_extra(0, s));
+        TRY((launch_item_domain<C>(a, (uint32_t)n, s)));
+        if (c->profile) TRY(c->prof.mark_extra(1, s));
+        c->launches += n ? 1 : 0;
+        item = ItemKeyView{(const uint32_t*)c->s_ik.p, (const uint32_t*)c->s_idom.p, (const uint32_t*)c->s_ifl.p};
+        return BBS_OK;
+    }
+    // host headers staged, then item_keys_dev
+    static int item_keys(Ctx* c, size_t n, const uint8_t* headers, const uint64_t* hdr_off, ItemKeyView& item) {
+        TRY(stage(c->s_hdr, headers, hdr_off[n], c->stream));
+        TRY(stage(c->s_hdr_off, hdr_off, (n + 1) * 8, c->stream));
+        return item_keys_dev(c, n, (const uint8_t*)c->s_hdr.p, (const uint64_t*)c->s_hdr_off.p, item, c->stream);
+    }
+    // verify / core_verify with a header per item (msgs == nullptr: `scalars` holds the message scalars).  Always one shot:
+    // batches large enough for verify_chunked are not split into chunks here.
+    static int verify_hdr(Ctx* c, size_t n, const uint8_t* sigs, const uint8_t* scalars, const uint8_t* msgs, const uint64_t* off,
+                          uint32_t n_msgs, const uint8_t* headers, const uint64_t* hdr_off, uint8_t* status) {
+        rt_stream_t s = c->stream;
+        const size_t count = n * n_msgs;
+        ItemKeyView item{};
+        TRY(item_keys(c, n, headers, hdr_off, item));
+        TRY(stage(c->s_sigs, sigs, n * SIG, s));
+        TRY(c->s_status.reserve(n));
+        if (off) {
+            TRY(stage(c->s_msgs, msgs, off[count], s));
+            TRY(stage(c->s_offsets, off, (count + 1) * 8, s));
+            TRY(c->s_scalars.reserve(count * 32));
+            PROF(c, 0, s);
+            TRY(h2s_dev(c, count, (const uint8_t*)c->s_msgs.p, (const uint64_t*)c->s_offsets.p, (uint8_t*)c->s_scalars.p, s));
+        } else {
+            TRY(stage(c->s_scalars, scalars, count * 32, s));
+        }
+        TRY(core_verify_dev(c, n, (const uint8_t*)c->s_sigs.p, (const uint8_t*)c->s_scalars.p, n_msgs, (uint8_t*)c->s_status.p,
+                            s, nullptr, &item));
+        return finish_status(c, n, status);
+    }
+    static int core_verify_hdr_dev(Ctx* c, size_t n, const uint8_t* d_sigs, const uint8_t* d_scalars, uint32_t n_msgs,
+                                   const uint8_t* d_headers, const uint64_t* d_hdr_off, uint8_t* d_status, rt_stream_t s) {
+        ItemKeyView item{};
+        TRY(item_keys_dev(c, n, d_headers, d_hdr_off, item, s));
+        return core_verify_dev(c, n, d_sigs, d_scalars, n_msgs, d_status, s, nullptr, &item);
+    }
+    // sign / core_sign with a header per item (one shot, like verify_hdr)
+    static int sign_hdr(Ctx* c, const uint8_t* sk, size_t n, const uint8_t* scalars, const uint8_t* msgs, const uint64_t* off,
+                        uint32_t n_msgs, const uint8_t* headers, const uint64_t* hdr_off, uint8_t* sigs_out, uint8_t* b_out,
+                        uint8_t* status) {
+        rt_stream_t s = c->stream;
+        const size_t count = n * n_msgs;
+        ItemKeyView item{};
+        TRY(item_keys(c, n, headers, hdr_off, item));
+        if (off) {
+            TRY(stage(c->s_msgs, msgs, off[count], s));
+            TRY(stage(c->s_offsets, off, (count + 1) * 8, s));
+            TRY(c->s_scalars.reserve(count * 32));
+            PROF(c, 0, s);
+            TRY(h2s_dev(c, count, (const uint8_t*)c->s_msgs.p, (const uint64_t*)c->s_offsets.p, (uint8_t*)c->s_scalars.p, s));
+        } else {
+            TRY(stage(c->s_scalars, scalars, count * 32, s));
+        }
+        return sign_common(c, sk, n, n_msgs, sigs_out, b_out, status, &item);
     }
 #ifndef BBS_HOSTSIM
     // Host buffers of a LARGE verify batch (>= 2 * VERIFY_CHUNK items) in up to 8 chunks of doubling size: all uploads are
@@ -423,9 +537,10 @@ struct Impl {
     }
 
     static int core_sign_dev(Ctx* c, const uint8_t* sk, size_t n, const uint8_t* d_scalars, uint32_t n_msgs,
-                             uint8_t* d_sigs, uint8_t* d_b, uint8_t* d_status, rt_stream_t s) {
+                             uint8_t* d_sigs, uint8_t* d_b, uint8_t* d_status, rt_stream_t s, const ItemKeyView* item = nullptr) {
         SignArgs a{};
         a.ctx = c->view;
+        if (item) a.item = *item;
         uint32_t skl[8];
         limbs_from_le<8>(skl, sk);
         const bool canon = fe_is_canonical<typename C::Fr>(skl);
@@ -443,13 +558,15 @@ struct Impl {
         TRY(rc);
         TRY(rc2);
         PROF(c, 2, s);
+        if (item) c->prof.xslot = 2;
         return BBS_OK;
     }
 
     static int core_proof_verify_dev(Ctx* c, size_t n, const uint8_t* d_proofs, const uint8_t* d_commit,
                                      const uint64_t* d_commit_off, const uint32_t* d_idx, const uint8_t* d_dis_scalars,
                                      const uint64_t* d_dis_off, const uint8_t* d_ph, size_t ph_len, uint8_t* d_status,
-                                     rt_stream_t s, const IssuerSet* S = nullptr) {
+                                     rt_stream_t s, const IssuerSet* S = nullptr, const ItemKeyView* item = nullptr,
+                                     const uint64_t* d_ph_off = nullptr) {
         TRY(c->s_pair.reserve(n * 6 * C::Fp::N * 4));
         TRY(c->s_flags.reserve(n * 4));
         ProofG1Args a{c->view, d_proofs, d_commit, d_commit_off, d_idx, d_dis_scalars, d_dis_off, d_ph,
@@ -459,7 +576,9 @@ struct Impl {
             a.iss = IssuerSetView{(const uint32_t*)S->K.p, (const uint32_t*)S->flags.p, (const uint32_t*)S->lines.p,
                                   S->line_stride, (uint32_t)S->n_issuers, (const uint32_t*)S->domains.p};
         }
-        if (S || n <= c->split_max) {
+        a.ph_off = d_ph_off;
+        if (item) a.item = *item;         // per-item headers, like issuer sets, take the task split at every size
+        if (S || item || n <= c->split_max) {
             TRY(c->s_g1t.reserve(n * 3 * C::Fp::N * 4));
             TRY(c->s_g1v.reserve(n * 3 * C::Fp::N * 4));
             TRY(c->s_g1f.reserve(n * 3 * C::Fp::N * 4));
@@ -473,15 +592,33 @@ struct Impl {
         PROF(c, 2, s);
         TRY(pairing_dev(c, n, d_status, s, S));
         PROF(c, 3, s);
+        if (item) c->prof.xslot = 3;
         return BBS_OK;
+    }
+    // bbs_core_proof_verify_batch_hdr_dev: d_hdr_off == nullptr = the context's header
+    static int core_proof_verify_hdr_dev(Ctx* c, size_t n, const uint8_t* d_proofs, const uint8_t* d_commit,
+                                         const uint64_t* d_commit_off, const uint32_t* d_idx, const uint8_t* d_dis_scalars,
+                                         const uint64_t* d_dis_off, const uint8_t* d_headers, const uint64_t* d_hdr_off,
+                                         const uint8_t* d_phs, const uint64_t* d_ph_off, uint8_t* d_status, rt_stream_t s) {
+        ItemKeyView item{};
+        if (d_hdr_off) TRY(item_keys_dev(c, n, d_headers, d_hdr_off, item, s));
+        return core_proof_verify_dev(c, n, d_proofs, d_commit, d_commit_off, d_idx, d_dis_scalars, d_dis_off, d_phs, 0, d_status,
+                                     s, nullptr, d_hdr_off ? &item : nullptr, d_ph_off);
     }
 
     // ---- core_proof_gen (proof_gen.rs:116-365) -----------------------------------------------------------
     static int proof_gen_common(Ctx* c, size_t n, const uint8_t* sigs, uint32_t n_msgs, const uint32_t* idx,
                                 const uint64_t* dis_off, const uint8_t* rand, const uint64_t* rand_off,
                                 const uint64_t* commit_off, const uint8_t* ph, size_t ph_len, uint8_t* proofs_out,
-                                uint8_t* commitments_out, uint8_t* status) {
+                                uint8_t* commitments_out, uint8_t* status, const uint64_t* ph_off = nullptr,
+                                const uint8_t* headers = nullptr, const uint64_t* hdr_off = nullptr) {
         rt_stream_t s = c->stream;
+        ItemKeyView item{};
+        if (hdr_off) TRY(item_keys(c, n, headers, hdr_off, item));
+        if (ph_off) {
+            ph_len = ph_off[n];
+            TRY(stage(c->s_ph_off, ph_off, (n + 1) * 8, s));
+        }
         TRY(stage(c->s_sigs, sigs, n * SIG, s));
         TRY(stage(c->s_dis_idx, idx, dis_off[n] * 4, s));
         TRY(stage(c->s_dis_off, dis_off, (n + 1) * 8, s));
@@ -498,24 +635,29 @@ struct Impl {
                        (const uint32_t*)c->s_dis_idx.p, (const uint64_t*)c->s_dis_off.p, (const uint8_t*)c->s_rand.p,
                        (const uint64_t*)c->s_rand_off.p, (const uint64_t*)c->s_commit_off.p, (const uint8_t*)c->s_ph.p,
                        (uint32_t)ph_len, (uint8_t*)c->s_out.p, (uint8_t*)c->s_commit.p, (uint8_t*)c->s_status.p};
+        a.item = item;
+        a.ph_off = ph_off ? (const uint64_t*)c->s_ph_off.p : nullptr;
         TRY((launch_proof_gen<C>(a, (uint32_t)n, s)));
         c->launches += n ? 1 : 0;
         TRY(rt_d2h(proofs_out, c->s_out.p, n * PROOF, s));
         TRY(rt_d2h(commitments_out, c->s_commit.p, commit_off[n] * 32, s));
         return finish_status(c, n, status);
     }
+    // ph_off != nullptr: per-item phs in `ph`; hdr_off != nullptr: per-item headers (bbs_*proof_gen_batch_hdr)
     static int core_proof_gen(Ctx* c, size_t n, const uint8_t* sigs, const uint8_t* scalars, uint32_t n_msgs,
                               const uint32_t* idx, const uint64_t* dis_off, const uint8_t* rand, const uint64_t* rand_off,
                               const uint64_t* commit_off, const uint8_t* ph, size_t ph_len, uint8_t* proofs_out,
-                              uint8_t* commitments_out, uint8_t* status) {
+                              uint8_t* commitments_out, uint8_t* status, const uint64_t* ph_off = nullptr,
+                              const uint8_t* headers = nullptr, const uint64_t* hdr_off = nullptr) {
         TRY(stage(c->s_scalars, scalars, n * n_msgs * 32, c->stream));
         return proof_gen_common(c, n, sigs, n_msgs, idx, dis_off, rand, rand_off, commit_off, ph, ph_len, proofs_out,
-                                commitments_out, status);
+                                commitments_out, status, ph_off, headers, hdr_off);
     }
     static int proof_gen(Ctx* c, size_t n, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* off, uint32_t n_msgs,
                          const uint32_t* idx, const uint64_t* dis_off, const uint8_t* rand, const uint64_t* rand_off,
                          const uint64_t* commit_off, const uint8_t* ph, size_t ph_len, uint8_t* proofs_out,
-                         uint8_t* commitments_out, uint8_t* status) {
+                         uint8_t* commitments_out, uint8_t* status, const uint64_t* ph_off = nullptr,
+                         const uint8_t* headers = nullptr, const uint64_t* hdr_off = nullptr) {
         rt_stream_t s = c->stream;
         const size_t count = n * n_msgs;
         TRY(stage(c->s_msgs, msgs, off[count], s));
@@ -523,7 +665,7 @@ struct Impl {
         TRY(c->s_scalars.reserve(count * 32));
         TRY(h2s_dev(c, count, (const uint8_t*)c->s_msgs.p, (const uint64_t*)c->s_offsets.p, (uint8_t*)c->s_scalars.p, s));
         return proof_gen_common(c, n, sigs, n_msgs, idx, dis_off, rand, rand_off, commit_off, ph, ph_len, proofs_out,
-                                commitments_out, status);
+                                commitments_out, status, ph_off, headers, hdr_off);
     }
 
     // ---- random-linear-combination batch mode (rlc.cuh) ---------------------------------------------
@@ -768,14 +910,14 @@ struct Impl {
         return finish_status(c, n, status);
     }
     static int sign_common(Ctx* c, const uint8_t* sk, size_t n, uint32_t n_msgs, uint8_t* sigs_out, uint8_t* b_out,
-                           uint8_t* status) {
+                           uint8_t* status, const ItemKeyView* item = nullptr) {
         rt_stream_t s = c->stream;
         TRY(c->s_out.reserve(n * SIG));
         TRY(c->s_out2.reserve(n * C::G1_BYTES));
         TRY(c->s_status.reserve(n));
         TRY(rt_memset(c->s_out.p, 0, n * SIG, s));
         TRY(core_sign_dev(c, sk, n, (const uint8_t*)c->s_scalars.p, n_msgs, (uint8_t*)c->s_out.p,
-                          b_out ? (uint8_t*)c->s_out2.p : nullptr, (uint8_t*)c->s_status.p, s));
+                          b_out ? (uint8_t*)c->s_out2.p : nullptr, (uint8_t*)c->s_status.p, s, item));
         TRY(rt_d2h(sigs_out, c->s_out.p, n * SIG, s));
         if (b_out) TRY(rt_d2h(b_out, c->s_out2.p, n * C::G1_BYTES, s));
         // the signer's staging copies of the messages and their scalars do not outlive the call
@@ -877,10 +1019,18 @@ struct Impl {
         TRY(h2s_dev(c, count, (const uint8_t*)c->s_msgs.p, (const uint64_t*)c->s_offsets.p, (uint8_t*)c->s_scalars.p, s));
         return sign_common(c, sk, n, n_msgs, sigs_out, b_out, status);
     }
+    // ph_off != nullptr: per-item phs in `ph`; hdr_off != nullptr: per-item headers (bbs_*proof_verify_batch_hdr)
     static int proof_common(Ctx* c, size_t n, const uint8_t* proofs, const uint8_t* commit, const uint64_t* commit_off,
                             const uint32_t* idx, const uint64_t* dis_off, const uint8_t* ph, size_t ph_len,
-                            uint8_t* status, IssuerSet* S = nullptr, const uint32_t* item_issuer = nullptr) {
+                            uint8_t* status, IssuerSet* S = nullptr, const uint32_t* item_issuer = nullptr,
+                            const uint64_t* ph_off = nullptr, const uint8_t* headers = nullptr, const uint64_t* hdr_off = nullptr) {
         rt_stream_t s = c->stream;
+        ItemKeyView item{};
+        if (hdr_off) TRY(item_keys(c, n, headers, hdr_off, item));
+        if (ph_off) {
+            ph_len = ph_off[n];
+            TRY(stage(c->s_ph_off, ph_off, (n + 1) * 8, s));
+        }
         if (S) TRY(stage(S->item_issuer, item_issuer, n * 4, s));
         TRY(stage(c->s_sigs, proofs, n * PROOF, s));
         TRY(stage(c->s_commit, commit, commit_off[n] * 32, s));
@@ -892,20 +1042,24 @@ struct Impl {
         TRY(core_proof_verify_dev(c, n, (const uint8_t*)c->s_sigs.p, (const uint8_t*)c->s_commit.p,
                                   (const uint64_t*)c->s_commit_off.p, (const uint32_t*)c->s_dis_idx.p,
                                   (const uint8_t*)c->s_dis_scalars.p, (const uint64_t*)c->s_dis_off.p,
-                                  (const uint8_t*)c->s_ph.p, ph_len, (uint8_t*)c->s_status.p, s, S));
+                                  (const uint8_t*)c->s_ph.p, ph_len, (uint8_t*)c->s_status.p, s, S, hdr_off ? &item : nullptr,
+                                  ph_off ? (const uint64_t*)c->s_ph_off.p : nullptr));
         return finish_status(c, n, status);
     }
     static int core_proof_verify(Ctx* c, size_t n, const uint8_t* proofs, const uint8_t* commit, const uint64_t* commit_off,
                                  const uint32_t* idx, const uint8_t* dis_scalars, const uint64_t* dis_off,
                                  const uint8_t* ph, size_t ph_len, uint8_t* status, IssuerSet* S = nullptr,
-                                 const uint32_t* item_issuer = nullptr) {
+                                 const uint32_t* item_issuer = nullptr, const uint64_t* ph_off = nullptr,
+                                 const uint8_t* headers = nullptr, const uint64_t* hdr_off = nullptr) {
         TRY(stage(c->s_dis_scalars, dis_scalars, dis_off[n] * 32, c->stream));
-        return proof_common(c, n, proofs, commit, commit_off, idx, dis_off, ph, ph_len, status, S, item_issuer);
+        return proof_common(c, n, proofs, commit, commit_off, idx, dis_off, ph, ph_len, status, S, item_issuer, ph_off, headers,
+                            hdr_off);
     }
     static int proof_verify(Ctx* c, size_t n, const uint8_t* proofs, const uint8_t* commit, const uint64_t* commit_off,
                             const uint32_t* idx, const uint8_t* dis_msgs, const uint64_t* dis_msg_off,
                             const uint64_t* dis_off, const uint8_t* ph, size_t ph_len, uint8_t* status,
-                            IssuerSet* S = nullptr, const uint32_t* item_issuer = nullptr) {
+                            IssuerSet* S = nullptr, const uint32_t* item_issuer = nullptr, const uint64_t* ph_off = nullptr,
+                            const uint8_t* headers = nullptr, const uint64_t* hdr_off = nullptr) {
         rt_stream_t s = c->stream;
         const size_t count = dis_off[n];
         TRY(stage(c->s_dis_msgs, dis_msgs, dis_msg_off[count], s));
@@ -913,7 +1067,8 @@ struct Impl {
         TRY(c->s_dis_scalars.reserve(count * 32));
         TRY(h2s_dev(c, count, (const uint8_t*)c->s_dis_msgs.p, (const uint64_t*)c->s_dis_msg_off.p,
                     (uint8_t*)c->s_dis_scalars.p, s));
-        return proof_common(c, n, proofs, commit, commit_off, idx, dis_off, ph, ph_len, status, S, item_issuer);
+        return proof_common(c, n, proofs, commit, commit_off, idx, dis_off, ph, ph_len, status, S, item_issuer, ph_off, headers,
+                            hdr_off);
     }
 };
 
@@ -932,6 +1087,13 @@ int fresh_seed(uint8_t out[32]) {
     return 0;
 }
 
+// the per-item header arguments of a *_hdr call: `required` (verify / sign) or NULL = the context's header (proofs)
+int check_hdr_args(Ctx* c, size_t n, const uint8_t* headers, const uint64_t* hdr_off, bool required) {
+    if (!c) return arg_error("null context");
+    if (!hdr_off) return required ? arg_error("hdr_off is null") : BBS_OK;
+    if (!c->per_item_header) return arg_error("per-item headers need a context created with BBS_CTX_PER_ITEM_HEADER");
+    return check_items(n, headers, hdr_off, "header");
+}
 #define DISPATCH(c, call)                                              \
     do {                                                               \
         if (!(c)) return arg_error("null context");                    \
@@ -981,7 +1143,7 @@ int bbs_ctx_create_ex(int curve, int device, uint32_t flags, const uint8_t* pk, 
     if (!out) return arg_error("out is null");
     *out = nullptr;
     if (curve != BBS_CURVE_BLS12_381 && curve != BBS_CURVE_BN254) return arg_error("unknown curve id");
-    if (flags & ~(uint32_t)BBS_CTX_SMALL_TABLES) return arg_error("unknown context flag");
+    if (flags & ~(uint32_t)(BBS_CTX_SMALL_TABLES | BBS_CTX_PER_ITEM_HEADER)) return arg_error("unknown context flag");
     if (!pk || !generators || n_generators < 1) return arg_error("pk / generators missing");
     if (n_generators - 1 > BBS_MAX_MESSAGES) return arg_error("too many generators");
     if ((header_len && !header) || (api_id_len && !api_id)) return arg_error("null header / api_id");
@@ -1169,6 +1331,100 @@ int bbs_proof_gen_batch(bbs_ctx* p, size_t n, const uint8_t* sigs, const uint8_t
                           commitments_out, status));
 }
 
+// ---- per-item headers and presentation headers ------------------------------------------------------------------
+int bbs_core_verify_batch_hdr(bbs_ctx* p, size_t n, const uint8_t* sigs, const uint8_t* scalars, uint32_t n_msgs,
+                              const uint8_t* headers, const uint64_t* hdr_off, uint8_t* status) {
+    Ctx* c = as_ctx(p);
+    if (!n) return BBS_OK;
+    if (!sigs || !status || (n_msgs && !scalars)) return arg_error("null");
+    CHECK_COUNTS(n, n_msgs);
+    TRY(check_hdr_args(c, n, headers, hdr_off, true));
+    DISPATCH(c, verify_hdr(c, n, sigs, scalars, nullptr, nullptr, n_msgs, headers, hdr_off, status));
+}
+int bbs_verify_batch_hdr(bbs_ctx* p, size_t n, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* off, uint32_t n_msgs,
+                         const uint8_t* headers, const uint64_t* hdr_off, uint8_t* status) {
+    Ctx* c = as_ctx(p);
+    if (!n) return BBS_OK;
+    if (!sigs || !status || !off) return arg_error("null");
+    CHECK_COUNTS(n, n_msgs);
+    TRY(check_hdr_args(c, n, headers, hdr_off, true));
+    DISPATCH(c, verify_hdr(c, n, sigs, nullptr, msgs, off, n_msgs, headers, hdr_off, status));
+}
+int bbs_core_sign_batch_hdr(bbs_ctx* p, const uint8_t sk[32], size_t n, const uint8_t* scalars, uint32_t n_msgs,
+                            const uint8_t* headers, const uint64_t* hdr_off, uint8_t* sigs_out, uint8_t* b_out, uint8_t* status) {
+    Ctx* c = as_ctx(p);
+    if (!n) return BBS_OK;
+    if (!sk || !sigs_out || !status || (n_msgs && !scalars)) return arg_error("null");
+    CHECK_COUNTS(n, n_msgs);
+    TRY(check_hdr_args(c, n, headers, hdr_off, true));
+    DISPATCH(c, sign_hdr(c, sk, n, scalars, nullptr, nullptr, n_msgs, headers, hdr_off, sigs_out, b_out, status));
+}
+int bbs_sign_batch_hdr(bbs_ctx* p, const uint8_t sk[32], size_t n, const uint8_t* msgs, const uint64_t* off, uint32_t n_msgs,
+                       const uint8_t* headers, const uint64_t* hdr_off, uint8_t* sigs_out, uint8_t* b_out, uint8_t* status) {
+    Ctx* c = as_ctx(p);
+    if (!n) return BBS_OK;
+    if (!sk || !sigs_out || !status || !off) return arg_error("null");
+    CHECK_COUNTS(n, n_msgs);
+    TRY(check_hdr_args(c, n, headers, hdr_off, true));
+    DISPATCH(c, sign_hdr(c, sk, n, nullptr, msgs, off, n_msgs, headers, hdr_off, sigs_out, b_out, status));
+}
+int bbs_core_proof_verify_batch_hdr(bbs_ctx* p, size_t n, const uint8_t* proofs, const uint8_t* commit,
+                                    const uint64_t* commit_off, const uint32_t* idx, const uint8_t* dis_scalars,
+                                    const uint64_t* dis_off, const uint8_t* headers, const uint64_t* hdr_off,
+                                    const uint8_t* phs, const uint64_t* ph_off, uint8_t* status) {
+    Ctx* c = as_ctx(p);
+    if (!n) return BBS_OK;
+    if (!proofs || !commit_off || !dis_off || !status || !ph_off) return arg_error("null");
+    CHECK_COUNTS(n, 1);
+    if (commit_off[n] > 0xffffffffull || dis_off[n] > 0xffffffffull) return arg_error("batch too large: flat counts must fit in 32 bits");
+    TRY(check_hdr_args(c, n, headers, hdr_off, false));
+    TRY(check_items(n, phs, ph_off, "ph"));
+    DISPATCH(c, core_proof_verify(c, n, proofs, commit, commit_off, idx, dis_scalars, dis_off, phs, 0, status, nullptr, nullptr,
+                                  ph_off, headers, hdr_off));
+}
+int bbs_proof_verify_batch_hdr(bbs_ctx* p, size_t n, const uint8_t* proofs, const uint8_t* commit, const uint64_t* commit_off,
+                               const uint32_t* idx, const uint8_t* dis_msgs, const uint64_t* dis_msg_off, const uint64_t* dis_off,
+                               const uint8_t* headers, const uint64_t* hdr_off, const uint8_t* phs, const uint64_t* ph_off,
+                               uint8_t* status) {
+    Ctx* c = as_ctx(p);
+    if (!n) return BBS_OK;
+    if (!proofs || !commit_off || !dis_off || !dis_msg_off || !status || !ph_off) return arg_error("null");
+    CHECK_COUNTS(n, 1);
+    if (commit_off[n] > 0xffffffffull || dis_off[n] > 0xffffffffull) return arg_error("batch too large: flat counts must fit in 32 bits");
+    TRY(check_hdr_args(c, n, headers, hdr_off, false));
+    TRY(check_items(n, phs, ph_off, "ph"));
+    DISPATCH(c, proof_verify(c, n, proofs, commit, commit_off, idx, dis_msgs, dis_msg_off, dis_off, phs, 0, status, nullptr, nullptr,
+                             ph_off, headers, hdr_off));
+}
+int bbs_core_proof_gen_batch_hdr(bbs_ctx* p, size_t n, const uint8_t* sigs, const uint8_t* scalars, uint32_t n_msgs,
+                                 const uint32_t* idx, const uint64_t* dis_off, const uint8_t* rand, const uint64_t* rand_off,
+                                 const uint64_t* commit_off, const uint8_t* headers, const uint64_t* hdr_off, const uint8_t* phs,
+                                 const uint64_t* ph_off, uint8_t* proofs_out, uint8_t* commitments_out, uint8_t* status) {
+    Ctx* c = as_ctx(p);
+    if (!n) return BBS_OK;
+    if (!sigs || !dis_off || !rand || !rand_off || !commit_off || !proofs_out || !status || !ph_off) return arg_error("null");
+    CHECK_COUNTS(n, n_msgs);
+    if (n_msgs > BBS_MAX_MESSAGES) return arg_error("n_msgs exceeds BBS_MAX_MESSAGES");
+    TRY(check_hdr_args(c, n, headers, hdr_off, false));
+    TRY(check_items(n, phs, ph_off, "ph"));
+    DISPATCH(c, core_proof_gen(c, n, sigs, scalars, n_msgs, idx, dis_off, rand, rand_off, commit_off, phs, 0, proofs_out,
+                               commitments_out, status, ph_off, headers, hdr_off));
+}
+int bbs_proof_gen_batch_hdr(bbs_ctx* p, size_t n, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* off, uint32_t n_msgs,
+                            const uint32_t* idx, const uint64_t* dis_off, const uint8_t* rand, const uint64_t* rand_off,
+                            const uint64_t* commit_off, const uint8_t* headers, const uint64_t* hdr_off, const uint8_t* phs,
+                            const uint64_t* ph_off, uint8_t* proofs_out, uint8_t* commitments_out, uint8_t* status) {
+    Ctx* c = as_ctx(p);
+    if (!n) return BBS_OK;
+    if (!sigs || !off || !dis_off || !rand || !rand_off || !commit_off || !proofs_out || !status || !ph_off) return arg_error("null");
+    CHECK_COUNTS(n, n_msgs);
+    if (n_msgs > BBS_MAX_MESSAGES) return arg_error("n_msgs exceeds BBS_MAX_MESSAGES");
+    TRY(check_hdr_args(c, n, headers, hdr_off, false));
+    TRY(check_items(n, phs, ph_off, "ph"));
+    DISPATCH(c, proof_gen(c, n, sigs, msgs, off, n_msgs, idx, dis_off, rand, rand_off, commit_off, phs, 0, proofs_out,
+                          commitments_out, status, ph_off, headers, hdr_off));
+}
+
 // ---- issuer sets (multi-issuer batches) -------------------------------------------------------------------
 int bbs_issuer_set_create(int curve, int device, size_t n_issuers, const uint8_t* pks, const uint8_t* generators,
                           uint32_t n_generators, const uint8_t* header, size_t header_len, const uint8_t* api_id,
@@ -1339,6 +1595,27 @@ int bbs_core_proof_verify_batch_dev(bbs_ctx* p, size_t n, const uint8_t* d_proof
     CHECK_COUNTS(n, 1);
     DISPATCH(c, core_proof_verify_dev(c, n, d_proofs, d_commit, d_commit_off, d_idx, d_dis_scalars, d_dis_off, d_ph,
                                       ph_len, d_status, (rt_stream_t)stream));
+}
+
+// device-buffer forms: the offsets are device memory and, as for every *_dev call, the caller's contract
+int bbs_core_verify_batch_hdr_dev(bbs_ctx* p, size_t n, const uint8_t* d_sigs, const uint8_t* d_scalars, uint32_t n_msgs,
+                                  const uint8_t* d_headers, const uint64_t* d_hdr_off, uint8_t* d_status, void* stream) {
+    Ctx* c = as_ctx(p);
+    CHECK_COUNTS(n, n_msgs);
+    if (!d_hdr_off) return arg_error("hdr_off is null");
+    if (c && !c->per_item_header) return arg_error("per-item headers need a context created with BBS_CTX_PER_ITEM_HEADER");
+    DISPATCH(c, core_verify_hdr_dev(c, n, d_sigs, d_scalars, n_msgs, d_headers, d_hdr_off, d_status, (rt_stream_t)stream));
+}
+int bbs_core_proof_verify_batch_hdr_dev(bbs_ctx* p, size_t n, const uint8_t* d_proofs, const uint8_t* d_commit,
+                                        const uint64_t* d_commit_off, const uint32_t* d_idx, const uint8_t* d_dis_scalars,
+                                        const uint64_t* d_dis_off, const uint8_t* d_headers, const uint64_t* d_hdr_off,
+                                        const uint8_t* d_phs, const uint64_t* d_ph_off, uint8_t* d_status, void* stream) {
+    Ctx* c = as_ctx(p);
+    CHECK_COUNTS(n, 1);
+    if (!d_ph_off) return arg_error("ph_off is null");
+    if (c && d_hdr_off && !c->per_item_header) return arg_error("per-item headers need a context created with BBS_CTX_PER_ITEM_HEADER");
+    DISPATCH(c, core_proof_verify_hdr_dev(c, n, d_proofs, d_commit, d_commit_off, d_idx, d_dis_scalars, d_dis_off, d_headers,
+                                          d_hdr_off, d_phs, d_ph_off, d_status, (rt_stream_t)stream));
 }
 
 int bbs_selftest_field(int curve, int device, int op, size_t n, const uint8_t* a, const uint8_t* b, uint8_t* out) {

@@ -3,6 +3,7 @@
 // loop (BBS_HOSTSIM) for GPU-less debugging.
 //
 //   ctx creation : ctx_decode_item, ctx_domain_item, ctx_table_item, ctx_lines_item
+//   per-item hdr : item_domain_item                (calculate_domain + K per item, bbs_*_hdr calls)
 //   hashing      : h2s_item                      (msg_to_scalars, interface_utilities.rs:76-88)
 //   verify       : verify_g1_item -> pairing_item (core_verify, verify.rs:53-93)
 //   sign         : sign_item                      (core_sign, sign.rs:63-133)
@@ -90,20 +91,45 @@ struct CtxDomainArgs {
     const uint8_t* api_id; uint32_t api_id_len; const uint8_t* header; uint32_t header_len;
     const uint8_t* dst_h2s; uint32_t dst_h2s_len;
     const uint32_t* gens; uint32_t* domain; uint32_t* K; uint32_t* k_inf;
+    uint32_t* prefix;          // optional: the hash state after domain_prefix (SHA_STATE_WORDS), for per-item headers
 };
-// calculate_domain (core_utilities.rs:24-63) + K = P1 + Q1*domain (verify.rs:81-82)
-template <class C> BBS_HD void ctx_domain_item(const CtxDomainArgs& a, uint32_t) {
-    Xmd48 x;
+// Sha256 state as plain words: h, the partial block w, fill, total
+constexpr int SHA_STATE_WORDS = 26;
+BBS_HD void sha_store(uint32_t* dst, const Sha256& s) {
+    for (int k = 0; k < 8; k++) dst[k] = s.h[k];
+    for (int k = 0; k < 16; k++) dst[8 + k] = s.w[k];
+    dst[24] = s.fill; dst[25] = s.total;
+}
+BBS_HD void sha_load(Sha256& s, const uint32_t* src) {
+    for (int k = 0; k < 8; k++) s.h[k] = src[k];
+    for (int k = 0; k < 16; k++) s.w[k] = src[8 + k];
+    s.fill = src[24]; s.total = src[25];
+}
+// calculate_domain (core_utilities.rs:24-63) in two parts.  The prefix Z_pad || comp(pk) || I2OSP(L, 8) || comp(Q1) ..
+// comp(H_L) || api_id does not depend on the header, so a per-item-header context keeps the state after it.
+template <class C> BBS_HD void domain_prefix(Xmd48& x, const CtxDomainArgs& a) {
     x.begin();
     x.s.update(a.pk_comp, C::G2_BYTES);
     x.s.put_be64(a.L);
     x.s.update(a.gens_comp, (a.L + 1) * C::G1_BYTES);
     x.s.update(a.api_id, a.api_id_len);
-    x.s.put_be64(a.header_len);
-    x.s.update(a.header, a.header_len);
-    BBS_A16 uint32_t okm[12], dom[8];
-    x.finish(a.dst_h2s, a.dst_h2s_len, okm);
+}
+// ... then I2OSP(header_len, 8) || header, expanded and reduced to the domain scalar (canonical limbs)
+template <class C> BBS_HD void domain_finish(Xmd48& x, const uint8_t* header, uint32_t header_len, const uint8_t* dst,
+                                             uint32_t dst_len, uint32_t* dom) {
+    x.s.put_be64(header_len);
+    x.s.update(header, header_len);
+    BBS_A16 uint32_t okm[12];
+    x.finish(dst, dst_len, okm);
     okm48_to_scalar<typename C::Fr>(dom, okm);
+}
+// calculate_domain + K = P1 + Q1*domain (verify.rs:81-82)
+template <class C> BBS_HD void ctx_domain_item(const CtxDomainArgs& a, uint32_t) {
+    Xmd48 x;
+    domain_prefix<C>(x, a);
+    if (a.prefix) sha_store(a.prefix, x.s);
+    BBS_A16 uint32_t dom[8];
+    domain_finish<C>(x, a.header, a.header_len, a.dst_h2s, a.dst_h2s_len, dom);
     bn_copy<8>(a.domain, dom);
     BBS_A16 uint32_t acc[G1J], p1[G1J];
     g1_mul_affine<C>(acc, a.gens, dom, 256);
@@ -112,7 +138,8 @@ template <class C> BBS_HD void ctx_domain_item(const CtxDomainArgs& a, uint32_t)
     *a.k_inf = g1_to_affine_vt<C>(a.K, acc) ? 0u : 1u;
 }
 
-struct CtxTableArgs { const uint32_t* K; const uint32_t* gens; uint32_t* tab; uint32_t* wbase; uint32_t tab_bits; };
+// q1_slot != 0: generator slot q1_slot is Q1 again (slot L + 1 of a per-item-header context)
+struct CtxTableArgs { const uint32_t* K; const uint32_t* gens; uint32_t* tab; uint32_t* wbase; uint32_t tab_bits; uint32_t q1_slot; };
 // entry (g, w, d) = (d * 2^(BITS w)) * base_g in affine form, in two steps:
 //   ctx_wbase_item: the window bases 2^(BITS w) * base_g, affine (one thread per (g, w); a K at infinity gives zeros);
 //   ctx_table_item: d * window base by a BITS-bit double-and-add, then to affine.
@@ -121,7 +148,7 @@ template <class C> BBS_HD void ctx_wbase_item(const CtxTableArgs& a, uint32_t i)
     const uint32_t TAB_WINDOWS = (uint32_t)G.windows;
     const int TAB_BITS = G.bits;
     const uint32_t w = i % TAB_WINDOWS, g = i / TAB_WINDOWS;
-    const uint32_t* base = g == 0 ? a.K : a.gens + g * G1A;
+    const uint32_t* base = g == 0 ? a.K : a.gens + (g == a.q1_slot ? 0u : g) * G1A;
     BBS_A16 uint32_t acc[G1J];
     g1_from_affine<C>(acc, base);
     if (bn_is_zero<2 * C::Fp::N>(base)) g1_set_inf<C>(acc);          // K at infinity is stored as zeros
@@ -275,6 +302,71 @@ template <class C> BBS_HDN void tab_accumulate(uint32_t* acc, const CtxView& cx,
 #define PAIR_WORDS (6 * C::Fp::N)
 enum : uint32_t { FL_SKIP0 = 1, FL_SKIP1 = 2, FL_DONE = 4 };   // FL_DONE: status already final, no pairing
 
+// ---- per-item headers (bbs_*_hdr) ------------------------------------------------------------------------
+// A call with a header per item hashes domain_i and builds K_i = P1 + Q1 * domain_i per item (item_domain_kernel below) into
+// arrays indexed by item; W and the line tables stay the context's.  K == nullptr: every item uses the context's K and domain.
+struct ItemKeyView {
+    const uint32_t* K;         // n x affine K_i (zeros for the identity)
+    const uint32_t* domains;   // n x 8 words, canonical limbs
+    const uint32_t* flags;     // n x (ISS_K_INF or 0)
+};
+// K, domain and identity flags (ISS_W_INF | ISS_K_INF) of item i
+template <class C> BBS_HD uint32_t item_key(const CtxView& cx, const ItemKeyView& it, uint32_t i, const uint32_t*& K,
+                                            const uint32_t*& domain) {
+    const uint32_t w = cx.w_inf ? (uint32_t)ISS_W_INF : 0u;
+    if (!it.K) { K = cx.K; domain = cx.domain; return w | (cx.k_inf ? (uint32_t)ISS_K_INF : 0u); }
+    K = it.K + (size_t)i * G1A; domain = it.domains + (size_t)i * 8;
+    return w | it.flags[i];
+}
+// domain of item i alone: sign and proof gen read it where they hash it, so that no pointer is held across the G1 work
+// (that cost those kernels spill slots)
+template <class C> BBS_HD const uint32_t* item_domain(const CtxView& cx, const ItemKeyView& it, uint32_t i) {
+    return it.K ? it.domains + (size_t)i * 8 : cx.domain;
+}
+// presentation header of item i: the call's shared ph, or ph[ph_off[i] .. ph_off[i+1]) when the call has one per item
+BBS_HD const uint8_t* item_ph(const uint8_t* ph, uint32_t ph_len, const uint64_t* ph_off, uint32_t i, uint32_t& len) {
+    if (!ph_off) { len = ph_len; return ph; }
+    len = (uint32_t)(ph_off[i + 1] - ph_off[i]);
+    return ph + ph_off[i];
+}
+
+struct ItemDomainArgs {
+    CtxView ctx;
+    const uint32_t* prefix;                         // hash state after domain_prefix (SHA_STATE_WORDS)
+    const uint8_t* headers; const uint64_t* hdr_off;  // header i = headers[hdr_off[i] .. hdr_off[i+1])
+    uint32_t* domains; uint32_t* K; uint32_t* flags;  // the arrays of ItemKeyView
+};
+// domain_i (written out) and the Jacobian K_i; Q1's window table is slot L + 1 of a per-item-header context
+template <class C> BBS_HD void item_domain_head(const ItemDomainArgs& a, uint32_t i, uint32_t* Kj) {
+    Xmd48 x;
+    sha_load(x.s, a.prefix);
+    const uint64_t b = a.hdr_off[i];
+    BBS_A16 uint32_t dom[8];
+    domain_finish<C>(x, a.headers + b, (uint32_t)(a.hdr_off[i + 1] - b), a.ctx.dst_h2s, a.ctx.dst_h2s_len, dom);
+    bn_copy<8>(a.domains + (size_t)i * 8, dom);
+    g1_from_affine<C>(Kj, C::P1());
+    tab_accumulate<C>(Kj, a.ctx, a.ctx.L + 1, dom);
+}
+// K_i to affine with zinv = 1 / Z (unused for the identity)
+template <class C> BBS_HD void item_domain_tail(const ItemDomainArgs& a, uint32_t i, const uint32_t* Kj, const uint32_t* zinv) {
+    using F = typename C::Fp;
+    uint32_t* K = a.K + (size_t)i * G1A;
+    if (g1_is_inf_ool<C>(Kj)) { bn_zero<2 * C::Fp::N>(K); a.flags[i] = ISS_K_INF; return; }
+    BBS_A16 uint32_t zi2[FPN];
+    fe_sqr<F>(zi2, zinv);
+    fe_mul<F>(K, Kj, zi2);
+    fe_mul<F>(zi2, zi2, zinv);
+    fe_mul<F>(K + FPN, Kj + FPN, zi2);
+    a.flags[i] = 0;
+}
+// one item, its own inversion (host simulation; the CUDA build uses item_domain_kernel)
+template <class C> BBS_HD void item_domain_item(const ItemDomainArgs& a, uint32_t i) {
+    BBS_A16 uint32_t Kj[G1J], z[FPN];
+    item_domain_head<C>(a, i, Kj);
+    if (!g1_is_inf_ool<C>(Kj)) fe_inv<typename C::Fp>(z, Kj + 2 * FPN);
+    item_domain_tail<C>(a, i, Kj, z);
+}
+
 // ---- core_verify, G1 half ------------------------------------------------------------------------------
 struct VerifyG1Args {
     CtxView ctx;
@@ -286,11 +378,12 @@ struct VerifyG1Args {
     IssuerSetView iss;
     // split path (verify_g1_split_kernel + verify_g1_combine_kernel): per item the Jacobian e*A and B and a state byte
     uint32_t* part_v; uint32_t* part_f; uint8_t* part_st;
+    ItemKeyView item;              // per-item headers (not with issuer sets)
 };
 enum : uint8_t { VST_PA = 3, VST_VDONE = 4, VST_FBAD = 8 };      // part_st: PT_* of A | status already final | bad scalar
 // the key-dependent inputs of item i: K and the two identity flags
 template <class C> BBS_HD uint32_t verify_issuer(const VerifyG1Args& a, uint32_t i, const uint32_t*& K) {
-    if (!a.item_issuer) { K = a.ctx.K; return (a.ctx.w_inf ? ISS_W_INF : 0u) | (a.ctx.k_inf ? ISS_K_INF : 0u); }
+    if (!a.item_issuer) { const uint32_t* domain; return item_key<C>(a.ctx, a.item, i, K, domain); }
     const uint32_t s = a.item_issuer[i];
     if (s >= a.iss.n_issuers) { K = a.ctx.K; return ISS_BAD; }
     K = a.iss.K + (size_t)s * G1A;
@@ -529,6 +622,21 @@ verify_g1_combine_kernel(const VerifyG1Args a, uint32_t n, const uint8_t* fbad) 
 }
 #endif
 
+#if defined(__CUDACC__) && !defined(BBS_HOSTSIM)
+// domain_i and K_i of a call with per-item headers, one inversion per block for the affine K_i
+template <class C, int TPB> __global__ void __launch_bounds__(TPB, 4) item_domain_kernel(const ItemDomainArgs a, uint32_t n) {
+    using F = typename C::Fp;
+    __shared__ BBS_A16 uint32_t tree[2 * TPB][C::Fp::N];
+    const uint32_t i = blockIdx.x * TPB + threadIdx.x;
+    BBS_A16 uint32_t Kj[G1J], z[FPN];
+    const bool live = i < n;
+    if (live) item_domain_head<C>(a, i, Kj);
+    if (live && !g1_is_inf_ool<C>(Kj)) bn_copy<C::Fp::N>(z, Kj + 2 * FPN); else fe_set_one<F>(z);
+    block_batch_inverse<F, TPB, true>(z, tree);
+    if (live) item_domain_tail<C>(a, i, Kj, z);
+}
+#endif
+
 // ---- pairing half (shared by verify and proof verify) ----------------------------------------------------
 struct PairingArgs {
     const uint32_t* lines; const uint32_t* pair; const uint32_t* flags; uint8_t* status;
@@ -554,13 +662,16 @@ struct SignArgs {
     uint8_t* sigs_out;         // n x (G1 compressed || LE32 e)
     uint8_t* b_out;            // optional: n x G1 compressed B (row a7)
     uint8_t* status;
+    ItemKeyView item;          // per-item headers
 };
 // core_sign in three parts around its three inversions (1 / B.Z, 1 / (sk + e), 1 / A.Z), so that the CUDA build can take
 // each of them once per block (sign_kernel below) while the host simulation inverts per item (sign_item).
 // Part 1: B (Jacobian), e, and sk + e in Montgomery form.  false: the item's status is final.
-template <class C> BBS_HD bool sign_head(const SignArgs& a, uint32_t i, uint32_t* B, uint32_t* e, uint32_t* sm) {
+// PER_ITEM = false: a call without per-item headers; the per-item reads are compiled out (sign_kernel)
+template <class C, bool PER_ITEM> BBS_HD bool sign_head(const SignArgs& a, uint32_t i, uint32_t* B, uint32_t* e, uint32_t* sm) {
     using Fr = typename C::Fr;
     const CtxView& cx = a.ctx;
+    const ItemKeyView item = PER_ITEM ? a.item : ItemKeyView{};
     if (a.n_msgs != cx.L) { a.status[i] = ST_ERR_MSG_GEN_LEN; return false; }     // sign.rs:76-79
     const uint8_t* sc = a.scalars + (size_t)i * a.n_msgs * 32;
     // e = H2S(BE(sk) || BE(m_1..m_L) || BE(domain), api_id || "H2S_")   (sign.rs:90-118)
@@ -569,7 +680,10 @@ template <class C> BBS_HD bool sign_head(const SignArgs& a, uint32_t i, uint32_t
     BBS_A16 uint32_t sk[8];
     for (int k = 0; k < 8; k++) sk[k] = a.sk[k];
     for (int k = 7; k >= 0; k--) x.s.update_words(&sk[k], 1);
-    if (cx.k_inf) g1_set_inf<C>(B); else g1_from_affine<C>(B, cx.K);
+    {
+        const uint32_t *Kp, *domain;
+        if (item_key<C>(cx, item, i, Kp, domain) & ISS_K_INF) g1_set_inf<C>(B); else g1_from_affine<C>(B, Kp);
+    }
     bool ok = true;
     for (uint32_t j = 0; j < a.n_msgs && ok; j++) {
         BBS_A16 uint32_t m[8];
@@ -579,7 +693,8 @@ template <class C> BBS_HD bool sign_head(const SignArgs& a, uint32_t i, uint32_t
         tab_accumulate<C>(B, cx, j + 1, m);                                      // sign.rs:120-126
     }
     if (!ok) { a.status[i] = ST_ERR_MALFORMED; return false; }
-    for (int k = 7; k >= 0; k--) x.s.update_words(&cx.domain[k], 1);
+    const uint32_t* domain = item_domain<C>(cx, item, i);
+    for (int k = 7; k >= 0; k--) x.s.update_words(&domain[k], 1);
     BBS_A16 uint32_t okm[12], s[8];
     x.finish(cx.dst_h2s, cx.dst_h2s_len, okm);
     okm48_to_scalar<Fr>(e, okm);
@@ -633,7 +748,7 @@ template <class C> BBS_HD void sign_tail(const SignArgs& a, uint32_t i, const ui
 template <class C> BBS_HD void sign_item(const SignArgs& a, uint32_t i) {
     using F = typename C::Fp;
     BBS_A16 uint32_t B[G1J], e[8], sm[8], zinv[FPN], Aj[G1J], Baff[G1A];
-    if (!sign_head<C>(a, i, B, e, sm)) return;
+    if (!sign_head<C, true>(a, i, B, e, sm)) return;
     if (!g1_is_inf_ool<C>(B)) fe_inv<F>(zinv, B + 2 * FPN);
     fe_inv<typename C::Fr>(sm, sm);
     bool bfin;
@@ -644,13 +759,15 @@ template <class C> BBS_HD void sign_item(const SignArgs& a, uint32_t i) {
 
 #if defined(__CUDACC__) && !defined(BBS_HOSTSIM)
 // the three inversions of core_sign, each taken once per block (block_batch_inverse: Montgomery's trick as a product tree)
-template <class C, int TPB, int MINB> __global__ void __launch_bounds__(TPB, MINB) sign_kernel(const SignArgs a, uint32_t n) {
+// PER_ITEM = false (calls without per-item headers): the per-item reads are compiled out, so that these calls run the code
+// they ran before per-item headers existed
+template <class C, int TPB, int MINB, bool PER_ITEM> __global__ void __launch_bounds__(TPB, MINB) sign_kernel(const SignArgs a, uint32_t n) {
     using F = typename C::Fp;
     using Fr = typename C::Fr;
     __shared__ BBS_A16 uint32_t tree[2 * TPB][C::Fp::N];
     const uint32_t i = blockIdx.x * TPB + threadIdx.x;
     BBS_A16 uint32_t B[G1J], e[8], sm[8], z[FPN], Aj[G1J], Baff[G1A];
-    const bool live = i < n && sign_head<C>(a, i, B, e, sm);
+    const bool live = i < n && sign_head<C, PER_ITEM>(a, i, B, e, sm);
     if (live && !g1_is_inf_ool<C>(B)) bn_copy<C::Fp::N>(z, B + 2 * FPN); else fe_set_one<F>(z);
     if (!live) fe_set_one<Fr>(sm);
     block_batch_inverse<F, TPB, true>(z, tree);
@@ -683,7 +800,14 @@ struct ProofG1Args {
     uint32_t* part_t1; uint32_t* part_v2; uint32_t* part_f; uint8_t* part_st;
     // issuer sets (split path only): proof i is checked under issuer item_issuer[i]; K_i * c is variable-base then
     const uint32_t* item_issuer; IssuerSetView iss;
+    // per-item headers (split path only, as issuer sets); per-item ph: ph[ph_off[i] .. ph_off[i+1]) (nullptr: shared ph)
+    ItemKeyView item; const uint64_t* ph_off;
 };
+// K_i has no window table when it is per item (issuer sets, per-item headers): K_i * c is then part of task V2.
+// PER_ITEM (here and in the proof_task_* / proof_join_* functions) = false: a call without per-item headers or phs, whose
+// kernels are compiled without the per-item reads (the host simulation passes true: the reads check for themselves)
+template <bool PER_ITEM> BBS_HD bool proof_k_variable(const ProofG1Args& a) { return a.item_issuer || (PER_ITEM && a.item.K); }
+template <bool PER_ITEM> BBS_HD const uint64_t* proof_ph_off(const ProofG1Args& a) { return PER_ITEM ? a.ph_off : nullptr; }
 template <class C> BBS_HD void proof_g1_item(const ProofG1Args& a, uint32_t i) {
     using F = typename C::Fp;
     using Fr = typename C::Fr;
@@ -771,8 +895,10 @@ template <class C> BBS_HD void proof_g1_item(const ProofG1Args& a, uint32_t i) {
         g1_compress_affine<C>(enc, aff, i2); x.s.update(enc, GB);
     }
     for (int q = 7; q >= 0; q--) x.s.update_words(&cx.domain[q], 1);
-    x.s.put_be64(a.ph_len);
-    x.s.update(a.ph, a.ph_len);
+    uint32_t ph_len;
+    const uint8_t* ph = item_ph(a.ph, a.ph_len, a.ph_off, i, ph_len);
+    x.s.put_be64(ph_len);
+    x.s.update(ph, ph_len);
     BBS_A16 uint32_t okm[12], c2[8];
     x.finish(cx.dst_h2s, cx.dst_h2s_len, okm);
     okm48_to_scalar<Fr>(c2, okm);
@@ -814,15 +940,15 @@ template <class C> BBS_HD uint8_t proof_shape(const ProofG1Args& a, uint32_t i, 
     return 0;
 }
 // the key-dependent inputs of proof i: K, domain and the identity flags (issuer sets: per item)
-template <class C> BBS_HD uint32_t proof_issuer(const ProofG1Args& a, uint32_t i, const uint32_t*& K, const uint32_t*& domain) {
+template <class C, bool PER_ITEM> BBS_HD uint32_t proof_issuer(const ProofG1Args& a, uint32_t i, const uint32_t*& K, const uint32_t*& domain) {
     K = a.ctx.K; domain = a.ctx.domain;
-    if (!a.item_issuer) return (a.ctx.w_inf ? ISS_W_INF : 0u) | (a.ctx.k_inf ? ISS_K_INF : 0u);
+    if (!a.item_issuer) return item_key<C>(a.ctx, PER_ITEM ? a.item : ItemKeyView{}, i, K, domain);
     const uint32_t s = a.item_issuer[i];
     if (s >= a.iss.n_issuers) return ISS_BAD;
     K = a.iss.K + (size_t)s * G1A; domain = a.iss.domains + (size_t)s * 8;
     return a.iss.flags[s];
 }
-template <class C> BBS_HD void proof_task_v1(const ProofG1Args& a, uint32_t i) {
+template <class C, bool PER_ITEM> BBS_HD void proof_task_v1(const ProofG1Args& a, uint32_t i) {
     using F = typename C::Fp;
     constexpr int GB = C::G1_BYTES;
     const uint8_t* pf = a.proofs + (size_t)i * (3 * GB + 128);
@@ -832,7 +958,7 @@ template <class C> BBS_HD void proof_task_v1(const ProofG1Args& a, uint32_t i) {
     if (err) { a.status[i] = err; a.flags[i] = FL_DONE; return; }
     {
         const uint32_t *Kp, *dom;
-        if (proof_issuer<C>(a, i, Kp, dom) & ISS_BAD) { a.status[i] = ST_ERR_MALFORMED; a.flags[i] = FL_DONE; return; }   // undecodable issuer key
+        if (proof_issuer<C, PER_ITEM>(a, i, Kp, dom) & ISS_BAD) { a.status[i] = ST_ERR_MALFORMED; a.flags[i] = FL_DONE; return; }   // undecodable issuer key
     }
     BBS_A16 uint32_t Ab[G1A], Bb[G1A], D[G1A], ecap[8], r1cap[8], r3cap[8], c[8];
     int pA = g1_decompress<C>(Ab, pf), pB = g1_decompress<C>(Bb, pf + GB), pD = g1_decompress<C>(D, pf + 2 * GB);
@@ -854,16 +980,16 @@ template <class C> BBS_HD void proof_task_v1(const ProofG1Args& a, uint32_t i) {
     bn_copy<C::Fp::N>(pr + 3 * FPN, Bb); fe_neg<F>(pr + 4 * FPN, Bb + FPN); fe_set_one<F>(pr + 5 * FPN);
     a.part_st[i] = (uint8_t)(pA | (pB << 2) | (pD << 4));
 }
-template <class C> BBS_HD void proof_task_v2(const ProofG1Args& a, uint32_t i) {
+template <class C, bool PER_ITEM> BBS_HD void proof_task_v2(const ProofG1Args& a, uint32_t i) {
     constexpr int GB = C::G1_BYTES;
     const uint8_t* pf = a.proofs + (size_t)i * (3 * GB + 128);
     ProofShape sh;
     if (proof_shape<C>(a, i, sh)) return;
     BBS_A16 uint32_t D[G1A], r3cap[8], t[G1J];
-    if (a.item_issuer) {
-        // issuer sets: K_i has no window table, so K_i * c joins D * r3^ in one two-point multiplication
+    if (proof_k_variable<PER_ITEM>(a)) {
+        // issuer sets / per-item headers: K_i has no window table, so K_i * c joins D * r3^ in one two-point multiplication
         const uint32_t *Kp, *dom;
-        const uint32_t ifl = proof_issuer<C>(a, i, Kp, dom);
+        const uint32_t ifl = proof_issuer<C, PER_ITEM>(a, i, Kp, dom);
         BBS_A16 uint32_t c[8], Ka[G1A];
         const int pD = g1_decompress<C>(D, pf + 2 * GB);
         if ((ifl & ISS_BAD) || pD == PT_BAD || !fr_from_le32<C>(r3cap, pf + 3 * GB + 64) || !fr_from_le32<C>(c, pf + 3 * GB + 96)) return;
@@ -878,7 +1004,7 @@ template <class C> BBS_HD void proof_task_v2(const ProofG1Args& a, uint32_t i) {
     g1_mul_scalar<C>(t, D, r3cap);
     g1_copy<C>(a.part_v2 + (size_t)i * G1J, t);
 }
-template <class C> BBS_HD void proof_task_f(const ProofG1Args& a, uint32_t i, uint8_t* fbad) {
+template <class C, bool PER_ITEM> BBS_HD void proof_task_f(const ProofG1Args& a, uint32_t i, uint8_t* fbad) {
     using Fr = typename C::Fr;
     const CtxView& cx = a.ctx;
     constexpr int GB = C::G1_BYTES;
@@ -891,7 +1017,7 @@ template <class C> BBS_HD void proof_task_f(const ProofG1Args& a, uint32_t i, ui
     // Bv*c = K*c + sum H_disclosed (c m), then sum H_undisclosed m^   (proof_verify.rs:165-182)
     fe_to_mont<Fr>(cm, c);
     g1_set_inf<C>(T2);
-    if (!a.item_issuer && !cx.k_inf) tab_accumulate<C>(T2, cx, 0, c);       // issuer sets: K_i * c is part of task V2
+    if (!proof_k_variable<PER_ITEM>(a) && !cx.k_inf) tab_accumulate<C>(T2, cx, 0, c);    // else K_i * c is part of task V2
     for (uint64_t k = 0; k < sh.R; k++) {
         BBS_A16 uint32_t m[8];
         if (!fr_from_le32<C>(m, a.dis_scalars + (sh.db + k) * 32)) { *fbad = 1; return; }
@@ -909,17 +1035,17 @@ template <class C> BBS_HD void proof_task_f(const ProofG1Args& a, uint32_t i, ui
     g1_copy<C>(a.part_f + (size_t)i * G1J, T2);
 }
 // join, part 1: T2 = F part (+ V2 part); false when the item's status is already final
-template <class C> BBS_HD bool proof_join_head(const ProofG1Args& a, uint32_t i, const uint8_t* fbad, uint32_t* T1, uint32_t* T2, uint8_t& st) {
+template <class C, bool PER_ITEM> BBS_HD bool proof_join_head(const ProofG1Args& a, uint32_t i, const uint8_t* fbad, uint32_t* T1, uint32_t* T2, uint8_t& st) {
     st = a.part_st[i];
     if (st & PST_DONE) return false;
     if (fbad[i]) { a.status[i] = ST_ERR_MALFORMED; a.flags[i] = FL_DONE; return false; }
     g1_copy<C>(T1, a.part_t1 + (size_t)i * G1J);
     g1_copy<C>(T2, a.part_f + (size_t)i * G1J);
-    if (((st >> 4) & 3) == PT_OK || a.item_issuer) g1_add<C>(T2, T2, a.part_v2 + (size_t)i * G1J);
+    if (((st >> 4) & 3) == PT_OK || proof_k_variable<PER_ITEM>(a)) g1_add<C>(T2, T2, a.part_v2 + (size_t)i * G1J);
     return true;
 }
 // join, part 2: zinv = 1 / (Z(T1) Z(T2)) with identities counted as Z = 1; challenge (proof_gen.rs:272-328), comparison, flags
-template <class C> BBS_HD void proof_join_tail(const ProofG1Args& a, uint32_t i, const uint32_t* T1, const uint32_t* T2, const uint32_t* zinv, uint8_t st) {
+template <class C, bool PER_ITEM> BBS_HD void proof_join_tail(const ProofG1Args& a, uint32_t i, const uint32_t* T1, const uint32_t* T2, const uint32_t* zinv, uint8_t st) {
     using F = typename C::Fp;
     using Fr = typename C::Fr;
     const CtxView& cx = a.ctx;
@@ -927,7 +1053,7 @@ template <class C> BBS_HD void proof_join_tail(const ProofG1Args& a, uint32_t i,
     const uint8_t* pf = a.proofs + (size_t)i * (3 * GB + 128);
     const uint64_t db = a.dis_off[i], R = a.dis_off[i + 1] - db;
     const uint32_t *Kp, *domain;
-    const uint32_t ifl = proof_issuer<C>(a, i, Kp, domain);
+    const uint32_t ifl = proof_issuer<C, PER_ITEM>(a, i, Kp, domain);
     Xmd48 x;
     x.begin();
     x.s.put_be64(R);
@@ -952,8 +1078,10 @@ template <class C> BBS_HD void proof_join_tail(const ProofG1Args& a, uint32_t i,
         g1_compress_affine<C>(enc, aff, i2); x.s.update(enc, GB);
     }
     for (int q = 7; q >= 0; q--) x.s.update_words(&domain[q], 1);
-    x.s.put_be64(a.ph_len);
-    x.s.update(a.ph, a.ph_len);
+    uint32_t ph_len;
+    const uint8_t* ph = item_ph(a.ph, a.ph_len, proof_ph_off<PER_ITEM>(a), i, ph_len);
+    x.s.put_be64(ph_len);
+    x.s.update(ph, ph_len);
     BBS_A16 uint32_t okm[12], c2[8], c[8];
     x.finish(cx.dst_h2s, cx.dst_h2s_len, okm);
     okm48_to_scalar<Fr>(c2, okm);
@@ -966,16 +1094,16 @@ template <class C> BBS_HD void proof_join_tail(const ProofG1Args& a, uint32_t i,
 }
 
 // the join with one inversion per proof (host simulation of proof_g1_join_kernel)
-template <class C> BBS_HD void proof_join_item(const ProofG1Args& a, uint32_t i, const uint8_t* fbad) {
+template <class C, bool PER_ITEM> BBS_HD void proof_join_item(const ProofG1Args& a, uint32_t i, const uint8_t* fbad) {
     using F = typename C::Fp;
     BBS_A16 uint32_t T1[G1J], T2[G1J], z[FPN];
     uint8_t st = 0;
-    if (!proof_join_head<C>(a, i, fbad, T1, T2, st)) return;
+    if (!proof_join_head<C, PER_ITEM>(a, i, fbad, T1, T2, st)) return;
     fe_set_one<F>(z);
     if (!g1_is_inf_ool<C>(T1)) bn_copy<C::Fp::N>(z, T1 + 2 * FPN);
     if (!g1_is_inf_ool<C>(T2)) fe_mul<F>(z, z, T2 + 2 * FPN);
     fe_inv<F>(z, z);
-    proof_join_tail<C>(a, i, T1, T2, z, st);
+    proof_join_tail<C, PER_ITEM>(a, i, T1, T2, z, st);
 }
 
 // ---- core_proof_gen (proof_gen.rs:116-365: proof_init, proof_challenge_calculate, proof_finalize) ---------------
@@ -995,11 +1123,17 @@ struct ProofGenArgs {
     uint8_t* proofs_out;           // n x (3 G1 compressed || LE32 e^, r1^, r3^, c)
     uint8_t* commitments_out;      // flat LE32
     uint8_t* status;
+    ItemKeyView item;              // per-item headers
+    const uint64_t* ph_off;        // per-item ph: ph[ph_off[i] .. ph_off[i+1]) (nullptr: shared ph)
 };
-template <class C> BBS_HD void proof_gen_item(const ProofGenArgs& a, uint32_t i) {
+// PER_ITEM = false: the calls without per-item headers / phs; their kernel is compiled without the per-item reads, which
+// cost it spill slots (proof generation runs at the register cap)
+template <class C, bool PER_ITEM> BBS_HD void proof_gen_item(const ProofGenArgs& a, uint32_t i) {
     using F = typename C::Fp;
     using Fr = typename C::Fr;
     const CtxView& cx = a.ctx;
+    const ItemKeyView item = PER_ITEM ? a.item : ItemKeyView{};
+    const uint64_t* ph_off = PER_ITEM ? a.ph_off : nullptr;
     constexpr int GB = C::G1_BYTES;
     const uint64_t L = a.n_msgs;
     const uint64_t db = a.dis_off[i], R = a.dis_off[i + 1] - db;
@@ -1027,7 +1161,10 @@ template <class C> BBS_HD void proof_gen_item(const ProofGenArgs& a, uint32_t i)
     if (!ok) GEN_FAIL(ST_ERR_MALFORMED)
     // B = P1 + Q1*domain + sum H_j m_j   (:247-253)
     BBS_A16 uint32_t B[G1J];
-    if (cx.k_inf) g1_set_inf<C>(B); else g1_from_affine<C>(B, cx.K);
+    {
+        const uint32_t *Kp, *domain;
+        if (item_key<C>(cx, item, i, Kp, domain) & ISS_K_INF) g1_set_inf<C>(B); else g1_from_affine<C>(B, Kp);
+    }
     for (uint32_t j = 0; j < (uint32_t)L; j++) {
         BBS_A16 uint32_t m[8];
         if (!fr_from_le32<C>(m, sc + j * 32)) GEN_FAIL(ST_ERR_MALFORMED)
@@ -1115,9 +1252,12 @@ template <class C> BBS_HD void proof_gen_item(const ProofGenArgs& a, uint32_t i)
     x.s.update(out, 3 * GB);
     x.s.update(encT1, GB);
     x.s.update(encT2, GB);
-    for (int q = 7; q >= 0; q--) x.s.update_words(&cx.domain[q], 1);
-    x.s.put_be64(a.ph_len);
-    x.s.update(a.ph, a.ph_len);
+    const uint32_t* domain = item_domain<C>(cx, item, i);
+    for (int q = 7; q >= 0; q--) x.s.update_words(&domain[q], 1);
+    uint32_t ph_len;
+    const uint8_t* ph = item_ph(a.ph, a.ph_len, ph_off, i, ph_len);
+    x.s.put_be64(ph_len);
+    x.s.update(ph, ph_len);
     BBS_A16 uint32_t okm[12], c[8], cm[8];
     x.finish(cx.dst_h2s, cx.dst_h2s_len, okm);
     okm48_to_scalar<Fr>(c, okm);
@@ -1148,27 +1288,29 @@ template <class C> BBS_HD void proof_gen_item(const ProofGenArgs& a, uint32_t i)
 
 #if defined(__CUDACC__) && !defined(BBS_HOSTSIM)
 // 3 * nb blocks: V1 for items [0, n), then F, then V2 (longest tasks first)
-template <class C, int TPB, int MINB> __global__ void __launch_bounds__(TPB, MINB)
+// PER_ITEM = false (no per-item headers or phs): the per-item reads are compiled out, as in sign_kernel
+template <class C, int TPB, int MINB, bool PER_ITEM> __global__ void __launch_bounds__(TPB, MINB)
 proof_g1_split_kernel(const ProofG1Args a, uint32_t n, uint32_t nb, uint8_t* fbad) {
     const uint32_t kind = blockIdx.x / nb;
     const uint32_t i = (blockIdx.x - kind * nb) * TPB + threadIdx.x;
     if (i >= n) return;
-    if (kind == 0) proof_task_v1<C>(a, i); else if (kind == 1) proof_task_f<C>(a, i, fbad + i); else proof_task_v2<C>(a, i);
+    if (kind == 0) proof_task_v1<C, PER_ITEM>(a, i); else if (kind == 1) proof_task_f<C, PER_ITEM>(a, i, fbad + i); else proof_task_v2<C, PER_ITEM>(a, i);
 }
-template <class C, int TPB> __global__ void __launch_bounds__(TPB, 4) proof_g1_join_kernel(const ProofG1Args a, uint32_t n, const uint8_t* fbad) {
+template <class C, int TPB, bool PER_ITEM> __global__ void __launch_bounds__(TPB, 4) proof_g1_join_kernel(const ProofG1Args a, uint32_t n,
+                                                                                            const uint8_t* fbad) {
     using F = typename C::Fp;
     __shared__ BBS_A16 uint32_t tree[2 * TPB][C::Fp::N];
     const uint32_t i = blockIdx.x * TPB + threadIdx.x;
     BBS_A16 uint32_t T1[G1J], T2[G1J], z[FPN];
     uint8_t st = 0;
-    const bool live = i < n && proof_join_head<C>(a, i, fbad, T1, T2, st);
+    const bool live = i < n && proof_join_head<C, PER_ITEM>(a, i, fbad, T1, T2, st);
     fe_set_one<F>(z);
     if (live) {
         if (!g1_is_inf_ool<C>(T1)) bn_copy<C::Fp::N>(z, T1 + 2 * FPN);
         if (!g1_is_inf_ool<C>(T2)) fe_mul<F>(z, z, T2 + 2 * FPN);
     }
     block_batch_inverse<F, TPB, true>(z, tree);
-    if (live) proof_join_tail<C>(a, i, T1, T2, z, st);
+    if (live) proof_join_tail<C, PER_ITEM>(a, i, T1, T2, z, st);
 }
 #endif
 

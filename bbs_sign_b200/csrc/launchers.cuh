@@ -19,6 +19,7 @@ template <class C> int launch_iss_decode(const IssDecodeArgs& a, uint32_t n, rt_
 template <class C> int launch_iss_domain(const IssDomainArgs& a, uint32_t n, rt_stream_t s);
 template <class C> int launch_iss_lines(const IssLinesArgs& a, uint32_t n, rt_stream_t s);
 template <class C> int launch_iss_lines_coop(const IssLinesCoopArgs& a, uint32_t n, rt_stream_t s);
+template <class C> int launch_item_domain(const ItemDomainArgs& a, uint32_t n, rt_stream_t s);
 int launch_gen_seed(const GenSeedArgs& a, rt_stream_t s);
 template <class C> int launch_gen_point(const GenPointArgs& a, uint32_t n, rt_stream_t s);
 template <class C> int launch_h2s(const H2sArgs& a, uint32_t n, rt_stream_t s);
@@ -38,8 +39,10 @@ template <class C> int launch_pairing_coop(const CoopArgs& a, rt_stream_t s);
 template <class C> size_t coop_gscratch_size(size_t n);
 #endif
 template <class C> int launch_sign(const SignArgs& a, uint32_t n, rt_stream_t s);
+template <class C> int launch_sign_per_item(const SignArgs& a, uint32_t n, rt_stream_t s);
 template <class C> int launch_proof_g1(const ProofG1Args& a, uint32_t n, rt_stream_t s);
 template <class C> int launch_proof_gen(const ProofGenArgs& a, uint32_t n, rt_stream_t s);
+template <class C> int launch_proof_gen_per_item(const ProofGenArgs& a, uint32_t n, rt_stream_t s);
 template <class C> int launch_field_test(const FieldTestArgs& a, uint32_t n, rt_stream_t s);
 template <class C> int launch_g1_mul_test(const G1MulTestArgs& a, uint32_t n, rt_stream_t s);
 template <class C> int launch_pair_test_prep(const PairTestPrepArgs& a, uint32_t n, rt_stream_t s);

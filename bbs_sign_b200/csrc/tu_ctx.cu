@@ -54,8 +54,20 @@ template <class C> int launch_iss_lines(const IssLinesArgs& a, uint32_t n, rt_st
 template <class C> int launch_iss_lines_coop(const IssLinesCoopArgs& a, uint32_t n, rt_stream_t s) {
     return rt_launch<IssLinesCoopArgs, &iss_lines_coop_item<C>, 64>(a, n, s);
 }
+// per-item headers (kernels.cuh item_domain_kernel): one thread per item
+template <class C> int launch_item_domain(const ItemDomainArgs& a, uint32_t n, rt_stream_t s) {
+#ifdef BBS_HOSTSIM
+    return rt_launch<ItemDomainArgs, &item_domain_item<C>, 128>(a, n, s);
+#else
+    if (n == 0) return 0;
+    item_domain_kernel<C, 128><<<(n + 127) / 128, 128, 0, s>>>(a, n);
+    RT_CHECK(cudaGetLastError());
+    return 0;
+#endif
+}
 
 #if defined(BBS_TU_BLS) || !defined(BBS_TU_BN)
+template int launch_item_domain<Bls>(const ItemDomainArgs&, uint32_t, rt_stream_t);
 template int launch_ctx_lines_coop<Bls>(const CtxLinesCoopArgs&, uint32_t, rt_stream_t);
 template int launch_iss_decode<Bls>(const IssDecodeArgs&, uint32_t, rt_stream_t);
 template int launch_iss_domain<Bls>(const IssDomainArgs&, uint32_t, rt_stream_t);
@@ -67,6 +79,7 @@ template int launch_ctx_table<Bls>(const CtxTableArgs&, uint32_t, rt_stream_t);
 template int launch_ctx_lines<Bls>(const CtxLinesArgs&, uint32_t, rt_stream_t);
 #endif
 #if defined(BBS_TU_BN) || !defined(BBS_TU_BLS)
+template int launch_item_domain<Bn>(const ItemDomainArgs&, uint32_t, rt_stream_t);
 template int launch_ctx_lines_coop<Bn>(const CtxLinesCoopArgs&, uint32_t, rt_stream_t);
 template int launch_iss_decode<Bn>(const IssDecodeArgs&, uint32_t, rt_stream_t);
 template int launch_iss_domain<Bn>(const IssDomainArgs&, uint32_t, rt_stream_t);

@@ -19,17 +19,23 @@ template <class C> int launch_proof_g1(const ProofG1Args& a, uint32_t n, rt_stre
         constexpr int TPB = BBS_PROOF_G1_TPB, MINB = BBS_PROOF_G1_MINB;
         const uint32_t nb = (n + TPB - 1) / TPB;
         uint8_t* fbad = a.part_st + n;
-        proof_g1_split_kernel<C, TPB, MINB><<<3 * nb, TPB, 0, s>>>(a, n, nb, fbad);
-        RT_CHECK(cudaGetLastError());
-        proof_g1_join_kernel<C, 128><<<(n + 127) / 128, 128, 0, s>>>(a, n, fbad);
+        if (a.item.K || a.ph_off) {
+            proof_g1_split_kernel<C, TPB, MINB, true><<<3 * nb, TPB, 0, s>>>(a, n, nb, fbad);
+            RT_CHECK(cudaGetLastError());
+            proof_g1_join_kernel<C, 128, true><<<(n + 127) / 128, 128, 0, s>>>(a, n, fbad);
+        } else {
+            proof_g1_split_kernel<C, TPB, MINB, false><<<3 * nb, TPB, 0, s>>>(a, n, nb, fbad);
+            RT_CHECK(cudaGetLastError());
+            proof_g1_join_kernel<C, 128, false><<<(n + 127) / 128, 128, 0, s>>>(a, n, fbad);
+        }
         RT_CHECK(cudaGetLastError());
         return 0;
     }
 #else
     if (a.part_t1) {                                    // the task functions of the split path, run in sequence
         uint8_t* fbad = a.part_st + n;
-        for (uint32_t i = 0; i < n; i++) { proof_task_v1<C>(a, i); proof_task_f<C>(a, i, fbad + i); proof_task_v2<C>(a, i); }
-        for (uint32_t i = 0; i < n; i++) proof_join_item<C>(a, i, fbad);
+        for (uint32_t i = 0; i < n; i++) { proof_task_v1<C, true>(a, i); proof_task_f<C, true>(a, i, fbad + i); proof_task_v2<C, true>(a, i); }
+        for (uint32_t i = 0; i < n; i++) proof_join_item<C, true>(a, i, fbad);
         return 0;
     }
 #endif
@@ -37,7 +43,8 @@ template <class C> int launch_proof_g1(const ProofG1Args& a, uint32_t n, rt_stre
 }
 
 template <class C> int launch_proof_gen(const ProofGenArgs& a, uint32_t n, rt_stream_t s) {
-    return rt_launch<ProofGenArgs, &proof_gen_item<C>, BBS_PROOF_G1_TPB, BBS_PROOF_G1_MINB>(a, n, s);
+    if (a.item.K || a.ph_off) return launch_proof_gen_per_item<C>(a, n, s);     // tu_proofitem.cu
+    return rt_launch<ProofGenArgs, &proof_gen_item<C, false>, BBS_PROOF_G1_TPB, BBS_PROOF_G1_MINB>(a, n, s);
 }
 
 #if defined(BBS_TU_BLS) || !defined(BBS_TU_BN)

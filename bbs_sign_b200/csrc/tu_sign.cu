@@ -18,7 +18,8 @@ template <class C> int launch_sign(const SignArgs& a, uint32_t n, rt_stream_t s)
     return rt_launch<SignArgs, &sign_item<C>, BBS_SIGN_TPB, BBS_SIGN_MINB>(a, n, s);
 #else
     if (n == 0) return 0;
-    sign_kernel<C, BBS_SIGN_TPB, BBS_SIGN_MINB><<<(n + BBS_SIGN_TPB - 1) / BBS_SIGN_TPB, BBS_SIGN_TPB, 0, s>>>(a, n);
+    if (a.item.K) return launch_sign_per_item<C>(a, n, s);        // tu_signitem.cu
+    sign_kernel<C, BBS_SIGN_TPB, BBS_SIGN_MINB, false><<<(n + BBS_SIGN_TPB - 1) / BBS_SIGN_TPB, BBS_SIGN_TPB, 0, s>>>(a, n);
     RT_CHECK(cudaGetLastError());
     return 0;
 #endif

@@ -9,7 +9,7 @@ from typing import List, Optional, Sequence, Tuple
 
 import numpy as np
 
-from .api import BatchContext, Ciphersuite, IssuerSet
+from .api import BatchContext, Ciphersuite, IssuerSet, _is_per_item
 
 
 def shard_bounds(n: int, world: int) -> List[Tuple[int, int]]:
@@ -18,14 +18,17 @@ def shard_bounds(n: int, world: int) -> List[Tuple[int, int]]:
 
 
 class ShardedVerifier:
-    """`verify_batch` over several GPUs of one box (one BatchContext per device)."""
+    """`verify_batch` over several GPUs of one box (one BatchContext per device).  `per_item_headers=True` builds contexts
+    that also take one header per item (`headers=`)."""
 
     def __init__(self, suite: Ciphersuite, pk: bytes, header: bytes, n_messages: int, devices: Sequence[int],
-                 lib_path: Optional[str] = None):
+                 lib_path: Optional[str] = None, per_item_headers: bool = False):
         self.suite = suite
-        self.ctxs = [BatchContext(suite, pk, header, n_messages, device=d, lib_path=lib_path) for d in devices]
+        self.ctxs = [BatchContext(suite, pk, header, n_messages, device=d, lib_path=lib_path, per_item_headers=per_item_headers)
+                     for d in devices]
 
-    def verify_batch(self, signatures, messages: Sequence[Sequence[bytes]]) -> np.ndarray:
+    def verify_batch(self, signatures, messages: Sequence[Sequence[bytes]], *,
+                     headers: Optional[Sequence[bytes]] = None) -> np.ndarray:
         sigs = np.frombuffer(signatures, dtype=np.uint8) if not isinstance(signatures, np.ndarray) else signatures.reshape(-1)
         sb = self.suite.signature_bytes
         n = sigs.size // sb
@@ -35,7 +38,8 @@ class ShardedVerifier:
         def work(ctx, lo, hi):
             try:
                 if hi > lo:
-                    out[lo:hi] = ctx.verify_batch(sigs[lo * sb: hi * sb], messages[lo:hi])
+                    out[lo:hi] = ctx.verify_batch(sigs[lo * sb: hi * sb], messages[lo:hi],
+                                                  headers=None if headers is None else headers[lo:hi])
             except Exception as e:  # pragma: no cover
                 errs.append(e)
 
@@ -67,13 +71,17 @@ class ShardedVerifier:
         if errs:
             raise errs[0]
 
-    def proof_verify_batch(self, proofs, ph: bytes, disclosed_messages, disclosed_indexes) -> np.ndarray:
-        """`proof_verify_batch` split by proof index (same contract as BatchContext.proof_verify_batch)."""
+    def proof_verify_batch(self, proofs, ph, disclosed_messages, disclosed_indexes, *,
+                           headers: Optional[Sequence[bytes]] = None) -> np.ndarray:
+        """`proof_verify_batch` split by proof index (same contract as BatchContext.proof_verify_batch: `ph` shared or
+        one per proof, `headers` one per proof)."""
         n = len(proofs)
         out = np.full(n, 255, dtype=np.uint8)
+        per_item_ph = _is_per_item(ph)
 
         def work(ctx, g, lo, hi):
-            out[lo:hi] = ctx.proof_verify_batch(proofs[lo:hi], ph, disclosed_messages[lo:hi], disclosed_indexes[lo:hi])
+            out[lo:hi] = ctx.proof_verify_batch(proofs[lo:hi], ph[lo:hi] if per_item_ph else ph, disclosed_messages[lo:hi],
+                                                disclosed_indexes[lo:hi], headers=None if headers is None else headers[lo:hi])
 
         self._run_sharded(n, work)
         return out

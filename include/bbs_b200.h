@@ -15,7 +15,8 @@
  *   Proof fixed : comp(Abar) || comp(Bbar) || comp(D) || LE32(e^) || LE32(r1^) || LE32(r3^) || LE32(c)
  *                 (the fixed-size fields of src/proof_gen.rs:29-39; commitments travel separately)
  *
- * Threading: one context per (GPU, issuer key, header, L).  A context is SINGLE-STREAM: every call on it (host-buffer or
+ * Threading: one context per (GPU, issuer key, header, L), or per (GPU, issuer key, L) for the *_hdr calls, which take a header
+ * per item on a context created with BBS_CTX_PER_ITEM_HEADER.  A context is SINGLE-STREAM: every call on it (host-buffer or
  * *_dev) shares the context's grow-only device scratch, so calls on one context must be serialized by the caller and
  * consecutive *_dev calls on one context must use the same stream (or be ordered by the caller's events).  Different
  * contexts are independent (one host thread per GPU for multi-GPU sharding).
@@ -104,8 +105,14 @@ int bbs_ctx_create(int curve_id, int device, const uint8_t* pk, const uint8_t* g
  *   BBS_CTX_SMALL_TABLES  8-bit windows instead of 16-bit: 390 KB (BLS12-381) / 260 KB (BN254) of table per generator instead of
  *                         50 / 34 MB -- the whole table set stays resident in L2, the context is built ~100x faster and
  *                         thousands of (key, header, L) contexts fit in HBM -- for twice the fixed-base additions per item
- *                         (the G1 kernels run ~1.5x longer; results are identical). */
+ *                         (the G1 kernels run ~1.5x longer; results are identical).
+ *   BBS_CTX_PER_ITEM_HEADER  the context can also serve the *_hdr calls (a header per item, below): it adds a window table for
+ *                         Q1 in generator slot L + 1 (+50 MB on BLS12-381, +34 MB on BN254; ~390 / 260 KB with small tables)
+ *                         and keeps the SHA-256 state of calculate_domain after its header-independent prefix.  The
+ *                         context's own header, domain and K are built as without the flag and serve every other call.
+ * The two flags may be combined. */
 #define BBS_CTX_SMALL_TABLES 1u
+#define BBS_CTX_PER_ITEM_HEADER 2u
 int bbs_ctx_create_ex(int curve_id, int device, uint32_t flags, const uint8_t* pk, const uint8_t* generators,
                       uint32_t n_generators, const uint8_t* header, size_t header_len, const uint8_t* api_id,
                       size_t api_id_len, bbs_ctx** out);
@@ -183,6 +190,48 @@ int bbs_proof_gen_batch(bbs_ctx* ctx, size_t n, const uint8_t* sigs, const uint8
                         const uint8_t* random_scalars, const uint64_t* rand_off, const uint64_t* commit_off,
                         const uint8_t* ph, size_t ph_len, uint8_t* proofs_fixed_out, uint8_t* commitments_out,
                         uint8_t* status);
+
+/* ---- per-item headers and presentation headers -----------------------------------------------------------------
+ * In the reference `header` and `ph` are arguments of every call (src/verify.rs:18-30, src/sign.rs:32-43,
+ * src/proof_verify.rs:19-34); these calls take them per item.  Item i's result is the reference's for header_i / ph_i;
+ * statuses are those of the calls without _hdr.
+ *   headers, hdr_off : header i = headers[hdr_off[i] .. hdr_off[i+1]), n + 1 offsets.  The verify and sign calls require
+ *                      them and a context created with BBS_CTX_PER_ITEM_HEADER (else BBS_E_ARG); the proof calls accept
+ *                      NULL for both, meaning the context's header for every item, and then work on any context.
+ *   phs, ph_off      : the proof calls' presentation headers, ph i = phs[ph_off[i] .. ph_off[i+1]) (required).
+ * Offsets must not decrease and every header / ph must be shorter than 2^28 bytes (BBS_E_ARG).  Per item the library hashes
+ * calculate_domain from the context's stored prefix state and computes K_i = P1 + Q1 * domain_i (one extra kernel,
+ * profiled in the slot after the call's others).  Per-item-header proof verification always takes the task-split G1 path
+ * (as issuer sets do).  These calls never take the chunked pipelines of large host-buffer batches: any size runs in one
+ * shot, with the same results. */
+int bbs_core_verify_batch_hdr(bbs_ctx* ctx, size_t n, const uint8_t* sigs, const uint8_t* msg_scalars, uint32_t n_msgs,
+                              const uint8_t* headers, const uint64_t* hdr_off, uint8_t* status);
+int bbs_verify_batch_hdr(bbs_ctx* ctx, size_t n, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* offsets,
+                         uint32_t n_msgs, const uint8_t* headers, const uint64_t* hdr_off, uint8_t* status);
+int bbs_core_sign_batch_hdr(bbs_ctx* ctx, const uint8_t sk_le32[32], size_t n, const uint8_t* msg_scalars, uint32_t n_msgs,
+                            const uint8_t* headers, const uint64_t* hdr_off, uint8_t* sigs_out, uint8_t* b_out,
+                            uint8_t* status);
+int bbs_sign_batch_hdr(bbs_ctx* ctx, const uint8_t sk_le32[32], size_t n, const uint8_t* msgs, const uint64_t* offsets,
+                       uint32_t n_msgs, const uint8_t* headers, const uint64_t* hdr_off, uint8_t* sigs_out, uint8_t* b_out,
+                       uint8_t* status);
+int bbs_core_proof_verify_batch_hdr(bbs_ctx* ctx, size_t n, const uint8_t* proofs_fixed, const uint8_t* commitments,
+                                    const uint64_t* commit_off, const uint32_t* disclosed_idx,
+                                    const uint8_t* disclosed_scalars, const uint64_t* dis_off, const uint8_t* headers,
+                                    const uint64_t* hdr_off, const uint8_t* phs, const uint64_t* ph_off, uint8_t* status);
+int bbs_proof_verify_batch_hdr(bbs_ctx* ctx, size_t n, const uint8_t* proofs_fixed, const uint8_t* commitments,
+                               const uint64_t* commit_off, const uint32_t* disclosed_idx, const uint8_t* dis_msgs,
+                               const uint64_t* dis_msg_off, const uint64_t* dis_off, const uint8_t* headers,
+                               const uint64_t* hdr_off, const uint8_t* phs, const uint64_t* ph_off, uint8_t* status);
+int bbs_core_proof_gen_batch_hdr(bbs_ctx* ctx, size_t n, const uint8_t* sigs, const uint8_t* msg_scalars, uint32_t n_msgs,
+                                 const uint32_t* disclosed_idx, const uint64_t* dis_off, const uint8_t* random_scalars,
+                                 const uint64_t* rand_off, const uint64_t* commit_off, const uint8_t* headers,
+                                 const uint64_t* hdr_off, const uint8_t* phs, const uint64_t* ph_off,
+                                 uint8_t* proofs_fixed_out, uint8_t* commitments_out, uint8_t* status);
+int bbs_proof_gen_batch_hdr(bbs_ctx* ctx, size_t n, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* offsets,
+                            uint32_t n_msgs, const uint32_t* disclosed_idx, const uint64_t* dis_off,
+                            const uint8_t* random_scalars, const uint64_t* rand_off, const uint64_t* commit_off,
+                            const uint8_t* headers, const uint64_t* hdr_off, const uint8_t* phs, const uint64_t* ph_off,
+                            uint8_t* proofs_fixed_out, uint8_t* commitments_out, uint8_t* status);
 
 /* ---- multi-issuer batches ---------------------------------------------------------------------------------
  * In the reference the public key is `&self` of every call (src/verify.rs:18-30), so a stream of signatures may name a
@@ -263,6 +312,16 @@ int bbs_core_proof_verify_batch_dev(bbs_ctx* ctx, size_t n, const uint8_t* d_pro
                                     const uint64_t* d_dis_off, const uint8_t* d_ph, size_t ph_len,
                                     uint8_t* d_status, void* stream);
 
+/* Device-buffer forms of bbs_core_verify_batch_hdr / bbs_core_proof_verify_batch_hdr (offsets in device memory, not checked). */
+int bbs_core_verify_batch_hdr_dev(bbs_ctx* ctx, size_t n, const uint8_t* d_sigs, const uint8_t* d_msg_scalars,
+                                  uint32_t n_msgs, const uint8_t* d_headers, const uint64_t* d_hdr_off, uint8_t* d_status,
+                                  void* stream);
+int bbs_core_proof_verify_batch_hdr_dev(bbs_ctx* ctx, size_t n, const uint8_t* d_proofs_fixed,
+                                        const uint8_t* d_commitments, const uint64_t* d_commit_off,
+                                        const uint32_t* d_disclosed_idx, const uint8_t* d_disclosed_scalars,
+                                        const uint64_t* d_dis_off, const uint8_t* d_headers, const uint64_t* d_hdr_off,
+                                        const uint8_t* d_phs, const uint64_t* d_ph_off, uint8_t* d_status, void* stream);
+
 /* Number of kernels the library has launched on this context since creation (for bench accounting). */
 uint64_t bbs_ctx_launch_count(bbs_ctx* ctx);
 /* Device memory the context holds (tables, key state and the grow-only batch scratch), bytes. */
@@ -287,7 +346,8 @@ int bbs_ctx_set_pairing_split(bbs_ctx* ctx, size_t max_items);
 /* ---- measurement hooks ------------------------------------------------------------------------------
  * With profiling on, every *_dev batch call records CUDA events on its launching stream around each of its
  * kernels; bbs_ctx_kernel_times returns the durations (ms) of the last call in launch order:
- *   verify / proof verify: [msg_to_scalars (0 if absent), G1 kernel, pairing kernel];  sign: [h2s, sign]. */
+ *   verify / proof verify: [msg_to_scalars (0 if absent), G1 kernel, pairing kernel];  sign: [h2s, sign].
+ * The *_hdr calls with per-item headers append the per-item domain kernel: verify / proof verify slot 3, sign slot 2. */
 int bbs_ctx_set_profiling(bbs_ctx* ctx, int on);
 int bbs_ctx_kernel_times(bbs_ctx* ctx, float* ms, int n);
 /* Integer-multiply roofline probe: 8 independent multiply-accumulate chains per thread on every SM.

@@ -9,7 +9,7 @@
 // The recipe is the engine's own Makefile: one object per (kernel group, curve) so the compile is parallel.
 use std::{env, path::PathBuf, process::Command, thread};
 
-const GROUPS: [&str; 8] = ["ctx", "h2s", "verify", "pairing", "sign", "proof", "rlc", "selftest"];
+const GROUPS: [&str; 10] = ["ctx", "h2s", "verify", "pairing", "sign", "signitem", "proof", "proofitem", "rlc", "selftest"];
 
 fn nvcc(args: &[String]) {
     let nvcc = env::var("NVCC").unwrap_or_else(|_| "nvcc".into());

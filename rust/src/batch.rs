@@ -79,6 +79,29 @@ extern "C" {
                            disclosed_idx: *const u32, dis_off: *const u64, random_scalars: *const u8, rand_off: *const u64,
                            commit_off: *const u64, ph: *const u8, ph_len: usize, proofs_fixed_out: *mut u8,
                            commitments_out: *mut u8, status: *mut u8) -> i32;
+    fn bbs_core_verify_batch_hdr(ctx: *mut BbsCtx, n: usize, sigs: *const u8, msg_scalars: *const u8, n_msgs: u32, headers: *const u8,
+                                 hdr_off: *const u64, status: *mut u8) -> i32;
+    fn bbs_verify_batch_hdr(ctx: *mut BbsCtx, n: usize, sigs: *const u8, msgs: *const u8, offsets: *const u64, n_msgs: u32,
+                            headers: *const u8, hdr_off: *const u64, status: *mut u8) -> i32;
+    fn bbs_core_sign_batch_hdr(ctx: *mut BbsCtx, sk_le32: *const u8, n: usize, msg_scalars: *const u8, n_msgs: u32,
+                               headers: *const u8, hdr_off: *const u64, sigs_out: *mut u8, b_out: *mut u8, status: *mut u8) -> i32;
+    fn bbs_sign_batch_hdr(ctx: *mut BbsCtx, sk_le32: *const u8, n: usize, msgs: *const u8, offsets: *const u64, n_msgs: u32,
+                          headers: *const u8, hdr_off: *const u64, sigs_out: *mut u8, b_out: *mut u8, status: *mut u8) -> i32;
+    fn bbs_core_proof_verify_batch_hdr(ctx: *mut BbsCtx, n: usize, proofs_fixed: *const u8, commitments: *const u8,
+                                       commit_off: *const u64, disclosed_idx: *const u32, disclosed_scalars: *const u8,
+                                       dis_off: *const u64, headers: *const u8, hdr_off: *const u64, phs: *const u8,
+                                       ph_off: *const u64, status: *mut u8) -> i32;
+    fn bbs_proof_verify_batch_hdr(ctx: *mut BbsCtx, n: usize, proofs_fixed: *const u8, commitments: *const u8, commit_off: *const u64,
+                                  disclosed_idx: *const u32, dis_msgs: *const u8, dis_msg_off: *const u64, dis_off: *const u64,
+                                  headers: *const u8, hdr_off: *const u64, phs: *const u8, ph_off: *const u64, status: *mut u8) -> i32;
+    fn bbs_core_proof_gen_batch_hdr(ctx: *mut BbsCtx, n: usize, sigs: *const u8, msg_scalars: *const u8, n_msgs: u32,
+                                    disclosed_idx: *const u32, dis_off: *const u64, random_scalars: *const u8, rand_off: *const u64,
+                                    commit_off: *const u64, headers: *const u8, hdr_off: *const u64, phs: *const u8,
+                                    ph_off: *const u64, proofs_fixed_out: *mut u8, commitments_out: *mut u8, status: *mut u8) -> i32;
+    fn bbs_proof_gen_batch_hdr(ctx: *mut BbsCtx, n: usize, sigs: *const u8, msgs: *const u8, offsets: *const u64, n_msgs: u32,
+                               disclosed_idx: *const u32, dis_off: *const u64, random_scalars: *const u8, rand_off: *const u64,
+                               commit_off: *const u64, headers: *const u8, hdr_off: *const u64, phs: *const u8, ph_off: *const u64,
+                               proofs_fixed_out: *mut u8, commitments_out: *mut u8, status: *mut u8) -> i32;
     fn bbs_issuer_set_create(curve_id: i32, device: i32, n_issuers: usize, pks: *const u8, generators: *const u8,
                              n_generators: u32, header: *const u8, header_len: usize, api_id: *const u8, api_id_len: usize,
                              issuer_status: *mut u8, out: *mut *mut BbsIssuerSet) -> i32;
@@ -116,6 +139,12 @@ extern "C" {
                                        d_commit_off: *const u64, d_disclosed_idx: *const u32, d_disclosed_scalars: *const u8,
                                        d_dis_off: *const u64, d_ph: *const u8, ph_len: usize, d_status: *mut u8,
                                        stream: *mut c_void) -> i32;
+    fn bbs_core_verify_batch_hdr_dev(ctx: *mut BbsCtx, n: usize, d_sigs: *const u8, d_msg_scalars: *const u8, n_msgs: u32,
+                                     d_headers: *const u8, d_hdr_off: *const u64, d_status: *mut u8, stream: *mut c_void) -> i32;
+    fn bbs_core_proof_verify_batch_hdr_dev(ctx: *mut BbsCtx, n: usize, d_proofs_fixed: *const u8, d_commitments: *const u8,
+                                           d_commit_off: *const u64, d_disclosed_idx: *const u32, d_disclosed_scalars: *const u8,
+                                           d_dis_off: *const u64, d_headers: *const u8, d_hdr_off: *const u64, d_phs: *const u8,
+                                           d_ph_off: *const u64, d_status: *mut u8, stream: *mut c_void) -> i32;
     fn bbs_ctx_launch_count(ctx: *mut BbsCtx) -> u64;
     fn bbs_ctx_memory_bytes(ctx: *mut BbsCtx) -> u64;
     fn bbs_ctx_use_per_thread_pairing(ctx: *mut BbsCtx, on: i32) -> i32;
@@ -140,7 +169,8 @@ const ST_ERR_IDX_MSG_LEN: u8 = 4;
 const ST_ERR_MALFORMED: u8 = 5;
 const ST_ERR_DISCLOSED_LEN: u8 = 6;
 const ST_ERR_RANDOM_LEN: u8 = 7;
-/// `BBS_CTX_*` flags of `bbs_ctx_create`'s device argument are not used here; contexts use the default (large) tables.
+/// `BBS_CTX_PER_ITEM_HEADER`: the context also serves calls with a header per item (`PublicKey::batch_ctx_per_item_header`).
+const BBS_CTX_PER_ITEM_HEADER: u32 = 2;
 const BBS_OK: i32 = 0;
 
 /// The reference's curve / constants pairing as the ABI's `curve_id` (include/bbs_b200.h `BBS_CURVE_*`).
@@ -263,6 +293,28 @@ impl<E: Pairing> PublicKey<E> {
         Ok(BatchCtx { raw, curve_id: C::ID, l })
     }
 
+    /// A context for batches whose items carry their own header (`verify_batch_per_header`, `SecretKey::sign_batch_per_header`,
+    /// `proof_verify_batch_per_item`): one per (key, `l`, device) instead of one per header.  Costs one more window table
+    /// (Q1's) than `batch_ctx`.
+    pub fn batch_ctx_per_item_header<H, C>(&self, l: usize, device: i32) -> Result<BatchCtx, BatchError>
+    where
+        H: HashToG1<E>,
+        C: for<'a> Constants<'a, E> + CurveId,
+    {
+        let api_id = [C::CIPHERSUITE_ID, b"H2G_HM2S_"].concat();
+        let (mut pk, mut gens) = (Vec::new(), Vec::new());
+        ser(&self.pk, &mut pk);
+        for g in create_generators::<E, H>(l + 1, &api_id) {
+            ser(&g, &mut gens);
+        }
+        let mut raw = std::ptr::null_mut();
+        check(unsafe {
+            bbs_ctx_create_ex(C::ID, device, BBS_CTX_PER_ITEM_HEADER, pk.as_ptr(), gens.as_ptr(), (l + 1) as u32, std::ptr::null(), 0,
+                              api_id.as_ptr(), api_id.len(), &mut raw)
+        })?;
+        Ok(BatchCtx { raw, curve_id: C::ID, l })
+    }
+
     /// Batch form of `verify` (src/verify.rs:18-50): `result[i]` is what `self.verify(sigs[i], header, messages[i])` returns.
     /// Builds a context for the call; use `batch_ctx` + `verify_batch_with` to amortise it over many calls.
     pub fn verify_batch<F, H, C>(&self, sigs: &[Signature<E, F>], header: &[u8], messages: &[&[&[u8]]])
@@ -290,6 +342,39 @@ pub fn verify_batch_with<E: Pairing, F: Field>(ctx: &BatchCtx, sigs: &[Signature
     let (flat, offs) = pack(messages);
     let mut st = vec![0u8; sigs.len()];
     check(unsafe { bbs_verify_batch(ctx.raw, sigs.len(), sb.as_ptr(), flat.as_ptr(), offs.as_ptr(), l as u32, st.as_mut_ptr()) })?;
+    Ok(st.into_iter().map(signature_status).collect())
+}
+
+/// Flat bytes + u64 offsets for one byte string per item (headers, presentation headers).
+fn pack_items(items: &[&[u8]]) -> (Vec<u8>, Vec<u64>) {
+    let (mut flat, mut offs) = (Vec::new(), vec![0u64]);
+    for it in items {
+        flat.extend_from_slice(it);
+        offs.push(flat.len() as u64);
+    }
+    if flat.is_empty() {
+        flat.push(0);
+    }
+    (flat, offs)
+}
+
+/// `verify_batch_with` where item i has its own header: `result[i]` is what `pk.verify(sigs[i], headers[i], messages[i])`
+/// returns.  `ctx` comes from `PublicKey::batch_ctx_per_item_header`.
+pub fn verify_batch_per_header<E: Pairing, F: Field>(ctx: &BatchCtx, sigs: &[Signature<E, F>], headers: &[&[u8]],
+    messages: &[&[&[u8]]]) -> Result<Vec<Result<bool, ItemError<SignatureError>>>, BatchError> {
+    assert!(sigs.len() == messages.len() && headers.len() == sigs.len(), "one header and message list per signature");
+    let l = uniform_len(messages)?;
+    let mut sb = Vec::new();
+    for s in sigs {
+        ser(s, &mut sb);
+    }
+    let (flat, offs) = pack(messages);
+    let (hdr, hoff) = pack_items(headers);
+    let mut st = vec![0u8; sigs.len()];
+    check(unsafe {
+        bbs_verify_batch_hdr(ctx.raw, sigs.len(), sb.as_ptr(), flat.as_ptr(), offs.as_ptr(), l as u32, hdr.as_ptr(), hoff.as_ptr(),
+                             st.as_mut_ptr())
+    })?;
     Ok(st.into_iter().map(signature_status).collect())
 }
 
@@ -344,6 +429,36 @@ impl<F: Field + FromOkm<48, F>> SecretKey<F> {
             })
             .collect())
     }
+
+    /// `sign_batch` where item i has its own header: `result[i]` is what `self.sign(messages[i], headers[i])` returns.
+    /// `ctx` comes from `PublicKey::batch_ctx_per_item_header` of this key's public key.
+    pub fn sign_batch_per_header<E: Pairing<ScalarField = F>>(&self, ctx: &BatchCtx, headers: &[&[u8]], messages: &[&[&[u8]]])
+        -> Result<Vec<Result<Signature<E, F>, ItemError<SignatureError>>>, BatchError> {
+        let n = messages.len();
+        assert_eq!(headers.len(), n, "one header per message list");
+        let l = uniform_len(messages)?;
+        let mut sk = Vec::new();
+        ser(&self.sk, &mut sk);
+        let (flat, offs) = pack(messages);
+        let (hdr, hoff) = pack_items(headers);
+        let rec = unsafe { bbs_signature_bytes(ctx.curve_id) };
+        let (mut out, mut st) = (vec![0u8; n * rec], vec![0u8; n]);
+        let rc = unsafe {
+            bbs_sign_batch_hdr(ctx.raw, sk.as_ptr(), n, flat.as_ptr(), offs.as_ptr(), l as u32, hdr.as_ptr(), hoff.as_ptr(),
+                               out.as_mut_ptr(), std::ptr::null_mut(), st.as_mut_ptr())
+        };
+        for b in sk.iter_mut() {
+            unsafe { std::ptr::write_volatile(b, 0) };
+        }
+        check(rc)?;
+        Ok((0..n)
+            .map(|i| match st[i] {
+                ST_ACCEPT => Ok(Signature::deserialize_compressed(&out[i * rec..(i + 1) * rec]).expect("library output")),
+                ST_ERR_MSG_GEN_LEN => Err(ItemError::Reference(SignatureError::InvalidMessageAndGeneratorsLength)),
+                _ => Err(ItemError::Malformed),
+            })
+            .collect())
+    }
 }
 
 /// The ABI splits ark's serialisation of `Proof` (src/proof_gen.rs:29-39) into the fixed fields
@@ -379,10 +494,22 @@ pub fn proof_verify_batch<E: Pairing, F: Field>(ctx: &BatchCtx, proofs: &[Proof<
     proof_verify_on(ProofTarget::Ctx(ctx.raw), proofs, ph, disclosed_messages, disclosed_indexes)
 }
 
-/// Where a proof batch is verified: under the one key of a context, or under a key per proof of an issuer set.
+/// `proof_verify_batch` with a presentation header per proof and, optionally, a header per proof: `result[i]` is what
+/// `proof_verify(pk, proofs[i], headers[i], phs[i], ..)` returns.  `headers = None` means the context's header (any context);
+/// per-item headers need a context from `PublicKey::batch_ctx_per_item_header`.
+pub fn proof_verify_batch_per_item<E: Pairing, F: Field>(ctx: &BatchCtx, proofs: &[Proof<E, F>], headers: Option<&[&[u8]]>,
+    phs: &[&[u8]], disclosed_messages: &[&[&[u8]]], disclosed_indexes: &[&[usize]])
+    -> Result<Vec<Result<bool, ItemError<ProofGenError>>>, BatchError> {
+    assert!(phs.len() == proofs.len() && headers.map_or(true, |h| h.len() == proofs.len()), "one ph (and header) per proof");
+    proof_verify_on(ProofTarget::CtxPerItem(ctx.raw, headers, phs), proofs, &[], disclosed_messages, disclosed_indexes)
+}
+
+/// Where a proof batch is verified: under the one key of a context, under a key per proof of an issuer set, or under the
+/// key of a context with a ph (and header) per proof.
 enum ProofTarget<'a> {
     Ctx(*mut BbsCtx),
     Set(*mut BbsIssuerSet, &'a [u32]),
+    CtxPerItem(*mut BbsCtx, Option<&'a [&'a [u8]]>, &'a [&'a [u8]]),
 }
 
 fn proof_verify_on<E: Pairing, F: Field>(target: ProofTarget, proofs: &[Proof<E, F>], ph: &[u8],
@@ -436,6 +563,17 @@ fn proof_verify_on<E: Pairing, F: Field>(target: ProofTarget, proofs: &[Proof<E,
                     bbs_proof_verify_batch_multi(raw, keep.len(), iss.as_ptr(), fixed.as_ptr(), commits.as_ptr(), coff.as_ptr(),
                                                  idx.as_ptr(), flat.as_ptr(), moffs.as_ptr(), doff.as_ptr(), ph.as_ptr(), ph.len(),
                                                  st.as_mut_ptr())
+                }
+            }
+            ProofTarget::CtxPerItem(raw, headers, phs) => {
+                // the items kept for the call, with their own ph / header
+                let (p, poff) = pack_items(&keep.iter().map(|&i| phs[i]).collect::<Vec<_>>());
+                let hs = headers.map(|h| pack_items(&keep.iter().map(|&i| h[i]).collect::<Vec<_>>()));
+                let (hp, hoff) = hs.as_ref().map_or((std::ptr::null(), std::ptr::null()), |(h, o)| (h.as_ptr(), o.as_ptr()));
+                unsafe {
+                    bbs_proof_verify_batch_hdr(raw, keep.len(), fixed.as_ptr(), commits.as_ptr(), coff.as_ptr(), idx.as_ptr(),
+                                               flat.as_ptr(), moffs.as_ptr(), doff.as_ptr(), hp, hoff, p.as_ptr(), poff.as_ptr(),
+                                               st.as_mut_ptr())
                 }
             }
         })?;
@@ -611,5 +749,8 @@ fn _unused_bindings() {
         bbs_ctx_launch_count as usize, bbs_ctx_memory_bytes as usize, bbs_core_verify_batch_multi as usize, bbs_core_proof_verify_batch_multi as usize, bbs_ctx_use_per_thread_pairing as usize,
         bbs_ctx_set_rlc_windows as usize, bbs_ctx_set_g1_split as usize, bbs_ctx_set_pairing_split as usize, bbs_ctx_set_profiling as usize, bbs_ctx_kernel_times as usize, bbs_imad_peak as usize,
         bbs_selftest_field as usize, bbs_selftest_g1_mul as usize, bbs_selftest_pairing as usize,
+        bbs_core_verify_batch_hdr as usize, bbs_core_sign_batch_hdr as usize, bbs_core_proof_verify_batch_hdr as usize,
+        bbs_core_proof_gen_batch_hdr as usize, bbs_proof_gen_batch_hdr as usize, bbs_core_verify_batch_hdr_dev as usize,
+        bbs_core_proof_verify_batch_hdr_dev as usize,
     );
 }
