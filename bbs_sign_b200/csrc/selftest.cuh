@@ -5,32 +5,50 @@
 
 namespace bbs {
 
+// op: the operation (low byte; list at bbs_selftest_field) | FIELD_TEST_MONT.  With FIELD_TEST_MONT the operands are taken as
+// Montgomery words and the result is returned as one, so a chosen limb pattern reaches the multiplication chains as it is.
+constexpr int FIELD_TEST_MONT = 0x100;
+constexpr int FIELD_TEST_LAST_OP = 13;
+BBS_HD bool field_test_on_fp(int op) { return op <= 4 || op == 7 || op == 9 || op == 10; }
+
 struct FieldTestArgs { int op; const uint8_t* a; const uint8_t* b; uint8_t* out; };
+
+// the operations both kinds of field have; false if op is not one of them
+template <class F> BBS_HD bool field_test_common(int op, uint32_t* r, const uint32_t* a, const uint32_t* b) {
+    if (op == 0 || op == 5) fe_mul<F>(r, a, b);
+    else if (op == 1 || op == 11) fe_add<F>(r, a, b);
+    else if (op == 2 || op == 12) fe_sub<F>(r, a, b);
+    else if (op == 3 || op == 6) fe_inv<F>(r, a);
+    else if (op == 7 || op == 8) fe_inv_vt<F>(r, a);
+    else if (op == 10 || op == 13) fe_neg<F>(r, a);
+    else return false;
+    return true;
+}
 
 template <class C> BBS_HD void field_test_item(const FieldTestArgs& t, uint32_t i) {
     using Fp = typename C::Fp;
     using Fr = typename C::Fr;
-    if (t.op <= 4 || t.op == 7) {
+    const int op = t.op & 0xff;
+    const bool mont = (t.op & FIELD_TEST_MONT) != 0;
+    if (field_test_on_fp(op)) {
         constexpr int N = Fp::N;
         BBS_A16 uint32_t a[N], b[N], r[N];
         limbs_from_le<N>(a, t.a + (size_t)i * 4 * N);
         limbs_from_le<N>(b, t.b + (size_t)i * 4 * N);
-        fe_to_mont<Fp>(a, a); fe_to_mont<Fp>(b, b);
-        if (t.op == 0) fe_mul<Fp>(r, a, b);
-        else if (t.op == 1) fe_add<Fp>(r, a, b);
-        else if (t.op == 2) fe_sub<Fp>(r, a, b);
-        else if (t.op == 3) fe_inv<Fp>(r, a);
-        else if (t.op == 7) fe_inv_vt<Fp>(r, a);
-        else { if (!fe_sqrt<Fp>(r, a)) bn_zero<N>(r); }
-        fe_from_mont<Fp>(r, r);
+        if (!mont) { fe_to_mont<Fp>(a, a); fe_to_mont<Fp>(b, b); }
+        if (!field_test_common<Fp>(op, r, a, b)) {
+            if (op == 9) fe_sqr<Fp>(r, a);
+            else if (!fe_sqrt<Fp>(r, a)) bn_zero<N>(r);
+        }
+        if (!mont) fe_from_mont<Fp>(r, r);
         limbs_to_le<N>(t.out + (size_t)i * 4 * N, r);
     } else {
         BBS_A16 uint32_t a[8], b[8], r[8];
         limbs_from_le<8>(a, t.a + (size_t)i * 32);
         limbs_from_le<8>(b, t.b + (size_t)i * 32);
-        fe_to_mont<Fr>(a, a); fe_to_mont<Fr>(b, b);
-        if (t.op == 5) fe_mul<Fr>(r, a, b); else if (t.op == 6) fe_inv<Fr>(r, a); else fe_inv_vt<Fr>(r, a);
-        fe_from_mont<Fr>(r, r);
+        if (!mont) { fe_to_mont<Fr>(a, a); fe_to_mont<Fr>(b, b); }
+        field_test_common<Fr>(op, r, a, b);
+        if (!mont) fe_from_mont<Fr>(r, r);
         limbs_to_le<8>(t.out + (size_t)i * 32, r);
     }
 }

@@ -357,8 +357,13 @@ int bbs_imad_peak(int device, int iters, int mode, double* gprod_per_s, float* m
 
 /* ---- arithmetic self-test hooks (parity tests of the field / curve layers against the oracle) ------
  * op: 0 = Fp mul, 1 = Fp add, 2 = Fp sub, 3 = Fp inv, 4 = Fp sqrt (0 if none), 5 = Fr mul, 6 = Fr inv,
- *     7 = Fp inv / 8 = Fr inv by the variable-time binary Euclid used where one thread inverts public data.
- * a, b, out: n x field-size canonical little-endian values (48 / 32 bytes for Fp, 32 for Fr). */
+ *     7 = Fp inv / 8 = Fr inv by the variable-time binary Euclid used where one thread inverts public data,
+ *     9 = Fp square (fe_sqr: on the device the dedicated squaring of the base fields), 10 = Fp neg,
+ *     11 = Fr add, 12 = Fr sub, 13 = Fr neg.  Unary ops ignore b.
+ * op | 0x100: Montgomery-domain I/O.  a, b and out are the Montgomery words A, B, op(...)·R mod m themselves (no
+ *     conversion on the way in or out), so out = mont(op(A·R^-1, B·R^-1)) with R = 2^(32N).  Without the flag a chosen
+ *     value is multiplied by R before the operation and its limb pattern is lost.
+ * a, b, out: n x field-size little-endian values below the modulus (48 / 32 bytes for Fp, 32 for Fr). */
 int bbs_selftest_field(int curve_id, int device, int op, size_t n, const uint8_t* a, const uint8_t* b, uint8_t* out);
 /* out[i] = comp(k_i * P_i) for compressed G1 points and LE32 scalars. */
 int bbs_selftest_g1_mul(int curve_id, int device, size_t n, const uint8_t* points, const uint8_t* scalars,

@@ -166,14 +166,16 @@ def wmul_prog(n, odd, rows_per_stmt=2):
     return P, top
 
 
-def check_wmul(n, trials=300):
+def check_wmul(n, trials=300, operands=None):
+    """operands: (a, b) pairs of n-word values to run instead of the edge and random ones"""
     rnd = random.Random(100 + n)
     pe, te = wmul_prog(n, False)
     po, to = wmul_prog(n, True)
     assert te == 2 * n and to == 2 * n - 1, (te, to)
-    for t in range(trials):
-        a = [0, (1 << (32 * n)) - 1, 1][t] if t < 3 else rnd.getrandbits(32 * n)
-        b = [(1 << (32 * n)) - 1, (1 << (32 * n)) - 1, 0][t] if t < 3 else rnd.getrandbits(32 * n)
+    if operands is None:
+        operands = [([0, (1 << (32 * n)) - 1, 1][t], [(1 << (32 * n)) - 1, (1 << (32 * n)) - 1, 0][t]) if t < 3 else
+                    (rnd.getrandbits(32 * n), rnd.getrandbits(32 * n)) for t in range(trials)]
+    for t, (a, b) in enumerate(operands):
         env = {}
         for i in range(n):
             env[f"a{i}"], env[f"b{i}"] = limbs(a, n)[i], limbs(b, n)[i]
@@ -229,14 +231,16 @@ def merge_prog(n):
     return P
 
 
-def check_merge(n, trials=200):
+def check_merge(n, trials=200, operands=None):
+    """operands: (a, b) pairs of n-word values to run instead of the edge and random ones"""
     rnd = random.Random(300 + n)
     pe, _ = wmul_prog(n, False)
     po, _ = wmul_prog(n, True)
     pm = merge_prog(n)
-    for t in range(trials):
-        a = (1 << (32 * n)) - 1 if t == 0 else rnd.getrandbits(32 * n)
-        b = (1 << (32 * n)) - 1 if t == 0 else rnd.getrandbits(32 * n)
+    if operands is None:
+        top = (1 << (32 * n)) - 1
+        operands = [(top, top)] + [(rnd.getrandbits(32 * n), rnd.getrandbits(32 * n)) for _ in range(trials - 1)]
+    for a, b in operands:
         env = {}
         for i in range(n):
             env[f"a{i}"], env[f"b{i}"] = limbs(a, n)[i], limbs(b, n)[i]
@@ -350,14 +354,17 @@ def redc_wide_prog(n, p):
     return P
 
 
-def check_redc_wide(n, p, limit_p2, trials=300):
+def check_redc_wide(n, p, limit_p2, trials=300, operands=None):
+    """operands: accumulators 0 <= T < limit_p2 p^2 to run instead of the edge and random ones"""
     R = 1 << (32 * n)
     rnd = random.Random(900 + n)
     P = redc_wide_prog(n, p)
     lim = limit_p2 * p * p
     assert lim < 1 << (32 * (2 * n + 1))
-    for t in range(trials):
-        T = [0, lim - 1, R - 1, p * p * 12][t] if t < 4 else rnd.randrange(lim)
+    if operands is None:
+        operands = [0, lim - 1, R - 1, p * p * 12] + [rnd.randrange(lim) for _ in range(trials - 4)]
+    for t, T in enumerate(operands):
+        assert 0 <= T < lim
         env = {"m": 0}
         for i in range(2 * n + 1):
             env[f"t{i}"] = limbs(T, 2 * n + 1)[i]
@@ -366,43 +373,54 @@ def check_redc_wide(n, p, limit_p2, trials=300):
         assert (r * R - T) % p == 0 and r < T // R + p + 1, (n, t)
 
 
-def check_canon_q(p, trials=200000):
-    """pairing_coop.cuh Coop<Bn>::canon_q: the quotient estimate from the top 29 bits is q or q - 1 for every w < 128 p"""
+def check_canon_q(p, trials=200000, operands=None):
+    """pairing_coop.cuh Coop<Bn>::canon_q: the quotient estimate from the top 29 bits is q or q - 1 for every w < 128 p.
+    operands: values w to run instead of the edge and random ones"""
     M = (1 << 32) // ((p >> 232) + 1)
     assert M == 1354
     rnd = random.Random(77)
-    cases = [k * p + d for k in range(128) for d in (-1, 0, 1, 1 << 200, -(1 << 200)) if 0 <= k * p + d < 128 * p]
-    cases += [rnd.randrange(128 * p) for _ in range(trials)]
+    cases = operands
+    if cases is None:
+        cases = [k * p + d for k in range(128) for d in (-1, 0, 1, 1 << 200, -(1 << 200)) if 0 <= k * p + d < 128 * p]
+        cases += [rnd.randrange(128 * p) for _ in range(trials)]
     for w in cases:
+        assert 0 <= w < 128 * p
         v = ((w >> 256) << 24) | (((w >> 224) & MASK) >> 8)
         assert v < 1 << 32
         q = (v * M) >> 32
         assert q in (w // p, w // p - 1), (w, q)
 
 
-def check_canon_q_bls(p, trials=200000):
+def check_canon_q_bls(p, trials=200000, operands=None):
     """pairing_coop.cuh Coop<Bls>::canon_q: for every 12-word w the estimate q^ = (w[11] * M) >> 56,
-    M = floor(2^56 / ((p >> 352) + 1)), is q or q - 1 with q = floor(w / p) < 10"""
+    M = floor(2^56 / ((p >> 352) + 1)), is q or q - 1 with q = floor(w / p) < 10.
+    operands: values w to run instead of the edge and random ones"""
     M = (1 << 56) // ((p >> 352) + 1)
     assert M == 165164498 and M < 1 << 32
     R = 1 << 384
     assert 9 * p < R < 10 * p
     rnd = random.Random(78)
-    cases = [k * p + d for k in range(11) for d in (-1, 0, 1, 1 << 352, -(1 << 352), (1 << 352) - 1) if 0 <= k * p + d < R]
-    cases += [R - 1, 0] + [rnd.randrange(R) for _ in range(trials)]
-    cases += [(v << 352) + d for v in (rnd.randrange(1 << 32) for _ in range(20000)) for d in (0, (1 << 352) - 1)]
+    cases = operands
+    if cases is None:
+        cases = [k * p + d for k in range(11) for d in (-1, 0, 1, 1 << 352, -(1 << 352), (1 << 352) - 1) if 0 <= k * p + d < R]
+        cases += [R - 1, 0] + [rnd.randrange(R) for _ in range(trials)]
+        cases += [(v << 352) + d for v in (rnd.randrange(1 << 32) for _ in range(20000)) for d in (0, (1 << 352) - 1)]
     for w in cases:
+        assert 0 <= w < R
         q = ((w >> 352) * M) >> 56
         assert q in (w // p, w // p - 1) and q < 10, (w, q)
 
 
-def check_redc(n, p, trials=300):
+def check_redc(n, p, trials=300, operands=None):
+    """operands: accumulators 0 <= T < (R - p) R to run instead of the edge and random ones"""
     R = 1 << (32 * n)
     rnd = random.Random(200 + n)
     P = redc_prog(n, p)
     lim = (R - p) * R
-    for t in range(trials):
-        T = [0, lim - 1, R - 1, p * p * 12][t] if t < 4 else rnd.randrange(lim)
+    if operands is None:
+        operands = [0, lim - 1, R - 1, p * p * 12] + [rnd.randrange(lim) for _ in range(trials - 4)]
+    for t, T in enumerate(operands):
+        assert 0 <= T < lim
         env = {"m": 0}
         for i in range(2 * n):
             env[f"t{i}"] = limbs(T, 2 * n)[i]

@@ -159,15 +159,17 @@ def mont_mul_prog(n, square=False):
     return P
 
 
-def check(n, p, trials=200):
+def check(n, p, trials=200, operands=None):
+    """operands: (a, b) pairs with a, b < p to run instead of the edge and random ones (the squaring takes each a once)"""
     R = 1 << (32 * n)
     inv = (-pow(p, -1, 1 << 32)) % (1 << 32)
     rnd = random.Random(n)
+    if operands is None:
+        operands = [([0, 1, p - 1, R % p][t], [p - 1, 0, p - 1, R % p][t]) if t < 4 else (rnd.randrange(p), rnd.randrange(p))
+                    for t in range(trials)]
     for square in (False, True):
         prog = mont_mul_prog(n, square)
-        for t in range(trials):
-            a = [0, 1, p - 1, R % p][t] if t < 4 else rnd.randrange(p)
-            b = a if square else ([p - 1, 0, p - 1, R % p][t] if t < 4 else rnd.randrange(p))
+        for t, (a, b) in enumerate(sorted({(a, a) for a, _ in operands}) if square else operands):
             env = {"inv": inv, "m": 0}
             for i in range(n):
                 env[f"a{i}"] = (a >> (32 * i)) & MASK

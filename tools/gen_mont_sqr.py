@@ -94,17 +94,20 @@ def env_for(a, n):
     return env
 
 
-def check(n, p, trials=400):
+def check(n, p, trials=400, operands=None):
+    """operands: values a < 2^(32n - 1) to run instead of the edge and random ones"""
     assert p < 1 << (32 * n - 1), "the doubled operand must fit in n limbs"
     R = 1 << (32 * n)
     rnd = random.Random(300 + n)
     W = sqr_wide_prog(n)
     M = merge_prog(n)
     Rd = redc_prog(n, p)
-    edge = [0, 1, p - 1, p - 2, R % p, (1 << (32 * n - 1)) - 1, int("5" * (8 * n), 16) % p, int("a" * (8 * n), 16) >> 1,
-            (1 << (32 * n - 1)) - (1 << 31), sum(0xffffffff << (64 * k) for k in range(n // 2)) >> 1]
-    for t in range(trials):
-        a = edge[t] if t < len(edge) else rnd.randrange(p)
+    if operands is None:
+        edge = [0, 1, p - 1, p - 2, R % p, (1 << (32 * n - 1)) - 1, int("5" * (8 * n), 16) % p, int("a" * (8 * n), 16) >> 1,
+                (1 << (32 * n - 1)) - (1 << 31), sum(0xffffffff << (64 * k) for k in range(n // 2)) >> 1]
+        operands = edge + [rnd.randrange(p) for _ in range(trials - len(edge))]
+    for t, a in enumerate(operands):
+        assert 0 <= a < 1 << (32 * n - 1)
         env = env_for(a, n)
         W.run(env)
         M.run(env)
