@@ -114,7 +114,15 @@ struct IssuerSet {
     DevBuf pks, W, K, domains, flags, lines, item_issuer;
     size_t per_issuer_bytes() const { return pks.cap + W.cap + K.cap + domains.cap + flags.cap + lines.cap; }
     void release_all() { for (DevBuf* b : {&pks, &W, &K, &domains, &flags, &lines, &item_issuer}) b->release(); }
+    IssuerSetView view() const {
+        return IssuerSetView{(const uint32_t*)K.p, (const uint32_t*)flags.p, (const uint32_t*)lines.p, line_stride,
+                             (uint32_t)n_issuers, (const uint32_t*)domains.p};
+    }
 };
+
+// The messages of a host-buffer batch call: byte messages `msgs` with their count + 1 offsets `off`, or (off == nullptr)
+// their scalars, 32 bytes each
+struct MsgIn { const uint8_t* scalars; const uint8_t* msgs; const uint64_t* off; };
 
 #define TRY(expr) do { int rc_ = (expr); if (rc_) return rc_; } while (0)
 #define PROF(c, slot, s) do { if ((c)->profile) TRY((c)->prof.mark(slot, s)); } while (0)
@@ -289,8 +297,7 @@ struct Impl {
         }
         if (S) {
             a.item_issuer = (const uint32_t*)S->item_issuer.p + first;
-            a.iss = IssuerSetView{(const uint32_t*)S->K.p, (const uint32_t*)S->flags.p, (const uint32_t*)S->lines.p,
-                                  S->line_stride, (uint32_t)S->n_issuers, (const uint32_t*)S->domains.p};
+            a.iss = S->view();
         }
         if (item) a.item = ItemKeyView{item->K + first * 2 * C::Fp::N, item->domains + first * 8, item->flags + first};
         TRY((launch_verify_g1<C>(a, (uint32_t)n, s)));
@@ -332,81 +339,69 @@ struct Impl {
         TRY(stage(c->s_hdr_off, hdr_off, (n + 1) * 8, c->stream));
         return item_keys_dev(c, n, (const uint8_t*)c->s_hdr.p, (const uint64_t*)c->s_hdr_off.p, item, c->stream);
     }
-    // verify / core_verify with a header per item (msgs == nullptr: `scalars` holds the message scalars).  Always one shot:
-    // batches large enough for verify_chunked are not split into chunks here.
-    static int verify_hdr(Ctx* c, size_t n, const uint8_t* sigs, const uint8_t* scalars, const uint8_t* msgs, const uint64_t* off,
-                          uint32_t n_msgs, const uint8_t* headers, const uint64_t* hdr_off, uint8_t* status) {
-        rt_stream_t s = c->stream;
-        const size_t count = n * n_msgs;
-        ItemKeyView item{};
-        TRY(item_keys(c, n, headers, hdr_off, item));
-        TRY(stage(c->s_sigs, sigs, n * SIG, s));
-        TRY(c->s_status.reserve(n));
-        if (off) {
-            TRY(stage(c->s_msgs, msgs, off[count], s));
-            TRY(stage(c->s_offsets, off, (count + 1) * 8, s));
-            TRY(c->s_scalars.reserve(count * 32));
-            PROF(c, 0, s);
-            TRY(h2s_dev(c, count, (const uint8_t*)c->s_msgs.p, (const uint64_t*)c->s_offsets.p, (uint8_t*)c->s_scalars.p, s));
-        } else {
-            TRY(stage(c->s_scalars, scalars, count * 32, s));
-        }
-        TRY(core_verify_dev(c, n, (const uint8_t*)c->s_sigs.p, (const uint8_t*)c->s_scalars.p, n_msgs, (uint8_t*)c->s_status.p,
-                            s, nullptr, &item));
-        return finish_status(c, n, status);
-    }
     static int core_verify_hdr_dev(Ctx* c, size_t n, const uint8_t* d_sigs, const uint8_t* d_scalars, uint32_t n_msgs,
                                    const uint8_t* d_headers, const uint64_t* d_hdr_off, uint8_t* d_status, rt_stream_t s) {
         ItemKeyView item{};
         TRY(item_keys_dev(c, n, d_headers, d_hdr_off, item, s));
         return core_verify_dev(c, n, d_sigs, d_scalars, n_msgs, d_status, s, nullptr, &item);
     }
-    // sign / core_sign with a header per item (one shot, like verify_hdr)
-    static int sign_hdr(Ctx* c, const uint8_t* sk, size_t n, const uint8_t* scalars, const uint8_t* msgs, const uint64_t* off,
-                        uint32_t n_msgs, const uint8_t* headers, const uint64_t* hdr_off, uint8_t* sigs_out, uint8_t* b_out,
-                        uint8_t* status) {
-        rt_stream_t s = c->stream;
-        const size_t count = n * n_msgs;
-        ItemKeyView item{};
-        TRY(item_keys(c, n, headers, hdr_off, item));
-        if (off) {
-            TRY(stage(c->s_msgs, msgs, off[count], s));
-            TRY(stage(c->s_offsets, off, (count + 1) * 8, s));
-            TRY(c->s_scalars.reserve(count * 32));
-            PROF(c, 0, s);
-            TRY(h2s_dev(c, count, (const uint8_t*)c->s_msgs.p, (const uint64_t*)c->s_offsets.p, (uint8_t*)c->s_scalars.p, s));
-        } else {
-            TRY(stage(c->s_scalars, scalars, count * 32, s));
-        }
-        return sign_common(c, sk, n, n_msgs, sigs_out, b_out, status, &item);
-    }
 #ifndef BBS_HOSTSIM
+    // ---- chunked host-buffer pipelines (verify, sign, rlc) ----------------------------------------------------------
+    // Bounds of up to 8 chunks covering [0, n): chunks of `first` items, or (doubling) of sizes doubling from `first`, where
+    // a remainder below `first` and everything past the 8th chunk joins the last chunk.  Returns the number of chunks.
+    static int plan_chunks(size_t n, size_t first, bool doubling, size_t bounds[9]) {
+        int k = 0;
+        bounds[0] = 0;
+        for (size_t at = 0, cur = first; at < n; cur = doubling ? 2 * cur : cur) {
+            size_t take = std::min(n - at, cur);
+            if (doubling && (n - at - take < first || k == 7)) take = n - at;
+            at += take;
+            bounds[++k] = at;
+        }
+        return k;
+    }
+    // Queues the uploads of every chunk on the copy stream, with event copy_done[k] after chunk k: the signatures (unless
+    // sigs == nullptr) into s_sigs, and the byte messages and offsets into s_msgs / s_offsets or the scalars into
+    // s_scalars.  The copy stream first waits for everything already queued on the compute stream, so that no buffer of a
+    // previous call is overwritten early.
+    static int upload_chunks(Ctx* c, size_t n, int n_chunks, const size_t* bounds, const uint8_t* sigs, const MsgIn& in,
+                             uint32_t n_msgs, rt_stream_t s) {
+        const size_t count = n * n_msgs;
+        if (sigs) TRY(c->s_sigs.reserve(n * SIG));
+        TRY(c->s_scalars.reserve(count * 32));
+        if (in.off) {
+            TRY(c->s_msgs.reserve(in.off[count]));
+            TRY(c->s_offsets.reserve((count + 1) * 8));
+        }
+        if (!c->copy_stream) RT_CHECK(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
+        if (!c->copy_done[0]) for (auto& e : c->copy_done) RT_CHECK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+        RT_CHECK(cudaEventRecord(c->copy_done[7], s));
+        RT_CHECK(cudaStreamWaitEvent(c->copy_stream, c->copy_done[7], 0));
+        for (int k = 0; k < n_chunks; k++) {
+            const size_t i0 = bounds[k], i1 = bounds[k + 1], m0 = i0 * n_msgs, m1 = i1 * n_msgs;
+            if (sigs) TRY(rt_h2d((uint8_t*)c->s_sigs.p + i0 * SIG, sigs + i0 * SIG, (i1 - i0) * SIG, c->copy_stream));
+            if (in.off) {
+                TRY(rt_h2d((uint8_t*)c->s_msgs.p + in.off[m0], in.msgs + in.off[m0], in.off[m1] - in.off[m0], c->copy_stream));
+                TRY(rt_h2d((uint64_t*)c->s_offsets.p + m0, in.off + m0, (m1 - m0 + 1) * 8, c->copy_stream));
+            } else {
+                TRY(rt_h2d((uint8_t*)c->s_scalars.p + m0 * 32, in.scalars + m0 * 32, (m1 - m0) * 32, c->copy_stream));
+            }
+            RT_CHECK(cudaEventRecord(c->copy_done[k], c->copy_stream));
+        }
+        return BBS_OK;
+    }
+
     // Host buffers of a LARGE verify batch (>= 2 * VERIFY_CHUNK items) in up to 8 chunks of doubling size: all uploads are
     // queued on the copy stream with one event per chunk; the compute stream hashes (byte messages) and runs the G1 half of
     // chunk k while chunk k + 1 is in flight; ONE pairing launch over the whole batch follows (it is 3/4 of the work and
     // loses nothing to chunking that way).  Statuses are those of the one-shot path: the items are independent.
     static constexpr size_t VERIFY_CHUNK = 131072;
-    static int verify_chunked(Ctx* c, size_t n, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* off, const uint8_t* scalars,
-                              uint32_t n_msgs, uint8_t* status) {
+    static int verify_chunked(Ctx* c, size_t n, const uint8_t* sigs, const MsgIn& in, uint32_t n_msgs, uint8_t* status) {
         rt_stream_t s = c->stream;
-        const size_t count = n * n_msgs;
         size_t bounds[9];
-        int n_chunks = 0;
+        const int n_chunks = plan_chunks(n, VERIFY_CHUNK, true, bounds);
         size_t largest = 0;
-        bounds[0] = 0;
-        for (size_t at = 0, cur = VERIFY_CHUNK; at < n; cur *= 2) {
-            size_t take = std::min(n - at, cur);
-            if (n - at - take < VERIFY_CHUNK || n_chunks == 7) take = n - at;
-            largest = std::max(largest, take);
-            at += take;
-            bounds[++n_chunks] = at;
-        }
-        TRY(c->s_sigs.reserve(n * SIG));
-        TRY(c->s_scalars.reserve(count * 32));
-        if (msgs) {
-            TRY(c->s_msgs.reserve(off[count]));
-            TRY(c->s_offsets.reserve((count + 1) * 8));
-        }
+        for (int k = 0; k < n_chunks; k++) largest = std::max(largest, bounds[k + 1] - bounds[k]);
         TRY(c->s_status.reserve(n));
         TRY(c->s_pair.reserve(n * 6 * C::Fp::N * 4));
         TRY(c->s_flags.reserve(n * 4));
@@ -415,27 +410,13 @@ struct Impl {
             TRY(c->s_g1f.reserve(largest * 3 * C::Fp::N * 4));
             TRY(c->s_g1st.reserve(2 * largest));
         }
-        if (!c->copy_stream) RT_CHECK(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
-        if (!c->copy_done[0]) for (auto& e : c->copy_done) RT_CHECK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        RT_CHECK(cudaEventRecord(c->copy_done[7], s));
-        RT_CHECK(cudaStreamWaitEvent(c->copy_stream, c->copy_done[7], 0));
-        for (int k = 0; k < n_chunks; k++) {
-            const size_t i0 = bounds[k], i1 = bounds[k + 1], m0 = i0 * n_msgs, m1 = i1 * n_msgs;
-            TRY(rt_h2d((uint8_t*)c->s_sigs.p + i0 * SIG, sigs + i0 * SIG, (i1 - i0) * SIG, c->copy_stream));
-            if (msgs) {
-                TRY(rt_h2d((uint8_t*)c->s_msgs.p + off[m0], msgs + off[m0], off[m1] - off[m0], c->copy_stream));
-                TRY(rt_h2d((uint64_t*)c->s_offsets.p + m0, off + m0, (m1 - m0 + 1) * 8, c->copy_stream));
-            } else {
-                TRY(rt_h2d((uint8_t*)c->s_scalars.p + m0 * 32, scalars + m0 * 32, (m1 - m0) * 32, c->copy_stream));
-            }
-            RT_CHECK(cudaEventRecord(c->copy_done[k], c->copy_stream));
-        }
+        TRY(upload_chunks(c, n, n_chunks, bounds, sigs, in, n_msgs, s));
         int rc = BBS_OK;
         for (int k = 0; k < n_chunks && !rc; k++) {
             const size_t i0 = bounds[k], i1 = bounds[k + 1], m0 = i0 * n_msgs, m1 = i1 * n_msgs;
             RT_CHECK(cudaStreamWaitEvent(s, c->copy_done[k], 0));
-            if (msgs) rc = h2s_dev(c, m1 - m0, (const uint8_t*)c->s_msgs.p, (const uint64_t*)c->s_offsets.p + m0,
-                                   (uint8_t*)c->s_scalars.p + m0 * 32, s);
+            if (in.off) rc = h2s_dev(c, m1 - m0, (const uint8_t*)c->s_msgs.p, (const uint64_t*)c->s_offsets.p + m0,
+                                     (uint8_t*)c->s_scalars.p + m0 * 32, s);
             if (!rc) rc = verify_g1_dev(c, i1 - i0, i0, (const uint8_t*)c->s_sigs.p, (const uint8_t*)c->s_scalars.p, n_msgs,
                                         (uint8_t*)c->s_status.p, s);
         }
@@ -507,26 +488,6 @@ struct Impl {
         for (size_t i = 0; i < n; i++) issuer_status[i] = (fl[i] & ISS_BAD) ? (uint8_t)ST_ERR_MALFORMED : (uint8_t)ST_ACCEPT;
         return BBS_OK;
     }
-    static int verify_multi(IssuerSet* S, size_t n, const uint32_t* item_issuer, const uint8_t* sigs, const uint8_t* scalars,
-                            const uint8_t* msgs, const uint64_t* off, uint32_t n_msgs, uint8_t* status) {
-        Ctx* c = S->base;
-        rt_stream_t s = c->stream;
-        const size_t count = n * n_msgs;
-        TRY(stage(S->item_issuer, item_issuer, n * 4, s));
-        TRY(stage(c->s_sigs, sigs, n * SIG, s));
-        TRY(c->s_status.reserve(n));
-        if (off) {
-            TRY(stage(c->s_msgs, msgs, off[count], s));
-            TRY(stage(c->s_offsets, off, (count + 1) * 8, s));
-            TRY(c->s_scalars.reserve(count * 32));
-            PROF(c, 0, s);
-            TRY(h2s_dev(c, count, (const uint8_t*)c->s_msgs.p, (const uint64_t*)c->s_offsets.p, (uint8_t*)c->s_scalars.p, s));
-        } else {
-            TRY(stage(c->s_scalars, scalars, count * 32, s));
-        }
-        TRY(core_verify_dev(c, n, (const uint8_t*)c->s_sigs.p, (const uint8_t*)c->s_scalars.p, n_msgs, (uint8_t*)c->s_status.p, s, S));
-        return finish_status(c, n, status);
-    }
 
     static int verify_dev(Ctx* c, size_t n, const uint8_t* d_sigs, const uint8_t* d_msgs, const uint64_t* d_off,
                           uint32_t n_msgs, uint8_t* d_status, rt_stream_t s) {
@@ -573,8 +534,7 @@ struct Impl {
                       (uint32_t)ph_len, (uint32_t*)c->s_pair.p, (uint32_t*)c->s_flags.p, d_status};
         if (S) {                           // issuer sets go through the task split (kernels.cuh proof_task_*) at every size
             a.item_issuer = (const uint32_t*)S->item_issuer.p;
-            a.iss = IssuerSetView{(const uint32_t*)S->K.p, (const uint32_t*)S->flags.p, (const uint32_t*)S->lines.p,
-                                  S->line_stride, (uint32_t)S->n_issuers, (const uint32_t*)S->domains.p};
+            a.iss = S->view();
         }
         a.ph_off = d_ph_off;
         if (item) a.item = *item;         // per-item headers, like issuer sets, take the task split at every size
@@ -607,12 +567,13 @@ struct Impl {
     }
 
     // ---- core_proof_gen (proof_gen.rs:116-365) -----------------------------------------------------------
-    static int proof_gen_common(Ctx* c, size_t n, const uint8_t* sigs, uint32_t n_msgs, const uint32_t* idx,
-                                const uint64_t* dis_off, const uint8_t* rand, const uint64_t* rand_off,
-                                const uint64_t* commit_off, const uint8_t* ph, size_t ph_len, uint8_t* proofs_out,
-                                uint8_t* commitments_out, uint8_t* status, const uint64_t* ph_off = nullptr,
-                                const uint8_t* headers = nullptr, const uint64_t* hdr_off = nullptr) {
+    // ph_off != nullptr: per-item phs in `ph`; hdr_off != nullptr: per-item headers (bbs_*proof_gen_batch_hdr)
+    static int proof_gen(Ctx* c, size_t n, const uint8_t* sigs, const MsgIn& in, uint32_t n_msgs, const uint32_t* idx,
+                         const uint64_t* dis_off, const uint8_t* rand, const uint64_t* rand_off, const uint64_t* commit_off,
+                         const uint8_t* ph, size_t ph_len, uint8_t* proofs_out, uint8_t* commitments_out, uint8_t* status,
+                         const uint64_t* ph_off = nullptr, const uint8_t* headers = nullptr, const uint64_t* hdr_off = nullptr) {
         rt_stream_t s = c->stream;
+        TRY(stage_scalars(c, n * n_msgs, in, c->s_msgs, c->s_offsets, c->s_scalars, false));
         ItemKeyView item{};
         if (hdr_off) TRY(item_keys(c, n, headers, hdr_off, item));
         if (ph_off) {
@@ -643,30 +604,6 @@ struct Impl {
         TRY(rt_d2h(commitments_out, c->s_commit.p, commit_off[n] * 32, s));
         return finish_status(c, n, status);
     }
-    // ph_off != nullptr: per-item phs in `ph`; hdr_off != nullptr: per-item headers (bbs_*proof_gen_batch_hdr)
-    static int core_proof_gen(Ctx* c, size_t n, const uint8_t* sigs, const uint8_t* scalars, uint32_t n_msgs,
-                              const uint32_t* idx, const uint64_t* dis_off, const uint8_t* rand, const uint64_t* rand_off,
-                              const uint64_t* commit_off, const uint8_t* ph, size_t ph_len, uint8_t* proofs_out,
-                              uint8_t* commitments_out, uint8_t* status, const uint64_t* ph_off = nullptr,
-                              const uint8_t* headers = nullptr, const uint64_t* hdr_off = nullptr) {
-        TRY(stage(c->s_scalars, scalars, n * n_msgs * 32, c->stream));
-        return proof_gen_common(c, n, sigs, n_msgs, idx, dis_off, rand, rand_off, commit_off, ph, ph_len, proofs_out,
-                                commitments_out, status, ph_off, headers, hdr_off);
-    }
-    static int proof_gen(Ctx* c, size_t n, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* off, uint32_t n_msgs,
-                         const uint32_t* idx, const uint64_t* dis_off, const uint8_t* rand, const uint64_t* rand_off,
-                         const uint64_t* commit_off, const uint8_t* ph, size_t ph_len, uint8_t* proofs_out,
-                         uint8_t* commitments_out, uint8_t* status, const uint64_t* ph_off = nullptr,
-                         const uint8_t* headers = nullptr, const uint64_t* hdr_off = nullptr) {
-        rt_stream_t s = c->stream;
-        const size_t count = n * n_msgs;
-        TRY(stage(c->s_msgs, msgs, off[count], s));
-        TRY(stage(c->s_offsets, off, (count + 1) * 8, s));
-        TRY(c->s_scalars.reserve(count * 32));
-        TRY(h2s_dev(c, count, (const uint8_t*)c->s_msgs.p, (const uint64_t*)c->s_offsets.p, (uint8_t*)c->s_scalars.p, s));
-        return proof_gen_common(c, n, sigs, n_msgs, idx, dis_off, rand, rand_off, commit_off, ph, ph_len, proofs_out,
-                                commitments_out, status, ph_off, headers, hdr_off);
-    }
 
     // ---- random-linear-combination batch mode (rlc.cuh) ---------------------------------------------
 #ifndef BBS_HOSTSIM
@@ -694,15 +631,11 @@ struct Impl {
         p.red_blocks = (threads + RLC_TPB - 1) / RLC_TPB;
         return p;
     }
-    // Host buffers of a shard, fed in up to 8 chunks: chunk k + 1 is uploaded on the copy stream while chunk k is hashed
-    // (msg_to_scalars) and prepared on the compute stream.  msgs == nullptr: `scalars` holds the n * L message scalars.
-    struct RlcFeed { const uint8_t* sigs; const uint8_t* scalars; const uint8_t* msgs; const uint64_t* off; };
-
     // shard -> comp(S1) || comp(S2) in c->s_rlc_parts (and the pairing record of the two sums); *bad != 0 when an item was
-    // malformed.  With `feed` the inputs come from host memory, otherwise d_sigs / d_scalars are already on the device.
-    static int rlc_partial_dev(Ctx* c, size_t n, const uint8_t* d_sigs, const uint8_t* d_scalars, uint32_t n_msgs,
-                               const uint8_t* seed, uint64_t index_base, uint32_t* bad, rt_stream_t s,
-                               const RlcFeed* feed = nullptr) {
+    // malformed.  The host buffers of the shard are fed in up to 8 chunks: chunk k + 1 is uploaded on the copy stream while
+    // chunk k is hashed (byte messages) and prepared on the compute stream.
+    static int rlc_partial_dev(Ctx* c, size_t n, const uint8_t* sigs, const MsgIn& in, uint32_t n_msgs, const uint8_t* seed,
+                               uint64_t index_base, uint32_t* bad, rt_stream_t s) {
         if (n >= (1ull << 31)) return arg_error("rlc shard too large");
         const uint32_t blocks = (uint32_t)((n + RLC_TPB - 1) / RLC_TPB);
         const MsmPlan plan = rlc_plan(n, c->rlc_windows);
@@ -716,18 +649,6 @@ struct Impl {
         TRY(c->s_msm_entries.reserve((n ? n : 1) * 3 * plan.W * 4));
         TRY(c->s_msm_buckets.reserve(nb * PT));
         TRY(c->s_rlc_pt.reserve((size_t)plan.rows * plan.red_blocks * PT));
-        const size_t count = n * n_msgs;
-        if (feed) {
-            TRY(c->s_sigs.reserve(n * SIG));
-            TRY(c->s_scalars.reserve(count * 32));
-            if (feed->msgs) {
-                TRY(c->s_msgs.reserve(feed->off[count]));
-                TRY(c->s_offsets.reserve((count + 1) * 8));
-            }
-            d_sigs = (const uint8_t*)c->s_sigs.p;
-            d_scalars = (const uint8_t*)c->s_scalars.p;
-            if (!c->copy_stream) RT_CHECK(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
-        }
         uint32_t* next = (uint32_t*)c->s_msm_idx.p;
         uint32_t* counts = next + 4;
         uint32_t* offsets = counts + nb;
@@ -743,43 +664,23 @@ struct Impl {
         pa.plan = plan; pa.counts = counts;
         // chunk = a whole number of waves of the prep kernel (4 blocks of RLC_TPB items per SM), at most 8 chunks; chunk
         // boundaries are multiples of the block size, so the blocks' partial sums keep their global index
-        size_t per_chunk = n ? n : 1;
-        if (feed) {
-            int sms = 0;
-            RT_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->device));
-            const size_t wave = (size_t)4 * sms * RLC_TPB;
-            const size_t waves = std::max<size_t>(2, ((n + 7) / 8 + wave - 1) / wave);
-            per_chunk = waves * wave;
-        }
-        if (feed) {
-            // all uploads are queued on the copy stream up front, one event per chunk; the copy stream first waits for the
-            // compute stream (the memsets above and, transitively, the previous call) so that no buffer is overwritten early
-            if (!c->copy_done[0]) for (auto& e : c->copy_done) RT_CHECK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-            RT_CHECK(cudaEventRecord(c->copy_done[7], s));
-            RT_CHECK(cudaStreamWaitEvent(c->copy_stream, c->copy_done[7], 0));
-            for (size_t k = 0, i0 = 0; i0 < n; k++, i0 += per_chunk) {
-                const size_t i1 = std::min(n, i0 + per_chunk), m0 = i0 * n_msgs, m1 = i1 * n_msgs;
-                TRY(rt_h2d((uint8_t*)c->s_sigs.p + i0 * SIG, feed->sigs + i0 * SIG, (i1 - i0) * SIG, c->copy_stream));
-                if (feed->msgs) {
-                    TRY(rt_h2d((uint8_t*)c->s_msgs.p + feed->off[m0], feed->msgs + feed->off[m0], feed->off[m1] - feed->off[m0], c->copy_stream));
-                    TRY(rt_h2d((uint64_t*)c->s_offsets.p + m0, feed->off + m0, (m1 - m0 + 1) * 8, c->copy_stream));
-                } else {
-                    TRY(rt_h2d((uint8_t*)c->s_scalars.p + m0 * 32, feed->scalars + m0 * 32, (m1 - m0) * 32, c->copy_stream));
-                }
-                RT_CHECK(cudaEventRecord(c->copy_done[k], c->copy_stream));
-            }
-        }
+        int sms = 0;
+        RT_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->device));
+        const size_t wave = (size_t)4 * sms * RLC_TPB;
+        const size_t waves = std::max<size_t>(2, ((n + 7) / 8 + wave - 1) / wave);
+        size_t bounds[9];
+        const int n_chunks = plan_chunks(n, waves * wave, false, bounds);
+        TRY(upload_chunks(c, n, n_chunks, bounds, sigs, in, n_msgs, s));      // after the memsets: the copy stream waits for them
         PROF(c, 0, s);
-        for (size_t k = 0, i0 = 0; i0 < n; k++, i0 += per_chunk) {
-            const size_t i1 = std::min(n, i0 + per_chunk), m0 = i0 * n_msgs, m1 = i1 * n_msgs;
-            if (feed) {
-                RT_CHECK(cudaStreamWaitEvent(s, c->copy_done[k], 0));
-                if (feed->msgs)
-                    TRY(h2s_dev(c, m1 - m0, (const uint8_t*)c->s_msgs.p, (const uint64_t*)c->s_offsets.p + m0,
-                                (uint8_t*)c->s_scalars.p + m0 * 32, s));
-            }
+        for (int k = 0; k < n_chunks; k++) {
+            const size_t i0 = bounds[k], i1 = bounds[k + 1], m0 = i0 * n_msgs, m1 = i1 * n_msgs;
+            RT_CHECK(cudaStreamWaitEvent(s, c->copy_done[k], 0));
+            if (in.off)
+                TRY(h2s_dev(c, m1 - m0, (const uint8_t*)c->s_msgs.p, (const uint64_t*)c->s_offsets.p + m0,
+                            (uint8_t*)c->s_scalars.p + m0 * 32, s));
             if (k == 0) PROF(c, 1, s);          // slot 0: first chunk's upload wait + hashing; slot 1: everything chunked after it
-            a.sigs = d_sigs + i0 * SIG; a.scalars = d_scalars + m0 * 32; a.n = (uint32_t)(i1 - i0);
+            a.sigs = (const uint8_t*)c->s_sigs.p + i0 * SIG; a.scalars = (const uint8_t*)c->s_scalars.p + m0 * 32;
+            a.n = (uint32_t)(i1 - i0);
             a.index_base = index_base + i0;
             a.sc_part = (uint32_t*)c->s_rlc_sc.p + (i0 / RLC_TPB) * (n_msgs + 1) * 8;
             pa.pts = (uint32_t*)c->s_msm_pts.p + i0 * 2 * C::Fp::N; pa.kv = (uint32_t*)c->s_msm_kv.p + i0 * 12;
@@ -809,38 +710,24 @@ struct Impl {
         TRY(rt_d2h(bad, c->s_rlc_bad.p, 4, s));
         return BBS_OK;
     }
-    static int rlc_partial(Ctx* c, size_t n, const uint8_t* sigs, const uint8_t* scalars, uint32_t n_msgs,
-                           const uint8_t* seed, uint64_t index_base, uint8_t* parts_out, uint8_t* status) {
+    static int rlc_partial(Ctx* c, size_t n, const uint8_t* sigs, const MsgIn& in, uint32_t n_msgs, const uint8_t* seed,
+                           uint64_t index_base, uint8_t* parts_out, uint8_t* status) {
         rt_stream_t s = c->stream;
         if (n_msgs != c->L) { *status = ST_ERR_MSG_GEN_LEN; return BBS_OK; }
-        const RlcFeed feed{sigs, scalars, nullptr, nullptr};
         uint32_t bad = 0;
-        TRY(rlc_partial_dev(c, n, nullptr, nullptr, n_msgs, seed, index_base, &bad, s, &feed));
-        TRY(rt_d2h(parts_out, c->s_rlc_parts.p, 2 * C::G1_BYTES, s));
-        TRY(rt_sync(s));
-        *status = bad ? ST_ERR_MALFORMED : ST_ACCEPT;
-        return BBS_OK;
-    }
-    static int rlc_partial_msgs(Ctx* c, size_t n, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* off,
-                                uint32_t n_msgs, const uint8_t* seed, uint64_t index_base, uint8_t* parts_out, uint8_t* status) {
-        rt_stream_t s = c->stream;
-        if (n_msgs != c->L) { *status = ST_ERR_MSG_GEN_LEN; return BBS_OK; }
-        const RlcFeed feed{sigs, nullptr, msgs, off};
-        uint32_t bad = 0;
-        TRY(rlc_partial_dev(c, n, nullptr, nullptr, n_msgs, seed, index_base, &bad, s, &feed));
+        TRY(rlc_partial_dev(c, n, sigs, in, n_msgs, seed, index_base, &bad, s));
         TRY(rt_d2h(parts_out, c->s_rlc_parts.p, 2 * C::G1_BYTES, s));
         TRY(rt_sync(s));
         *status = bad ? ST_ERR_MALFORMED : ST_ACCEPT;
         return BBS_OK;
     }
     // one shard = the whole batch: the finish kernel's pairing record goes straight to the pairing kernel
-    static int rlc_verify(Ctx* c, size_t n, const uint8_t* sigs, const uint8_t* scalars, const uint8_t* msgs, const uint64_t* off,
-                          uint32_t n_msgs, const uint8_t* seed, uint8_t* verdict) {
+    static int rlc_verify(Ctx* c, size_t n, const uint8_t* sigs, const MsgIn& in, uint32_t n_msgs, const uint8_t* seed,
+                          uint8_t* verdict) {
         rt_stream_t s = c->stream;
         if (n_msgs != c->L) { *verdict = ST_ERR_MSG_GEN_LEN; return BBS_OK; }
-        const RlcFeed feed{sigs, scalars, off ? msgs : nullptr, off};
         uint32_t bad = 0;
-        TRY(rlc_partial_dev(c, n, nullptr, nullptr, n_msgs, seed, 0, &bad, s, &feed));
+        TRY(rlc_partial_dev(c, n, sigs, in, n_msgs, seed, 0, &bad, s));
         TRY(pairing_dev(c, 1, (uint8_t*)c->s_status.p, s));
         PROF(c, 7, s);
         TRY(finish_status(c, 1, verdict));             // synchronises: `bad` has arrived too
@@ -863,7 +750,7 @@ struct Impl {
     }
 #endif
 
-    // ---- host-buffer wrappers ---------------------------------------------------------------------
+    // ---- host-buffer calls ------------------------------------------------------------------------------------------
     static int stage(DevBuf& b, const void* h, size_t bytes, rt_stream_t s) {
         TRY(b.reserve(bytes));
         return rt_h2d(b.p, h, bytes, s);
@@ -872,57 +759,40 @@ struct Impl {
         TRY(rt_d2h(status, c->s_status.p, n, c->stream));
         return rt_sync(c->stream);
     }
+    // the `count` message scalars of `in` into `out`: staged, or the byte messages staged into `msgs` / `off` and hashed.
+    // With `prof`, profiling slot 0 brackets the hashing kernel.
+    static int stage_scalars(Ctx* c, size_t count, const MsgIn& in, DevBuf& msgs, DevBuf& off, DevBuf& out, bool prof) {
+        rt_stream_t s = c->stream;
+        if (!in.off) return stage(out, in.scalars, count * 32, s);
+        TRY(stage(msgs, in.msgs, in.off[count], s));
+        TRY(stage(off, in.off, (count + 1) * 8, s));
+        TRY(out.reserve(count * 32));
+        if (prof) PROF(c, 0, s);
+        return h2s_dev(c, count, (const uint8_t*)msgs.p, (const uint64_t*)off.p, (uint8_t*)out.p, s);
+    }
 
     static int msg_to_scalars(Ctx* c, size_t count, const uint8_t* msgs, const uint64_t* off, uint8_t* out) {
-        rt_stream_t s = c->stream;
-        TRY(stage(c->s_msgs, msgs, off[count], s));
-        TRY(stage(c->s_offsets, off, (count + 1) * 8, s));
-        TRY(c->s_scalars.reserve(count * 32));
-        TRY(h2s_dev(c, count, (const uint8_t*)c->s_msgs.p, (const uint64_t*)c->s_offsets.p, (uint8_t*)c->s_scalars.p, s));
-        TRY(rt_d2h(out, c->s_scalars.p, count * 32, s));
-        return rt_sync(s);
+        TRY(stage_scalars(c, count, MsgIn{nullptr, msgs, off}, c->s_msgs, c->s_offsets, c->s_scalars, false));
+        TRY(rt_d2h(out, c->s_scalars.p, count * 32, c->stream));
+        return rt_sync(c->stream);
     }
-    static int core_verify(Ctx* c, size_t n, const uint8_t* sigs, const uint8_t* scalars, uint32_t n_msgs, uint8_t* status) {
+    // verify / core_verify; hdr_off != nullptr: a header per item (bbs_*verify_batch_hdr); S != nullptr: the issuer of each
+    // item in item_issuer (bbs_*verify_batch_multi, c = S->base)
+    static int verify(Ctx* c, size_t n, const uint8_t* sigs, const MsgIn& in, uint32_t n_msgs, uint8_t* status,
+                      const uint8_t* headers = nullptr, const uint64_t* hdr_off = nullptr, IssuerSet* S = nullptr,
+                      const uint32_t* item_issuer = nullptr) {
 #ifndef BBS_HOSTSIM
-        if (n >= 2 * VERIFY_CHUNK) return verify_chunked(c, n, sigs, nullptr, nullptr, scalars, n_msgs, status);
+        if (!hdr_off && !S && n >= 2 * VERIFY_CHUNK) return verify_chunked(c, n, sigs, in, n_msgs, status);
 #endif
         rt_stream_t s = c->stream;
+        ItemKeyView item{};
+        if (hdr_off) TRY(item_keys(c, n, headers, hdr_off, item));
+        if (S) TRY(stage(S->item_issuer, item_issuer, n * 4, s));
         TRY(stage(c->s_sigs, sigs, n * SIG, s));
-        TRY(stage(c->s_scalars, scalars, n * n_msgs * 32, s));
         TRY(c->s_status.reserve(n));
-        TRY(core_verify_dev(c, n, (const uint8_t*)c->s_sigs.p, (const uint8_t*)c->s_scalars.p, n_msgs,
-                            (uint8_t*)c->s_status.p, s));
-        return finish_status(c, n, status);
-    }
-    static int verify(Ctx* c, size_t n, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* off, uint32_t n_msgs,
-                      uint8_t* status) {
-#ifndef BBS_HOSTSIM
-        if (n >= 2 * VERIFY_CHUNK) return verify_chunked(c, n, sigs, msgs, off, nullptr, n_msgs, status);
-#endif
-        rt_stream_t s = c->stream;
-        const size_t count = n * n_msgs;
-        TRY(stage(c->s_sigs, sigs, n * SIG, s));
-        TRY(stage(c->s_msgs, msgs, off[count], s));
-        TRY(stage(c->s_offsets, off, (count + 1) * 8, s));
-        TRY(c->s_status.reserve(n));
-        TRY(verify_dev(c, n, (const uint8_t*)c->s_sigs.p, (const uint8_t*)c->s_msgs.p, (const uint64_t*)c->s_offsets.p,
-                       n_msgs, (uint8_t*)c->s_status.p, s));
-        return finish_status(c, n, status);
-    }
-    static int sign_common(Ctx* c, const uint8_t* sk, size_t n, uint32_t n_msgs, uint8_t* sigs_out, uint8_t* b_out,
-                           uint8_t* status, const ItemKeyView* item = nullptr) {
-        rt_stream_t s = c->stream;
-        TRY(c->s_out.reserve(n * SIG));
-        TRY(c->s_out2.reserve(n * C::G1_BYTES));
-        TRY(c->s_status.reserve(n));
-        TRY(rt_memset(c->s_out.p, 0, n * SIG, s));
-        TRY(core_sign_dev(c, sk, n, (const uint8_t*)c->s_scalars.p, n_msgs, (uint8_t*)c->s_out.p,
-                          b_out ? (uint8_t*)c->s_out2.p : nullptr, (uint8_t*)c->s_status.p, s, item));
-        TRY(rt_d2h(sigs_out, c->s_out.p, n * SIG, s));
-        if (b_out) TRY(rt_d2h(b_out, c->s_out2.p, n * C::G1_BYTES, s));
-        // the signer's staging copies of the messages and their scalars do not outlive the call
-        TRY(rt_memset(c->s_scalars.p, 0, n * (size_t)n_msgs * 32, s));
-        if (c->s_msgs.p && c->s_msgs.cap) TRY(rt_memset(c->s_msgs.p, 0, c->s_msgs.cap, s));
+        TRY(stage_scalars(c, n * n_msgs, in, c->s_msgs, c->s_offsets, c->s_scalars, true));
+        TRY(core_verify_dev(c, n, (const uint8_t*)c->s_sigs.p, (const uint8_t*)c->s_scalars.p, n_msgs, (uint8_t*)c->s_status.p,
+                            s, S, hdr_off ? &item : nullptr));
         return finish_status(c, n, status);
     }
 #ifndef BBS_HOSTSIM
@@ -930,54 +800,27 @@ struct Impl {
     // stream with one event per chunk, the compute stream hashes and signs chunk k while chunk k + 1 is in flight, and a
     // third stream brings the signatures of chunk k - 1 back (H2D and D2H run on separate copy engines).  The items are
     // independent, so the results are those of the one-shot path; 1.7 GB per 4 M signatures cross the bus either way.
+    // Chunk sizes double from SIGN_CHUNK: the first upload (the only one nothing hides) is small, and few launches keep the
+    // kernel's tail effects (~3 % per launch at 524,288 items) down.
     static constexpr size_t SIGN_CHUNK = 262144;
-    static int sign_chunked(Ctx* c, const uint8_t* sk, size_t n, const uint8_t* msgs, const uint64_t* off, const uint8_t* scalars,
-                            uint32_t n_msgs, uint8_t* sigs_out, uint8_t* b_out, uint8_t* status) {
+    static int sign_chunked(Ctx* c, const uint8_t* sk, size_t n, const MsgIn& in, uint32_t n_msgs, uint8_t* sigs_out,
+                            uint8_t* b_out, uint8_t* status) {
         rt_stream_t s = c->stream;
-        const size_t count = n * n_msgs;
-        // chunk sizes double from SIGN_CHUNK: the first upload (the only one nothing hides) is small, and few launches
-        // keep the kernel's tail effects (~3 % per launch at 524,288 items) down; at most 8 chunks
         size_t bounds[9];
-        int n_chunks = 0;
-        bounds[0] = 0;
-        for (size_t at = 0, cur = SIGN_CHUNK; at < n; cur *= 2) {
-            size_t take = std::min(n - at, cur);
-            if (n - at - take < SIGN_CHUNK || n_chunks == 7) take = n - at;
-            at += take;
-            bounds[++n_chunks] = at;
-        }
-        TRY(c->s_scalars.reserve(count * 32));
-        if (msgs) {
-            TRY(c->s_msgs.reserve(off[count]));
-            TRY(c->s_offsets.reserve((count + 1) * 8));
-        }
+        const int n_chunks = plan_chunks(n, SIGN_CHUNK, true, bounds);
         TRY(c->s_out.reserve(n * SIG));
         TRY(c->s_out2.reserve(n * C::G1_BYTES));
         TRY(c->s_status.reserve(n));
-        if (!c->copy_stream) RT_CHECK(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
         if (!c->down_stream) RT_CHECK(cudaStreamCreateWithFlags(&c->down_stream, cudaStreamNonBlocking));
-        if (!c->copy_done[0]) for (auto& e : c->copy_done) RT_CHECK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
         if (!c->comp_done[0]) for (auto& e : c->comp_done) RT_CHECK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
         TRY(rt_memset(c->s_out.p, 0, n * SIG, s));
-        // the copy stream starts after everything already queued on the compute stream (buffer reuse across calls)
-        RT_CHECK(cudaEventRecord(c->copy_done[7], s));
-        RT_CHECK(cudaStreamWaitEvent(c->copy_stream, c->copy_done[7], 0));
-        for (int k = 0; k < n_chunks; k++) {
-            const size_t i0 = bounds[k], i1 = bounds[k + 1], m0 = i0 * n_msgs, m1 = i1 * n_msgs;
-            if (msgs) {
-                TRY(rt_h2d((uint8_t*)c->s_msgs.p + off[m0], msgs + off[m0], off[m1] - off[m0], c->copy_stream));
-                TRY(rt_h2d((uint64_t*)c->s_offsets.p + m0, off + m0, (m1 - m0 + 1) * 8, c->copy_stream));
-            } else {
-                TRY(rt_h2d((uint8_t*)c->s_scalars.p + m0 * 32, scalars + m0 * 32, (m1 - m0) * 32, c->copy_stream));
-            }
-            RT_CHECK(cudaEventRecord(c->copy_done[k], c->copy_stream));
-        }
+        TRY(upload_chunks(c, n, n_chunks, bounds, nullptr, in, n_msgs, s));
         int rc = BBS_OK;
         for (int k = 0; k < n_chunks && !rc; k++) {
             const size_t i0 = bounds[k], i1 = bounds[k + 1], m0 = i0 * n_msgs, m1 = i1 * n_msgs, cnt = i1 - i0;
             RT_CHECK(cudaStreamWaitEvent(s, c->copy_done[k], 0));
-            if (msgs) rc = h2s_dev(c, m1 - m0, (const uint8_t*)c->s_msgs.p, (const uint64_t*)c->s_offsets.p + m0,
-                                   (uint8_t*)c->s_scalars.p + m0 * 32, s);
+            if (in.off) rc = h2s_dev(c, m1 - m0, (const uint8_t*)c->s_msgs.p, (const uint64_t*)c->s_offsets.p + m0,
+                                     (uint8_t*)c->s_scalars.p + m0 * 32, s);
             if (!rc) rc = core_sign_dev(c, sk, cnt, (const uint8_t*)c->s_scalars.p + m0 * 32, n_msgs, (uint8_t*)c->s_out.p + i0 * SIG,
                                         b_out ? (uint8_t*)c->s_out2.p + i0 * C::G1_BYTES : nullptr, (uint8_t*)c->s_status.p + i0, s);
             if (rc) break;
@@ -990,41 +833,45 @@ struct Impl {
         // the signer's staging copies of the messages and their scalars do not outlive the call (also on an error path:
         // everything queued so far is drained first)
         cudaStreamSynchronize(c->copy_stream);
-        int rc2 = rt_memset(c->s_scalars.p, 0, count * 32, s);
+        int rc2 = rt_memset(c->s_scalars.p, 0, n * n_msgs * 32, s);
         if (!rc2 && c->s_msgs.p && c->s_msgs.cap) rc2 = rt_memset(c->s_msgs.p, 0, c->s_msgs.cap, s);
         cudaStreamSynchronize(c->down_stream);
         const int rc3 = rt_sync(s);
         return rc ? rc : (rc2 ? rc2 : rc3);
     }
 #endif
-    static int core_sign(Ctx* c, const uint8_t* sk, size_t n, const uint8_t* scalars, uint32_t n_msgs, uint8_t* sigs_out,
-                         uint8_t* b_out, uint8_t* status) {
+    // sign / core_sign; hdr_off != nullptr: a header per item (bbs_*sign_batch_hdr)
+    static int sign(Ctx* c, const uint8_t* sk, size_t n, const MsgIn& in, uint32_t n_msgs, uint8_t* sigs_out, uint8_t* b_out,
+                    uint8_t* status, const uint8_t* headers = nullptr, const uint64_t* hdr_off = nullptr) {
 #ifndef BBS_HOSTSIM
-        if (n >= 2 * SIGN_CHUNK) return sign_chunked(c, sk, n, nullptr, nullptr, scalars, n_msgs, sigs_out, b_out, status);
-#endif
-        TRY(stage(c->s_scalars, scalars, n * n_msgs * 32, c->stream));
-        return sign_common(c, sk, n, n_msgs, sigs_out, b_out, status);
-    }
-    static int sign(Ctx* c, const uint8_t* sk, size_t n, const uint8_t* msgs, const uint64_t* off, uint32_t n_msgs,
-                    uint8_t* sigs_out, uint8_t* b_out, uint8_t* status) {
-#ifndef BBS_HOSTSIM
-        if (n >= 2 * SIGN_CHUNK) return sign_chunked(c, sk, n, msgs, off, nullptr, n_msgs, sigs_out, b_out, status);
+        if (!hdr_off && n >= 2 * SIGN_CHUNK) return sign_chunked(c, sk, n, in, n_msgs, sigs_out, b_out, status);
 #endif
         rt_stream_t s = c->stream;
-        const size_t count = n * n_msgs;
-        TRY(stage(c->s_msgs, msgs, off[count], s));
-        TRY(stage(c->s_offsets, off, (count + 1) * 8, s));
-        TRY(c->s_scalars.reserve(count * 32));
-        PROF(c, 0, s);
-        TRY(h2s_dev(c, count, (const uint8_t*)c->s_msgs.p, (const uint64_t*)c->s_offsets.p, (uint8_t*)c->s_scalars.p, s));
-        return sign_common(c, sk, n, n_msgs, sigs_out, b_out, status);
+        ItemKeyView item{};
+        if (hdr_off) TRY(item_keys(c, n, headers, hdr_off, item));
+        TRY(stage_scalars(c, n * n_msgs, in, c->s_msgs, c->s_offsets, c->s_scalars, true));
+        TRY(c->s_out.reserve(n * SIG));
+        TRY(c->s_out2.reserve(n * C::G1_BYTES));
+        TRY(c->s_status.reserve(n));
+        TRY(rt_memset(c->s_out.p, 0, n * SIG, s));
+        TRY(core_sign_dev(c, sk, n, (const uint8_t*)c->s_scalars.p, n_msgs, (uint8_t*)c->s_out.p,
+                          b_out ? (uint8_t*)c->s_out2.p : nullptr, (uint8_t*)c->s_status.p, s, hdr_off ? &item : nullptr));
+        TRY(rt_d2h(sigs_out, c->s_out.p, n * SIG, s));
+        if (b_out) TRY(rt_d2h(b_out, c->s_out2.p, n * C::G1_BYTES, s));
+        // the signer's staging copies of the messages and their scalars do not outlive the call
+        TRY(rt_memset(c->s_scalars.p, 0, n * (size_t)n_msgs * 32, s));
+        if (c->s_msgs.p && c->s_msgs.cap) TRY(rt_memset(c->s_msgs.p, 0, c->s_msgs.cap, s));
+        return finish_status(c, n, status);
     }
-    // ph_off != nullptr: per-item phs in `ph`; hdr_off != nullptr: per-item headers (bbs_*proof_verify_batch_hdr)
-    static int proof_common(Ctx* c, size_t n, const uint8_t* proofs, const uint8_t* commit, const uint64_t* commit_off,
-                            const uint32_t* idx, const uint64_t* dis_off, const uint8_t* ph, size_t ph_len,
+    // proof_verify / core_proof_verify: `dis` holds the disclosed messages (or their scalars); ph_off != nullptr: per-item
+    // phs in `ph`; hdr_off != nullptr: per-item headers (bbs_*proof_verify_batch_hdr); S != nullptr: the issuer of each
+    // item in item_issuer (bbs_*proof_verify_batch_multi, c = S->base)
+    static int proof_verify(Ctx* c, size_t n, const uint8_t* proofs, const uint8_t* commit, const uint64_t* commit_off,
+                            const uint32_t* idx, const MsgIn& dis, const uint64_t* dis_off, const uint8_t* ph, size_t ph_len,
                             uint8_t* status, IssuerSet* S = nullptr, const uint32_t* item_issuer = nullptr,
                             const uint64_t* ph_off = nullptr, const uint8_t* headers = nullptr, const uint64_t* hdr_off = nullptr) {
         rt_stream_t s = c->stream;
+        TRY(stage_scalars(c, dis_off[n], dis, c->s_dis_msgs, c->s_dis_msg_off, c->s_dis_scalars, false));
         ItemKeyView item{};
         if (hdr_off) TRY(item_keys(c, n, headers, hdr_off, item));
         if (ph_off) {
@@ -1046,30 +893,6 @@ struct Impl {
                                   ph_off ? (const uint64_t*)c->s_ph_off.p : nullptr));
         return finish_status(c, n, status);
     }
-    static int core_proof_verify(Ctx* c, size_t n, const uint8_t* proofs, const uint8_t* commit, const uint64_t* commit_off,
-                                 const uint32_t* idx, const uint8_t* dis_scalars, const uint64_t* dis_off,
-                                 const uint8_t* ph, size_t ph_len, uint8_t* status, IssuerSet* S = nullptr,
-                                 const uint32_t* item_issuer = nullptr, const uint64_t* ph_off = nullptr,
-                                 const uint8_t* headers = nullptr, const uint64_t* hdr_off = nullptr) {
-        TRY(stage(c->s_dis_scalars, dis_scalars, dis_off[n] * 32, c->stream));
-        return proof_common(c, n, proofs, commit, commit_off, idx, dis_off, ph, ph_len, status, S, item_issuer, ph_off, headers,
-                            hdr_off);
-    }
-    static int proof_verify(Ctx* c, size_t n, const uint8_t* proofs, const uint8_t* commit, const uint64_t* commit_off,
-                            const uint32_t* idx, const uint8_t* dis_msgs, const uint64_t* dis_msg_off,
-                            const uint64_t* dis_off, const uint8_t* ph, size_t ph_len, uint8_t* status,
-                            IssuerSet* S = nullptr, const uint32_t* item_issuer = nullptr, const uint64_t* ph_off = nullptr,
-                            const uint8_t* headers = nullptr, const uint64_t* hdr_off = nullptr) {
-        rt_stream_t s = c->stream;
-        const size_t count = dis_off[n];
-        TRY(stage(c->s_dis_msgs, dis_msgs, dis_msg_off[count], s));
-        TRY(stage(c->s_dis_msg_off, dis_msg_off, (count + 1) * 8, s));
-        TRY(c->s_dis_scalars.reserve(count * 32));
-        TRY(h2s_dev(c, count, (const uint8_t*)c->s_dis_msgs.p, (const uint64_t*)c->s_dis_msg_off.p,
-                    (uint8_t*)c->s_dis_scalars.p, s));
-        return proof_common(c, n, proofs, commit, commit_off, idx, dis_off, ph, ph_len, status, S, item_issuer, ph_off, headers,
-                            hdr_off);
-    }
 };
 
 #include "selftest_host.inc"
@@ -1087,12 +910,22 @@ int fresh_seed(uint8_t out[32]) {
     return 0;
 }
 
+// per-item headers (hdr_off != NULL) need a context created with the flag
+int check_hdr_flag(Ctx* c, const uint64_t* hdr_off) {
+    if (c && hdr_off && !c->per_item_header) return arg_error("per-item headers need a context created with BBS_CTX_PER_ITEM_HEADER");
+    return BBS_OK;
+}
 // the per-item header arguments of a *_hdr call: `required` (verify / sign) or NULL = the context's header (proofs)
 int check_hdr_args(Ctx* c, size_t n, const uint8_t* headers, const uint64_t* hdr_off, bool required) {
     if (!c) return arg_error("null context");
     if (!hdr_off) return required ? arg_error("hdr_off is null") : BBS_OK;
-    if (!c->per_item_header) return arg_error("per-item headers need a context created with BBS_CTX_PER_ITEM_HEADER");
+    TRY(check_hdr_flag(c, hdr_off));
     return check_items(n, headers, hdr_off, "header");
+}
+// the flat commitment and disclosed-index counts of a proof call
+int check_flat_counts(size_t n, const uint64_t* commit_off, const uint64_t* dis_off) {
+    if (commit_off[n] > 0xffffffffull || dis_off[n] > 0xffffffffull) return arg_error("batch too large: flat counts must fit in 32 bits");
+    return BBS_OK;
 }
 #define DISPATCH(c, call)                                              \
     do {                                                               \
@@ -1259,7 +1092,7 @@ int bbs_core_verify_batch(bbs_ctx* p, size_t n, const uint8_t* sigs, const uint8
     if (!n) return BBS_OK;
     if (!sigs || !status || (n_msgs && !scalars)) return arg_error("null");
     CHECK_COUNTS(n, n_msgs);
-    DISPATCH(c, core_verify(c, n, sigs, scalars, n_msgs, status));
+    DISPATCH(c, verify(c, n, sigs, MsgIn{scalars, nullptr, nullptr}, n_msgs, status));
 }
 int bbs_verify_batch(bbs_ctx* p, size_t n, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* off, uint32_t n_msgs,
                      uint8_t* status) {
@@ -1267,7 +1100,7 @@ int bbs_verify_batch(bbs_ctx* p, size_t n, const uint8_t* sigs, const uint8_t* m
     if (!n) return BBS_OK;
     if (!sigs || !status || !off) return arg_error("null");
     CHECK_COUNTS(n, n_msgs);
-    DISPATCH(c, verify(c, n, sigs, msgs, off, n_msgs, status));
+    DISPATCH(c, verify(c, n, sigs, MsgIn{nullptr, msgs, off}, n_msgs, status));
 }
 int bbs_core_sign_batch(bbs_ctx* p, const uint8_t sk[32], size_t n, const uint8_t* scalars, uint32_t n_msgs,
                         uint8_t* sigs_out, uint8_t* b_out, uint8_t* status) {
@@ -1275,7 +1108,7 @@ int bbs_core_sign_batch(bbs_ctx* p, const uint8_t sk[32], size_t n, const uint8_
     if (!n) return BBS_OK;
     if (!sk || !sigs_out || !status || (n_msgs && !scalars)) return arg_error("null");
     CHECK_COUNTS(n, n_msgs);
-    DISPATCH(c, core_sign(c, sk, n, scalars, n_msgs, sigs_out, b_out, status));
+    DISPATCH(c, sign(c, sk, n, MsgIn{scalars, nullptr, nullptr}, n_msgs, sigs_out, b_out, status));
 }
 int bbs_sign_batch(bbs_ctx* p, const uint8_t sk[32], size_t n, const uint8_t* msgs, const uint64_t* off, uint32_t n_msgs,
                    uint8_t* sigs_out, uint8_t* b_out, uint8_t* status) {
@@ -1283,7 +1116,7 @@ int bbs_sign_batch(bbs_ctx* p, const uint8_t sk[32], size_t n, const uint8_t* ms
     if (!n) return BBS_OK;
     if (!sk || !sigs_out || !status || !off) return arg_error("null");
     CHECK_COUNTS(n, n_msgs);
-    DISPATCH(c, sign(c, sk, n, msgs, off, n_msgs, sigs_out, b_out, status));
+    DISPATCH(c, sign(c, sk, n, MsgIn{nullptr, msgs, off}, n_msgs, sigs_out, b_out, status));
 }
 int bbs_core_proof_verify_batch(bbs_ctx* p, size_t n, const uint8_t* proofs, const uint8_t* commit,
                                 const uint64_t* commit_off, const uint32_t* idx, const uint8_t* dis_scalars,
@@ -1292,8 +1125,8 @@ int bbs_core_proof_verify_batch(bbs_ctx* p, size_t n, const uint8_t* proofs, con
     if (!n) return BBS_OK;
     if (!proofs || !commit_off || !dis_off || !status) return arg_error("null");
     CHECK_COUNTS(n, 1);
-    if (commit_off[n] > 0xffffffffull || dis_off[n] > 0xffffffffull) return arg_error("batch too large: flat counts must fit in 32 bits");
-    DISPATCH(c, core_proof_verify(c, n, proofs, commit, commit_off, idx, dis_scalars, dis_off, ph, ph_len, status));
+    TRY(check_flat_counts(n, commit_off, dis_off));
+    DISPATCH(c, proof_verify(c, n, proofs, commit, commit_off, idx, MsgIn{dis_scalars, nullptr, nullptr}, dis_off, ph, ph_len, status));
 }
 int bbs_proof_verify_batch(bbs_ctx* p, size_t n, const uint8_t* proofs, const uint8_t* commit, const uint64_t* commit_off,
                            const uint32_t* idx, const uint8_t* dis_msgs, const uint64_t* dis_msg_off,
@@ -1302,8 +1135,8 @@ int bbs_proof_verify_batch(bbs_ctx* p, size_t n, const uint8_t* proofs, const ui
     if (!n) return BBS_OK;
     if (!proofs || !commit_off || !dis_off || !dis_msg_off || !status) return arg_error("null");
     CHECK_COUNTS(n, 1);
-    if (commit_off[n] > 0xffffffffull || dis_off[n] > 0xffffffffull) return arg_error("batch too large: flat counts must fit in 32 bits");
-    DISPATCH(c, proof_verify(c, n, proofs, commit, commit_off, idx, dis_msgs, dis_msg_off, dis_off, ph, ph_len, status));
+    TRY(check_flat_counts(n, commit_off, dis_off));
+    DISPATCH(c, proof_verify(c, n, proofs, commit, commit_off, idx, MsgIn{nullptr, dis_msgs, dis_msg_off}, dis_off, ph, ph_len, status));
 }
 
 int bbs_core_proof_gen_batch(bbs_ctx* p, size_t n, const uint8_t* sigs, const uint8_t* scalars, uint32_t n_msgs,
@@ -1315,8 +1148,8 @@ int bbs_core_proof_gen_batch(bbs_ctx* p, size_t n, const uint8_t* sigs, const ui
     if (!sigs || !dis_off || !rand || !rand_off || !commit_off || !proofs_out || !status) return arg_error("null");
     CHECK_COUNTS(n, n_msgs);
     if (n_msgs > BBS_MAX_MESSAGES) return arg_error("n_msgs exceeds BBS_MAX_MESSAGES");
-    DISPATCH(c, core_proof_gen(c, n, sigs, scalars, n_msgs, idx, dis_off, rand, rand_off, commit_off, ph, ph_len,
-                               proofs_out, commitments_out, status));
+    DISPATCH(c, proof_gen(c, n, sigs, MsgIn{scalars, nullptr, nullptr}, n_msgs, idx, dis_off, rand, rand_off, commit_off, ph,
+                          ph_len, proofs_out, commitments_out, status));
 }
 int bbs_proof_gen_batch(bbs_ctx* p, size_t n, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* off, uint32_t n_msgs,
                         const uint32_t* idx, const uint64_t* dis_off, const uint8_t* rand, const uint64_t* rand_off,
@@ -1327,8 +1160,8 @@ int bbs_proof_gen_batch(bbs_ctx* p, size_t n, const uint8_t* sigs, const uint8_t
     if (!sigs || !off || !dis_off || !rand || !rand_off || !commit_off || !proofs_out || !status) return arg_error("null");
     CHECK_COUNTS(n, n_msgs);
     if (n_msgs > BBS_MAX_MESSAGES) return arg_error("n_msgs exceeds BBS_MAX_MESSAGES");
-    DISPATCH(c, proof_gen(c, n, sigs, msgs, off, n_msgs, idx, dis_off, rand, rand_off, commit_off, ph, ph_len, proofs_out,
-                          commitments_out, status));
+    DISPATCH(c, proof_gen(c, n, sigs, MsgIn{nullptr, msgs, off}, n_msgs, idx, dis_off, rand, rand_off, commit_off, ph, ph_len,
+                          proofs_out, commitments_out, status));
 }
 
 // ---- per-item headers and presentation headers ------------------------------------------------------------------
@@ -1339,7 +1172,7 @@ int bbs_core_verify_batch_hdr(bbs_ctx* p, size_t n, const uint8_t* sigs, const u
     if (!sigs || !status || (n_msgs && !scalars)) return arg_error("null");
     CHECK_COUNTS(n, n_msgs);
     TRY(check_hdr_args(c, n, headers, hdr_off, true));
-    DISPATCH(c, verify_hdr(c, n, sigs, scalars, nullptr, nullptr, n_msgs, headers, hdr_off, status));
+    DISPATCH(c, verify(c, n, sigs, MsgIn{scalars, nullptr, nullptr}, n_msgs, status, headers, hdr_off));
 }
 int bbs_verify_batch_hdr(bbs_ctx* p, size_t n, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* off, uint32_t n_msgs,
                          const uint8_t* headers, const uint64_t* hdr_off, uint8_t* status) {
@@ -1348,7 +1181,7 @@ int bbs_verify_batch_hdr(bbs_ctx* p, size_t n, const uint8_t* sigs, const uint8_
     if (!sigs || !status || !off) return arg_error("null");
     CHECK_COUNTS(n, n_msgs);
     TRY(check_hdr_args(c, n, headers, hdr_off, true));
-    DISPATCH(c, verify_hdr(c, n, sigs, nullptr, msgs, off, n_msgs, headers, hdr_off, status));
+    DISPATCH(c, verify(c, n, sigs, MsgIn{nullptr, msgs, off}, n_msgs, status, headers, hdr_off));
 }
 int bbs_core_sign_batch_hdr(bbs_ctx* p, const uint8_t sk[32], size_t n, const uint8_t* scalars, uint32_t n_msgs,
                             const uint8_t* headers, const uint64_t* hdr_off, uint8_t* sigs_out, uint8_t* b_out, uint8_t* status) {
@@ -1357,7 +1190,7 @@ int bbs_core_sign_batch_hdr(bbs_ctx* p, const uint8_t sk[32], size_t n, const ui
     if (!sk || !sigs_out || !status || (n_msgs && !scalars)) return arg_error("null");
     CHECK_COUNTS(n, n_msgs);
     TRY(check_hdr_args(c, n, headers, hdr_off, true));
-    DISPATCH(c, sign_hdr(c, sk, n, scalars, nullptr, nullptr, n_msgs, headers, hdr_off, sigs_out, b_out, status));
+    DISPATCH(c, sign(c, sk, n, MsgIn{scalars, nullptr, nullptr}, n_msgs, sigs_out, b_out, status, headers, hdr_off));
 }
 int bbs_sign_batch_hdr(bbs_ctx* p, const uint8_t sk[32], size_t n, const uint8_t* msgs, const uint64_t* off, uint32_t n_msgs,
                        const uint8_t* headers, const uint64_t* hdr_off, uint8_t* sigs_out, uint8_t* b_out, uint8_t* status) {
@@ -1366,7 +1199,7 @@ int bbs_sign_batch_hdr(bbs_ctx* p, const uint8_t sk[32], size_t n, const uint8_t
     if (!sk || !sigs_out || !status || !off) return arg_error("null");
     CHECK_COUNTS(n, n_msgs);
     TRY(check_hdr_args(c, n, headers, hdr_off, true));
-    DISPATCH(c, sign_hdr(c, sk, n, nullptr, msgs, off, n_msgs, headers, hdr_off, sigs_out, b_out, status));
+    DISPATCH(c, sign(c, sk, n, MsgIn{nullptr, msgs, off}, n_msgs, sigs_out, b_out, status, headers, hdr_off));
 }
 int bbs_core_proof_verify_batch_hdr(bbs_ctx* p, size_t n, const uint8_t* proofs, const uint8_t* commit,
                                     const uint64_t* commit_off, const uint32_t* idx, const uint8_t* dis_scalars,
@@ -1376,11 +1209,11 @@ int bbs_core_proof_verify_batch_hdr(bbs_ctx* p, size_t n, const uint8_t* proofs,
     if (!n) return BBS_OK;
     if (!proofs || !commit_off || !dis_off || !status || !ph_off) return arg_error("null");
     CHECK_COUNTS(n, 1);
-    if (commit_off[n] > 0xffffffffull || dis_off[n] > 0xffffffffull) return arg_error("batch too large: flat counts must fit in 32 bits");
+    TRY(check_flat_counts(n, commit_off, dis_off));
     TRY(check_hdr_args(c, n, headers, hdr_off, false));
     TRY(check_items(n, phs, ph_off, "ph"));
-    DISPATCH(c, core_proof_verify(c, n, proofs, commit, commit_off, idx, dis_scalars, dis_off, phs, 0, status, nullptr, nullptr,
-                                  ph_off, headers, hdr_off));
+    DISPATCH(c, proof_verify(c, n, proofs, commit, commit_off, idx, MsgIn{dis_scalars, nullptr, nullptr}, dis_off, phs, 0, status,
+                             nullptr, nullptr, ph_off, headers, hdr_off));
 }
 int bbs_proof_verify_batch_hdr(bbs_ctx* p, size_t n, const uint8_t* proofs, const uint8_t* commit, const uint64_t* commit_off,
                                const uint32_t* idx, const uint8_t* dis_msgs, const uint64_t* dis_msg_off, const uint64_t* dis_off,
@@ -1390,11 +1223,11 @@ int bbs_proof_verify_batch_hdr(bbs_ctx* p, size_t n, const uint8_t* proofs, cons
     if (!n) return BBS_OK;
     if (!proofs || !commit_off || !dis_off || !dis_msg_off || !status || !ph_off) return arg_error("null");
     CHECK_COUNTS(n, 1);
-    if (commit_off[n] > 0xffffffffull || dis_off[n] > 0xffffffffull) return arg_error("batch too large: flat counts must fit in 32 bits");
+    TRY(check_flat_counts(n, commit_off, dis_off));
     TRY(check_hdr_args(c, n, headers, hdr_off, false));
     TRY(check_items(n, phs, ph_off, "ph"));
-    DISPATCH(c, proof_verify(c, n, proofs, commit, commit_off, idx, dis_msgs, dis_msg_off, dis_off, phs, 0, status, nullptr, nullptr,
-                             ph_off, headers, hdr_off));
+    DISPATCH(c, proof_verify(c, n, proofs, commit, commit_off, idx, MsgIn{nullptr, dis_msgs, dis_msg_off}, dis_off, phs, 0, status,
+                             nullptr, nullptr, ph_off, headers, hdr_off));
 }
 int bbs_core_proof_gen_batch_hdr(bbs_ctx* p, size_t n, const uint8_t* sigs, const uint8_t* scalars, uint32_t n_msgs,
                                  const uint32_t* idx, const uint64_t* dis_off, const uint8_t* rand, const uint64_t* rand_off,
@@ -1407,8 +1240,8 @@ int bbs_core_proof_gen_batch_hdr(bbs_ctx* p, size_t n, const uint8_t* sigs, cons
     if (n_msgs > BBS_MAX_MESSAGES) return arg_error("n_msgs exceeds BBS_MAX_MESSAGES");
     TRY(check_hdr_args(c, n, headers, hdr_off, false));
     TRY(check_items(n, phs, ph_off, "ph"));
-    DISPATCH(c, core_proof_gen(c, n, sigs, scalars, n_msgs, idx, dis_off, rand, rand_off, commit_off, phs, 0, proofs_out,
-                               commitments_out, status, ph_off, headers, hdr_off));
+    DISPATCH(c, proof_gen(c, n, sigs, MsgIn{scalars, nullptr, nullptr}, n_msgs, idx, dis_off, rand, rand_off, commit_off, phs, 0,
+                          proofs_out, commitments_out, status, ph_off, headers, hdr_off));
 }
 int bbs_proof_gen_batch_hdr(bbs_ctx* p, size_t n, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* off, uint32_t n_msgs,
                             const uint32_t* idx, const uint64_t* dis_off, const uint8_t* rand, const uint64_t* rand_off,
@@ -1421,8 +1254,8 @@ int bbs_proof_gen_batch_hdr(bbs_ctx* p, size_t n, const uint8_t* sigs, const uin
     if (n_msgs > BBS_MAX_MESSAGES) return arg_error("n_msgs exceeds BBS_MAX_MESSAGES");
     TRY(check_hdr_args(c, n, headers, hdr_off, false));
     TRY(check_items(n, phs, ph_off, "ph"));
-    DISPATCH(c, proof_gen(c, n, sigs, msgs, off, n_msgs, idx, dis_off, rand, rand_off, commit_off, phs, 0, proofs_out,
-                          commitments_out, status, ph_off, headers, hdr_off));
+    DISPATCH(c, proof_gen(c, n, sigs, MsgIn{nullptr, msgs, off}, n_msgs, idx, dis_off, rand, rand_off, commit_off, phs, 0,
+                          proofs_out, commitments_out, status, ph_off, headers, hdr_off));
 }
 
 // ---- issuer sets (multi-issuer batches) -------------------------------------------------------------------
@@ -1482,7 +1315,7 @@ int bbs_verify_batch_multi(bbs_issuer_set* p, size_t n, const uint32_t* item_iss
     if (!n) return BBS_OK;
     if (!item_issuer || !sigs || !status || !off) return arg_error("null");
     CHECK_COUNTS(n, n_msgs);
-    DISPATCH_SET(S, verify_multi(S, n, item_issuer, sigs, nullptr, msgs, off, n_msgs, status));
+    DISPATCH_SET(S, verify(S->base, n, sigs, MsgIn{nullptr, msgs, off}, n_msgs, status, nullptr, nullptr, S, item_issuer));
 }
 int bbs_core_verify_batch_multi(bbs_issuer_set* p, size_t n, const uint32_t* item_issuer, const uint8_t* sigs,
                                 const uint8_t* scalars, uint32_t n_msgs, uint8_t* status) {
@@ -1490,7 +1323,7 @@ int bbs_core_verify_batch_multi(bbs_issuer_set* p, size_t n, const uint32_t* ite
     if (!n) return BBS_OK;
     if (!item_issuer || !sigs || !status || (n_msgs && !scalars)) return arg_error("null");
     CHECK_COUNTS(n, n_msgs);
-    DISPATCH_SET(S, verify_multi(S, n, item_issuer, sigs, scalars, nullptr, nullptr, n_msgs, status));
+    DISPATCH_SET(S, verify(S->base, n, sigs, MsgIn{scalars, nullptr, nullptr}, n_msgs, status, nullptr, nullptr, S, item_issuer));
 }
 
 int bbs_core_proof_verify_batch_multi(bbs_issuer_set* p, size_t n, const uint32_t* item_issuer, const uint8_t* proofs,
@@ -1501,8 +1334,9 @@ int bbs_core_proof_verify_batch_multi(bbs_issuer_set* p, size_t n, const uint32_
     if (!n) return BBS_OK;
     if (!item_issuer || !proofs || !commit_off || !dis_off || !status) return arg_error("null");
     CHECK_COUNTS(n, 1);
-    if (commit_off[n] > 0xffffffffull || dis_off[n] > 0xffffffffull) return arg_error("batch too large: flat counts must fit in 32 bits");
-    DISPATCH_SET(S, core_proof_verify(S->base, n, proofs, commit, commit_off, idx, dis_scalars, dis_off, ph, ph_len, status, S, item_issuer));
+    TRY(check_flat_counts(n, commit_off, dis_off));
+    DISPATCH_SET(S, proof_verify(S->base, n, proofs, commit, commit_off, idx, MsgIn{dis_scalars, nullptr, nullptr}, dis_off, ph,
+                                 ph_len, status, S, item_issuer));
 }
 int bbs_proof_verify_batch_multi(bbs_issuer_set* p, size_t n, const uint32_t* item_issuer, const uint8_t* proofs,
                                  const uint8_t* commit, const uint64_t* commit_off, const uint32_t* idx, const uint8_t* dis_msgs,
@@ -1512,8 +1346,9 @@ int bbs_proof_verify_batch_multi(bbs_issuer_set* p, size_t n, const uint32_t* it
     if (!n) return BBS_OK;
     if (!item_issuer || !proofs || !commit_off || !dis_off || !dis_msg_off || !status) return arg_error("null");
     CHECK_COUNTS(n, 1);
-    if (commit_off[n] > 0xffffffffull || dis_off[n] > 0xffffffffull) return arg_error("batch too large: flat counts must fit in 32 bits");
-    DISPATCH_SET(S, proof_verify(S->base, n, proofs, commit, commit_off, idx, dis_msgs, dis_msg_off, dis_off, ph, ph_len, status, S, item_issuer));
+    TRY(check_flat_counts(n, commit_off, dis_off));
+    DISPATCH_SET(S, proof_verify(S->base, n, proofs, commit, commit_off, idx, MsgIn{nullptr, dis_msgs, dis_msg_off}, dis_off, ph,
+                                 ph_len, status, S, item_issuer));
 }
 
 // ---- random-linear-combination batch mode ----------------------------------------------------------------
@@ -1523,14 +1358,14 @@ int bbs_rlc_partial_core(bbs_ctx* p, size_t n, const uint8_t* sigs, const uint8_
     Ctx* c = as_ctx(p);
     if (!seed || !parts_out || !status || (n && !sigs) || (n && n_msgs && !scalars)) return arg_error("null (shards must share one seed)");
     CHECK_COUNTS(n, n_msgs);
-    DISPATCH(c, rlc_partial(c, n, sigs, scalars, n_msgs, seed, index_base, parts_out, status));
+    DISPATCH(c, rlc_partial(c, n, sigs, MsgIn{scalars, nullptr, nullptr}, n_msgs, seed, index_base, parts_out, status));
 }
 int bbs_rlc_partial(bbs_ctx* p, size_t n, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* off, uint32_t n_msgs,
                     const uint8_t seed[32], uint64_t index_base, uint8_t* parts_out, uint8_t* status) {
     Ctx* c = as_ctx(p);
     if (!seed || !parts_out || !status || !off || (n && !sigs)) return arg_error("null (shards must share one seed)");
     CHECK_COUNTS(n, n_msgs);
-    DISPATCH(c, rlc_partial_msgs(c, n, sigs, msgs, off, n_msgs, seed, index_base, parts_out, status));
+    DISPATCH(c, rlc_partial(c, n, sigs, MsgIn{nullptr, msgs, off}, n_msgs, seed, index_base, parts_out, status));
 }
 int bbs_rlc_combine(bbs_ctx* p, size_t n_parts, const uint8_t* parts, uint8_t* verdict) {
     Ctx* c = as_ctx(p);
@@ -1544,7 +1379,7 @@ int bbs_rlc_core_verify_batch(bbs_ctx* p, size_t n, const uint8_t* sigs, const u
     CHECK_COUNTS(n, n_msgs);
     uint8_t fresh[32];
     if (!seed) { if (fresh_seed(fresh)) return BBS_E_ARG; seed = fresh; }
-    DISPATCH(c, rlc_verify(c, n, sigs, scalars, nullptr, nullptr, n_msgs, seed, verdict));
+    DISPATCH(c, rlc_verify(c, n, sigs, MsgIn{scalars, nullptr, nullptr}, n_msgs, seed, verdict));
 }
 int bbs_rlc_verify_batch(bbs_ctx* p, size_t n, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* off,
                          uint32_t n_msgs, const uint8_t seed[32], uint8_t* verdict) {
@@ -1553,7 +1388,7 @@ int bbs_rlc_verify_batch(bbs_ctx* p, size_t n, const uint8_t* sigs, const uint8_
     CHECK_COUNTS(n, n_msgs);
     uint8_t fresh[32];
     if (!seed) { if (fresh_seed(fresh)) return BBS_E_ARG; seed = fresh; }
-    DISPATCH(c, rlc_verify(c, n, sigs, nullptr, msgs, off, n_msgs, seed, verdict));
+    DISPATCH(c, rlc_verify(c, n, sigs, MsgIn{nullptr, msgs, off}, n_msgs, seed, verdict));
 }
 #else
 int bbs_rlc_partial_core(bbs_ctx*, size_t, const uint8_t*, const uint8_t*, uint32_t, const uint8_t*, uint64_t, uint8_t*, uint8_t*) { rt_set_error("rlc", "needs the CUDA build"); return BBS_E_CUDA; }
@@ -1603,7 +1438,7 @@ int bbs_core_verify_batch_hdr_dev(bbs_ctx* p, size_t n, const uint8_t* d_sigs, c
     Ctx* c = as_ctx(p);
     CHECK_COUNTS(n, n_msgs);
     if (!d_hdr_off) return arg_error("hdr_off is null");
-    if (c && !c->per_item_header) return arg_error("per-item headers need a context created with BBS_CTX_PER_ITEM_HEADER");
+    TRY(check_hdr_flag(c, d_hdr_off));
     DISPATCH(c, core_verify_hdr_dev(c, n, d_sigs, d_scalars, n_msgs, d_headers, d_hdr_off, d_status, (rt_stream_t)stream));
 }
 int bbs_core_proof_verify_batch_hdr_dev(bbs_ctx* p, size_t n, const uint8_t* d_proofs, const uint8_t* d_commit,
@@ -1613,7 +1448,7 @@ int bbs_core_proof_verify_batch_hdr_dev(bbs_ctx* p, size_t n, const uint8_t* d_p
     Ctx* c = as_ctx(p);
     CHECK_COUNTS(n, 1);
     if (!d_ph_off) return arg_error("ph_off is null");
-    if (c && d_hdr_off && !c->per_item_header) return arg_error("per-item headers need a context created with BBS_CTX_PER_ITEM_HEADER");
+    TRY(check_hdr_flag(c, d_hdr_off));
     DISPATCH(c, core_proof_verify_hdr_dev(c, n, d_proofs, d_commit, d_commit_off, d_idx, d_dis_scalars, d_dis_off, d_headers,
                                           d_hdr_off, d_phs, d_ph_off, d_status, (rt_stream_t)stream));
 }
