@@ -84,6 +84,10 @@ SYMBOLS = {
                                             C.c_void_p]),
     "bbs_rlc_verify_batch": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32,
                                        C.c_void_p, C.c_void_p]),
+    "bbs_rlc_core_proof_verify_batch": (C.c_int, [C.c_void_p, C.c_size_t] + [C.c_void_p] * 7 + [C.c_size_t] + [C.c_void_p] * 3),
+    "bbs_rlc_proof_verify_batch": (C.c_int, [C.c_void_p, C.c_size_t] + [C.c_void_p] * 8 + [C.c_size_t] + [C.c_void_p] * 3),
+    "bbs_rlc_core_proof_verify_batch_hdr": (C.c_int, [C.c_void_p, C.c_size_t] + [C.c_void_p] * 13),
+    "bbs_rlc_proof_verify_batch_hdr": (C.c_int, [C.c_void_p, C.c_size_t] + [C.c_void_p] * 14),
     "bbs_msg_to_scalars_dev": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "bbs_core_verify_batch_dev": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p,
                                             C.c_void_p]),

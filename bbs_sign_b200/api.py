@@ -385,32 +385,7 @@ class BatchContext:
                                 disclosed_indexes: Sequence[Sequence[int]], *, headers: Optional[Sequence[bytes]] = None) -> np.ndarray:
         """`ph`: one presentation header for the batch or one per proof; `headers`: one header per proof instead of the
         context's (needs `per_item_headers=True`)"""
-        n = len(proofs)
-        st = np.full(n, 255, dtype=np.uint8)
-        # InvalidIndicesAndMessagesLength (proof_verify.rs:144-146) is a property of the host-side lists
-        bad = [len(disclosed_scalars[i]) != len(disclosed_indexes[i]) for i in range(n)]
-        keep = [i for i in range(n) if not bad[i]]
-        if keep:
-            fixed, commit, commit_off, idx, dis_off = self._pack_proofs([proofs[i] for i in keep], [disclosed_indexes[i] for i in keep])
-            sc = np.frombuffer(b"".join(s for i in keep for s in disclosed_scalars[i]), dtype=np.uint8)
-            if sc.size == 0:
-                sc = np.zeros(1, np.uint8)
-            out = np.full(len(keep), 255, dtype=np.uint8)
-            if headers is not None or _is_per_item(ph):
-                hb, hoff, pb, poff = self._per_item_ph_args(keep, n, ph, headers)
-                self._check(self.lib.bbs_core_proof_verify_batch_hdr(self._h, len(keep), _ptr(fixed), _ptr(commit), _ptr(commit_off),
-                                                                     _ptr(idx), _ptr(sc), _ptr(dis_off), _ptr(hb), _ptr(hoff),
-                                                                     _ptr(pb), _ptr(poff), _ptr(out)), "bbs_core_proof_verify_batch_hdr")
-            else:
-                phb = _buf(ph) if len(ph) else None
-                self._check(self.lib.bbs_core_proof_verify_batch(self._h, len(keep), _ptr(fixed), _ptr(commit), _ptr(commit_off),
-                                                                 _ptr(idx), _ptr(sc), _ptr(dis_off), _ptr(phb), len(ph), _ptr(out)),
-                            "bbs_core_proof_verify_batch")
-            st[keep] = out
-        for i in range(n):
-            if bad[i]:
-                st[i] = self._length_error_status(proofs[i], disclosed_indexes[i])
-        return st
+        return self._proof_verify(True, proofs, ph, disclosed_scalars, disclosed_indexes, headers)[0]
 
     def _length_error_status(self, proof, idxs):
         # reference order (proof_verify.rs:139-146): index range check first, then the length check
@@ -421,29 +396,61 @@ class BatchContext:
                            disclosed_indexes: Sequence[Sequence[int]], *, headers: Optional[Sequence[bytes]] = None) -> np.ndarray:
         """`ph`: one presentation header for the batch or one per proof; `headers`: one header per proof instead of the
         context's (needs `per_item_headers=True`)"""
+        return self._proof_verify(False, proofs, ph, disclosed_messages, disclosed_indexes, headers)[0]
+
+    def rlc_core_proof_verify_batch(self, proofs, ph, disclosed_scalars: Sequence[Sequence[bytes]],
+                                    disclosed_indexes: Sequence[Sequence[int]], *, headers: Optional[Sequence[bytes]] = None,
+                                    seed: Optional[bytes] = None):
+        """`core_proof_verify_batch` with the pairing half checked by one random linear combination
+        (bbs_rlc_core_proof_verify_batch*, include/bbs_b200.h).  Returns (status, combined): the statuses are those of
+        `core_proof_verify_batch` (an ACCEPT holds except with probability 2^-128 over the seed); `combined` is ST_ACCEPT
+        when the one combined pairing check held (or no proof reached it), ST_REJECT when it failed and the per-item
+        pairing decided instead.  `seed=None` (the default) lets the library draw the seed after it has the batch; pass a
+        seed only for reproducible tests: a seed the submitter of the batch can predict lets crafted proofs pass."""
+        return self._proof_verify(True, proofs, ph, disclosed_scalars, disclosed_indexes, headers, rlc=True, seed=seed)
+
+    def rlc_proof_verify_batch(self, proofs, ph, disclosed_messages: Sequence[Sequence[bytes]],
+                               disclosed_indexes: Sequence[Sequence[int]], *, headers: Optional[Sequence[bytes]] = None,
+                               seed: Optional[bytes] = None):
+        """`proof_verify_batch` with the pairing half checked by one random linear combination; returns (status, combined)
+        as `rlc_core_proof_verify_batch`."""
+        return self._proof_verify(False, proofs, ph, disclosed_messages, disclosed_indexes, headers, rlc=True, seed=seed)
+
+    def _proof_verify(self, core: bool, proofs, ph, disclosed, disclosed_indexes, headers, rlc: bool = False,
+                      seed: Optional[bytes] = None):
+        """(status, combined) of the proof verify calls: `disclosed` holds message scalars (core) or messages.  Proofs whose
+        disclosed lists differ in length never reach the library; the combined verdict covers the rest (ST_ACCEPT when
+        none is left, or without rlc)."""
         n = len(proofs)
         st = np.full(n, 255, dtype=np.uint8)
-        bad = [len(disclosed_messages[i]) != len(disclosed_indexes[i]) for i in range(n)]
+        combined = np.full(1, ST_ACCEPT, dtype=np.uint8)
+        # InvalidIndicesAndMessagesLength (proof_verify.rs:144-146) is a property of the host-side lists
+        bad = [len(disclosed[i]) != len(disclosed_indexes[i]) for i in range(n)]
         keep = [i for i in range(n) if not bad[i]]
         if keep:
             fixed, commit, commit_off, idx, dis_off = self._pack_proofs([proofs[i] for i in keep], [disclosed_indexes[i] for i in keep])
-            flat, moffs = _pack_ragged([m for i in keep for m in disclosed_messages[i]])
+            if core:
+                dis = (np.frombuffer(b"".join(s for i in keep for s in disclosed[i]), dtype=np.uint8),)
+                if dis[0].size == 0:
+                    dis = (np.zeros(1, np.uint8),)
+            else:
+                dis = _pack_ragged([m for i in keep for m in disclosed[i]])
             out = np.full(len(keep), 255, dtype=np.uint8)
+            tail = (_ptr(_buf(seed)) if seed is not None else None, _ptr(out), _ptr(combined)) if rlc else (_ptr(out),)
+            name = ("bbs_rlc_" if rlc else "bbs_") + ("core_" if core else "") + "proof_verify_batch"
+            head = (self._h, len(keep), _ptr(fixed), _ptr(commit), _ptr(commit_off), _ptr(idx)) + tuple(_ptr(d) for d in dis) + (_ptr(dis_off),)
             if headers is not None or _is_per_item(ph):
                 hb, hoff, pb, poff = self._per_item_ph_args(keep, n, ph, headers)
-                self._check(self.lib.bbs_proof_verify_batch_hdr(self._h, len(keep), _ptr(fixed), _ptr(commit), _ptr(commit_off),
-                                                                _ptr(idx), _ptr(flat), _ptr(moffs), _ptr(dis_off), _ptr(hb), _ptr(hoff),
-                                                                _ptr(pb), _ptr(poff), _ptr(out)), "bbs_proof_verify_batch_hdr")
+                name += "_hdr"
+                self._check(getattr(self.lib, name)(*head, _ptr(hb), _ptr(hoff), _ptr(pb), _ptr(poff), *tail), name)
             else:
                 phb = _buf(ph) if len(ph) else None
-                self._check(self.lib.bbs_proof_verify_batch(self._h, len(keep), _ptr(fixed), _ptr(commit), _ptr(commit_off), _ptr(idx),
-                                                            _ptr(flat), _ptr(moffs), _ptr(dis_off), _ptr(phb), len(ph), _ptr(out)),
-                            "bbs_proof_verify_batch")
+                self._check(getattr(self.lib, name)(*head, _ptr(phb), len(ph), *tail), name)
             st[keep] = out
         for i in range(n):
             if bad[i]:
                 st[i] = self._length_error_status(proofs[i], disclosed_indexes[i])
-        return st
+        return st, int(combined[0])
 
 
 class IssuerSet:

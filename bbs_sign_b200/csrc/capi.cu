@@ -17,7 +17,7 @@ constexpr int TPB_LIGHT = 128;   // hashing
 
 // CUDA events on the launching stream: mark k sits before kernel k of a batch call (last mark = end)
 struct ProfEvents {
-    static constexpr int MAX = 8;
+    static constexpr int MAX = 10;
 #ifndef BBS_HOSTSIM
     cudaEvent_t ev[MAX] = {};
     int used = 0;
@@ -93,11 +93,12 @@ struct Ctx {
     DevBuf s_sigs, s_scalars, s_msgs, s_offsets, s_pair, s_flags, s_status, s_out, s_out2;
     DevBuf s_commit, s_commit_off, s_dis_idx, s_dis_scalars, s_dis_off, s_ph, s_dis_msgs, s_dis_msg_off;
     DevBuf s_hdr, s_hdr_off, s_ph_off, s_ik, s_idom, s_ifl;     // per-item headers / phs and the ItemKeyView arrays
+    DevBuf s_rlcp;                   // rlc proof calls: the combined pairing record, its flag word and its status
     template <class Fn> void each_buffer(Fn f) {
         DevBuf* all[] = {&pk_comp, &gens_comp, &api_id, &header, &dst_h2s, &dst_map, &gens, &W, &K, &domain, &tab, &wbase,
                          &lines, &lines_coop, &s_rand, &s_rand_off, &s_sk, &s_g1v, &s_g1f, &s_g1st, &s_g1t, &s_gscr, &s_rlc_pt, &s_rlc_sc, &s_rlc_parts, &s_rlc_bad, &s_msm_pts, &s_msm_kv, &s_msm_idx, &s_msm_entries, &s_msm_buckets, &misc, &s_sigs, &s_scalars, &s_msgs, &s_offsets, &s_pair, &s_flags, &s_status, &s_out,
                          &s_out2, &s_commit, &s_commit_off, &s_dis_idx, &s_dis_scalars, &s_dis_off, &s_ph, &s_dis_msgs,
-                         &s_dis_msg_off, &prefix, &s_hdr, &s_hdr_off, &s_ph_off, &s_ik, &s_idom, &s_ifl};
+                         &s_dis_msg_off, &prefix, &s_hdr, &s_hdr_off, &s_ph_off, &s_ik, &s_idom, &s_ifl, &s_rlcp};
         for (DevBuf* b : all) f(b);
     }
     void release_all() { each_buffer([](DevBuf* b) { b->release(); }); }
@@ -123,6 +124,10 @@ struct IssuerSet {
 // The messages of a host-buffer batch call: byte messages `msgs` with their count + 1 offsets `off`, or (off == nullptr)
 // their scalars, 32 bytes each
 struct MsgIn { const uint8_t* scalars; const uint8_t* msgs; const uint64_t* off; };
+
+// The random-linear-combination form of a proof verify call (bbs_rlc_*proof_verify_batch*): the 32-byte coefficient seed
+// and where the combined check's verdict goes (may be null)
+struct RlcProofIn { const uint8_t* seed; uint8_t* combined; };
 
 #define TRY(expr) do { int rc_ = (expr); if (rc_) return rc_; } while (0)
 #define PROF(c, slot, s) do { if ((c)->profile) TRY((c)->prof.mark(slot, s)); } while (0)
@@ -262,22 +267,24 @@ struct Impl {
         return BBS_OK;
     }
 
-    // S != nullptr: multi-issuer batch, item i is checked against the lines of issuer d_item_issuer[i] of the set
-    static int pairing_dev(Ctx* c, size_t n, uint8_t* d_status, rt_stream_t s, const IssuerSet* S = nullptr) {
+    // S != nullptr: multi-issuer batch, item i is checked against the lines of issuer d_item_issuer[i] of the set.
+    // The records and flags are the batch's (s_pair, s_flags) unless d_pair / d_flags name others.
+    static int pairing_dev(Ctx* c, size_t n, uint8_t* d_status, rt_stream_t s, const IssuerSet* S = nullptr,
+                           const uint32_t* d_pair = nullptr, const uint32_t* d_flags = nullptr) {
         const uint32_t* d_issuer = S ? (const uint32_t*)S->item_issuer.p : nullptr;
+        if (!d_pair) { d_pair = (const uint32_t*)c->s_pair.p; d_flags = (const uint32_t*)c->s_flags.p; }
 #ifndef BBS_HOSTSIM
         if (S || (c->coop && !c->force_per_thread)) {
             TRY(c->s_gscr.reserve(coop_gscratch_size<C>(n)));
-            CoopArgs ca{(const uint32_t*)(S ? S->lines.p : c->lines_coop.p), (const uint32_t*)c->s_pair.p,
-                        (const uint32_t*)c->s_flags.p, d_status, (uint32_t*)c->s_gscr.p, (uint32_t)n, d_issuer,
+            CoopArgs ca{(const uint32_t*)(S ? S->lines.p : c->lines_coop.p), d_pair, d_flags, d_status, (uint32_t*)c->s_gscr.p, (uint32_t)n, d_issuer,
                         S ? S->line_stride : 0u, c->pair_split_max};
             TRY((launch_pairing_coop<C>(ca, s)));
             c->launches += n ? 1 : 0;
             return BBS_OK;
         }
 #endif
-        PairingArgs pa{S ? (const uint32_t*)S->lines.p : c->view.lines, (const uint32_t*)c->s_pair.p,
-                       (const uint32_t*)c->s_flags.p, d_status, d_issuer, S ? S->line_stride : 0u};
+        PairingArgs pa{S ? (const uint32_t*)S->lines.p : c->view.lines, d_pair, d_flags, d_status, d_issuer,
+                       S ? S->line_stride : 0u};
         TRY((launch_pairing<C>(pa, (uint32_t)n, s)));
         c->launches += n ? 1 : 0;
         return BBS_OK;
@@ -527,7 +534,7 @@ struct Impl {
                                      const uint64_t* d_commit_off, const uint32_t* d_idx, const uint8_t* d_dis_scalars,
                                      const uint64_t* d_dis_off, const uint8_t* d_ph, size_t ph_len, uint8_t* d_status,
                                      rt_stream_t s, const IssuerSet* S = nullptr, const ItemKeyView* item = nullptr,
-                                     const uint64_t* d_ph_off = nullptr) {
+                                     const uint64_t* d_ph_off = nullptr, const RlcProofIn* rlc = nullptr) {
         TRY(c->s_pair.reserve(n * 6 * C::Fp::N * 4));
         TRY(c->s_flags.reserve(n * 4));
         ProofG1Args a{c->view, d_proofs, d_commit, d_commit_off, d_idx, d_dis_scalars, d_dis_off, d_ph,
@@ -550,6 +557,13 @@ struct Impl {
         TRY((launch_proof_g1<C>(a, (uint32_t)n, s)));
         c->launches += n ? (a.part_t1 ? 2 : 1) : 0;
         PROF(c, 2, s);
+#ifndef BBS_HOSTSIM
+        if (rlc) {
+            TRY(rlc_proof_pairing_dev(c, n, *rlc, d_status, s));
+            if (item) c->prof.xslot = 9;
+            return BBS_OK;
+        }
+#endif
         TRY(pairing_dev(c, n, d_status, s, S));
         PROF(c, 3, s);
         if (item) c->prof.xslot = 3;
@@ -609,8 +623,9 @@ struct Impl {
 #ifndef BBS_HOSTSIM
     // digits per 128-bit value for the bucket MSM.  Cost in field multiplications: 11 per bucket addition, inflated by the
     // quantisation of buckets over the persistent threads of msm_bucket_kernel (u buckets per thread), plus ~47 per bucket
-    // for the reduction (measured on B200 at n = 65,536 and 524,288: profiles/summary_r01.md)
-    static MsmPlan rlc_plan(size_t n, uint32_t force) {      // force != 0: bbs_ctx_set_rlc_windows (tests: other geometries)
+    // for the reduction (measured on B200 at n = 65,536 and 524,288: profiles/summary_r01.md).  `values`: 128-bit values
+    // per item (3 for signatures, 2 for proofs).
+    static MsmPlan rlc_plan(size_t n, uint32_t force, double values = 3.0) {   // force != 0: bbs_ctx_set_rlc_windows (tests)
         uint32_t best = 32;
         double best_cost = 1e300;
         for (uint32_t W = 8; W <= 32; W++) {
@@ -619,7 +634,7 @@ struct Impl {
             for (uint32_t w = 0; w < W; w++) used += (double)(1u << (((w + 1) * 128) / W - (w * 128) / W));
             used *= rows / W;
             const double u = used / (148.0 * 512.0);
-            const double cost = 11.0 * 3.0 * W * (double)n * (1.0 + 1.0 / u) + 47.0 * rows * (double)(1u << c);
+            const double cost = 11.0 * values * W * (double)n * (1.0 + 1.0 / u) + 47.0 * rows * (double)(1u << c);
             if (force ? force == W : cost < best_cost) { best = W; best_cost = cost; }
         }
         MsmPlan p;
@@ -748,6 +763,77 @@ struct Impl {
         TRY(pairing_dev(c, 1, (uint8_t*)c->s_status.p, s));
         return finish_status(c, 1, verdict);
     }
+    // The pairing half of a proof batch by one random linear combination (rlc_msm.cuh, proof batches): after the G1 half,
+    // the items without FL_DONE are checked with ONE pairing of S1 = sum r_i Abar_i and S2 = sum r_i (-Bbar_i).  If it
+    // holds they are accepted; if not, the per-item pairing kernel decides them from their records, which the MSM leaves
+    // intact (the combined record has its own slot, s_rlcp).  Profiling slots 2..8: prep, scan + scatter, buckets,
+    // reduction, finish, combined pairing, acceptance or per-item pairing.
+    static int rlc_proof_pairing_dev(Ctx* c, size_t n, const RlcProofIn& rlc, uint8_t* d_status, rt_stream_t s) {
+        const MsmPlan plan = rlc_plan(n, c->rlc_windows, 2.0);
+        const size_t nb = (size_t)plan.rows << plan.c, PT = 3 * C::Fp::N * 4, PW = 6 * C::Fp::N;
+        TRY(c->s_msm_kv.reserve(n * 48));
+        TRY(c->s_msm_idx.reserve((3 * nb + 5) * 4));                        // next (4 words) | counts | offsets (nb + 1) | cursor
+        TRY(c->s_msm_entries.reserve(n * 2 * plan.W * 4));
+        TRY(c->s_msm_buckets.reserve(nb * PT));
+        TRY(c->s_rlc_pt.reserve((size_t)plan.rows * plan.red_blocks * PT));
+        TRY(c->s_rlc_parts.reserve(2 * C::G1_BYTES));
+        TRY(c->s_rlc_bad.reserve(4));
+        TRY(c->s_rlcp.reserve((PW + 2) * 4));                               // record | flags | status
+        uint32_t* next = (uint32_t*)c->s_msm_idx.p;
+        uint32_t* counts = next + 4;
+        uint32_t* offsets = counts + nb;
+        uint32_t* cursor = offsets + nb + 1;
+        uint32_t* pair = (uint32_t*)c->s_rlcp.p;
+        uint8_t* verdict_d = (uint8_t*)(pair + PW + 1);
+        TRY(rt_memset(c->s_rlc_bad.p, 0, 4, s));
+        TRY(rt_memset(next, 0, (nb + 4) * 4, s));
+        RlcProofPrepArgs pa{};
+        pa.plan = plan; pa.flags = (const uint32_t*)c->s_flags.p; pa.kv = (uint32_t*)c->s_msm_kv.p; pa.counts = counts;
+        pa.live = (uint32_t*)c->s_rlc_bad.p; pa.n = (uint32_t)n;
+        for (int i = 0; i < 8; i++)
+            pa.seed[i] = ((uint32_t)rlc.seed[4 * i] << 24) | ((uint32_t)rlc.seed[4 * i + 1] << 16) |
+                         ((uint32_t)rlc.seed[4 * i + 2] << 8) | rlc.seed[4 * i + 3];
+        TRY((launch_rlc_proof_prep<C>(pa, s)));
+        c->launches += 1;
+        PROF(c, 3, s);
+        uint32_t live = 0;
+        TRY(rt_d2h(&live, c->s_rlc_bad.p, 4, s));
+        TRY(rt_sync(s));
+        uint8_t verdict = ST_ACCEPT;
+        if (live) {                                                          // else every status is final already
+            TRY(launch_msm_scan(counts, offsets, cursor, (uint32_t)nb, s));
+            MsmScatterArgs sa{plan, (const uint32_t*)c->s_msm_kv.p, cursor, (uint32_t*)c->s_msm_entries.p, (uint32_t)n};
+            TRY((launch_msm_scatter<C>(sa, s)));
+            PROF(c, 4, s);
+            MsmBucketArgs ba{offsets, (const uint32_t*)c->s_msm_entries.p, (const uint32_t*)c->s_pair.p,
+                             (uint32_t*)c->s_msm_buckets.p, next, (uint32_t)nb};
+            TRY((launch_msm_bucket_pair<C>(ba, s)));
+            PROF(c, 5, s);
+            MsmReduceArgs ra{plan, (const uint32_t*)c->s_msm_buckets.p, (uint32_t*)c->s_rlc_pt.p};
+            TRY((launch_msm_reduce<C>(ra, s)));
+            PROF(c, 6, s);
+            // the signature mode's finish kernel with no prep blocks and no messages: its Fr sums and fixed-base term are
+            // zero, so it yields S1 and S2 as they are
+            RlcMsmFinishArgs f{c->view, plan, (const uint32_t*)c->s_rlc_pt.p, nullptr, 0u, 0u, (uint8_t*)c->s_rlc_parts.p,
+                               pair, pair + PW, verdict_d};
+            TRY((launch_rlc_msm_finish<C>(f, s)));
+            c->launches += 5;
+            PROF(c, 7, s);
+            TRY(pairing_dev(c, 1, verdict_d, s, nullptr, pair, pair + PW));
+            TRY(rt_d2h(&verdict, verdict_d, 1, s));
+            TRY(rt_sync(s));
+            PROF(c, 8, s);
+            if (verdict == ST_ACCEPT) {
+                TRY((launch_rlc_proof_accept<C>((const uint32_t*)c->s_flags.p, d_status, (uint32_t)n, s)));
+                c->launches += 1;
+            } else {
+                TRY(pairing_dev(c, n, d_status, s));
+            }
+            PROF(c, 9, s);
+        }
+        if (rlc.combined) *rlc.combined = verdict;
+        return BBS_OK;
+    }
 #endif
 
     // ---- host-buffer calls ------------------------------------------------------------------------------------------
@@ -865,11 +951,13 @@ struct Impl {
     }
     // proof_verify / core_proof_verify: `dis` holds the disclosed messages (or their scalars); ph_off != nullptr: per-item
     // phs in `ph`; hdr_off != nullptr: per-item headers (bbs_*proof_verify_batch_hdr); S != nullptr: the issuer of each
-    // item in item_issuer (bbs_*proof_verify_batch_multi, c = S->base)
+    // item in item_issuer (bbs_*proof_verify_batch_multi, c = S->base); rlc != nullptr: the pairing half by one random
+    // linear combination (bbs_rlc_*proof_verify_batch*)
     static int proof_verify(Ctx* c, size_t n, const uint8_t* proofs, const uint8_t* commit, const uint64_t* commit_off,
                             const uint32_t* idx, const MsgIn& dis, const uint64_t* dis_off, const uint8_t* ph, size_t ph_len,
                             uint8_t* status, IssuerSet* S = nullptr, const uint32_t* item_issuer = nullptr,
-                            const uint64_t* ph_off = nullptr, const uint8_t* headers = nullptr, const uint64_t* hdr_off = nullptr) {
+                            const uint64_t* ph_off = nullptr, const uint8_t* headers = nullptr, const uint64_t* hdr_off = nullptr,
+                            const RlcProofIn* rlc = nullptr) {
         rt_stream_t s = c->stream;
         TRY(stage_scalars(c, dis_off[n], dis, c->s_dis_msgs, c->s_dis_msg_off, c->s_dis_scalars, false));
         ItemKeyView item{};
@@ -890,7 +978,7 @@ struct Impl {
                                   (const uint64_t*)c->s_commit_off.p, (const uint32_t*)c->s_dis_idx.p,
                                   (const uint8_t*)c->s_dis_scalars.p, (const uint64_t*)c->s_dis_off.p,
                                   (const uint8_t*)c->s_ph.p, ph_len, (uint8_t*)c->s_status.p, s, S, hdr_off ? &item : nullptr,
-                                  ph_off ? (const uint64_t*)c->s_ph_off.p : nullptr));
+                                  ph_off ? (const uint64_t*)c->s_ph_off.p : nullptr, rlc));
         return finish_status(c, n, status);
     }
 };
@@ -1390,12 +1478,82 @@ int bbs_rlc_verify_batch(bbs_ctx* p, size_t n, const uint8_t* sigs, const uint8_
     if (!seed) { if (fresh_seed(fresh)) return BBS_E_ARG; seed = fresh; }
     DISPATCH(c, rlc_verify(c, n, sigs, MsgIn{nullptr, msgs, off}, n_msgs, seed, verdict));
 }
+// proof verification with the pairing half by one random linear combination: the arguments of the call without rlc_,
+// then the seed (NULL = drawn here, after the batch has been handed over) and the combined check's verdict
+#define RLC_PROOF_ARGS(seed, combined)                                                                              \
+    if (!n) { if (combined) *(combined) = BBS_ST_ACCEPT; return BBS_OK; }                                           \
+    if (n >= (1ull << 31)) return arg_error("batch too large for the rlc mode: n must be below 2^31");             \
+    uint8_t fresh[32];                                                                                              \
+    if (!seed) { if (fresh_seed(fresh)) return BBS_E_ARG; seed = fresh; }                                           \
+    const RlcProofIn rlc{seed, combined}
+int bbs_rlc_core_proof_verify_batch(bbs_ctx* p, size_t n, const uint8_t* proofs, const uint8_t* commit,
+                                    const uint64_t* commit_off, const uint32_t* idx, const uint8_t* dis_scalars,
+                                    const uint64_t* dis_off, const uint8_t* ph, size_t ph_len, const uint8_t* seed,
+                                    uint8_t* status, uint8_t* combined) {
+    Ctx* c = as_ctx(p);
+    if (n && (!proofs || !commit_off || !dis_off || !status)) return arg_error("null");
+    CHECK_COUNTS(n, 1);
+    if (n) TRY(check_flat_counts(n, commit_off, dis_off));
+    RLC_PROOF_ARGS(seed, combined);
+    DISPATCH(c, proof_verify(c, n, proofs, commit, commit_off, idx, MsgIn{dis_scalars, nullptr, nullptr}, dis_off, ph, ph_len, status,
+                             nullptr, nullptr, nullptr, nullptr, nullptr, &rlc));
+}
+int bbs_rlc_proof_verify_batch(bbs_ctx* p, size_t n, const uint8_t* proofs, const uint8_t* commit, const uint64_t* commit_off,
+                               const uint32_t* idx, const uint8_t* dis_msgs, const uint64_t* dis_msg_off,
+                               const uint64_t* dis_off, const uint8_t* ph, size_t ph_len, const uint8_t* seed, uint8_t* status,
+                               uint8_t* combined) {
+    Ctx* c = as_ctx(p);
+    if (n && (!proofs || !commit_off || !dis_off || !dis_msg_off || !status)) return arg_error("null");
+    CHECK_COUNTS(n, 1);
+    if (n) TRY(check_flat_counts(n, commit_off, dis_off));
+    RLC_PROOF_ARGS(seed, combined);
+    DISPATCH(c, proof_verify(c, n, proofs, commit, commit_off, idx, MsgIn{nullptr, dis_msgs, dis_msg_off}, dis_off, ph, ph_len, status,
+                             nullptr, nullptr, nullptr, nullptr, nullptr, &rlc));
+}
+int bbs_rlc_core_proof_verify_batch_hdr(bbs_ctx* p, size_t n, const uint8_t* proofs, const uint8_t* commit,
+                                        const uint64_t* commit_off, const uint32_t* idx, const uint8_t* dis_scalars,
+                                        const uint64_t* dis_off, const uint8_t* headers, const uint64_t* hdr_off,
+                                        const uint8_t* phs, const uint64_t* ph_off, const uint8_t* seed, uint8_t* status,
+                                        uint8_t* combined) {
+    Ctx* c = as_ctx(p);
+    if (n && (!proofs || !commit_off || !dis_off || !status || !ph_off)) return arg_error("null");
+    CHECK_COUNTS(n, 1);
+    if (n) {
+        TRY(check_flat_counts(n, commit_off, dis_off));
+        TRY(check_hdr_args(c, n, headers, hdr_off, false));
+        TRY(check_items(n, phs, ph_off, "ph"));
+    }
+    RLC_PROOF_ARGS(seed, combined);
+    DISPATCH(c, proof_verify(c, n, proofs, commit, commit_off, idx, MsgIn{dis_scalars, nullptr, nullptr}, dis_off, phs, 0, status,
+                             nullptr, nullptr, ph_off, headers, hdr_off, &rlc));
+}
+int bbs_rlc_proof_verify_batch_hdr(bbs_ctx* p, size_t n, const uint8_t* proofs, const uint8_t* commit,
+                                   const uint64_t* commit_off, const uint32_t* idx, const uint8_t* dis_msgs,
+                                   const uint64_t* dis_msg_off, const uint64_t* dis_off, const uint8_t* headers,
+                                   const uint64_t* hdr_off, const uint8_t* phs, const uint64_t* ph_off, const uint8_t* seed,
+                                   uint8_t* status, uint8_t* combined) {
+    Ctx* c = as_ctx(p);
+    if (n && (!proofs || !commit_off || !dis_off || !dis_msg_off || !status || !ph_off)) return arg_error("null");
+    CHECK_COUNTS(n, 1);
+    if (n) {
+        TRY(check_flat_counts(n, commit_off, dis_off));
+        TRY(check_hdr_args(c, n, headers, hdr_off, false));
+        TRY(check_items(n, phs, ph_off, "ph"));
+    }
+    RLC_PROOF_ARGS(seed, combined);
+    DISPATCH(c, proof_verify(c, n, proofs, commit, commit_off, idx, MsgIn{nullptr, dis_msgs, dis_msg_off}, dis_off, phs, 0, status,
+                             nullptr, nullptr, ph_off, headers, hdr_off, &rlc));
+}
 #else
 int bbs_rlc_partial_core(bbs_ctx*, size_t, const uint8_t*, const uint8_t*, uint32_t, const uint8_t*, uint64_t, uint8_t*, uint8_t*) { rt_set_error("rlc", "needs the CUDA build"); return BBS_E_CUDA; }
 int bbs_rlc_partial(bbs_ctx*, size_t, const uint8_t*, const uint8_t*, const uint64_t*, uint32_t, const uint8_t*, uint64_t, uint8_t*, uint8_t*) { rt_set_error("rlc", "needs the CUDA build"); return BBS_E_CUDA; }
 int bbs_rlc_combine(bbs_ctx*, size_t, const uint8_t*, uint8_t*) { rt_set_error("rlc", "needs the CUDA build"); return BBS_E_CUDA; }
 int bbs_rlc_core_verify_batch(bbs_ctx*, size_t, const uint8_t*, const uint8_t*, uint32_t, const uint8_t*, uint8_t*) { rt_set_error("rlc", "needs the CUDA build"); return BBS_E_CUDA; }
 int bbs_rlc_verify_batch(bbs_ctx*, size_t, const uint8_t*, const uint8_t*, const uint64_t*, uint32_t, const uint8_t*, uint8_t*) { rt_set_error("rlc", "needs the CUDA build"); return BBS_E_CUDA; }
+int bbs_rlc_core_proof_verify_batch(bbs_ctx*, size_t, const uint8_t*, const uint8_t*, const uint64_t*, const uint32_t*, const uint8_t*, const uint64_t*, const uint8_t*, size_t, const uint8_t*, uint8_t*, uint8_t*) { rt_set_error("rlc", "needs the CUDA build"); return BBS_E_CUDA; }
+int bbs_rlc_proof_verify_batch(bbs_ctx*, size_t, const uint8_t*, const uint8_t*, const uint64_t*, const uint32_t*, const uint8_t*, const uint64_t*, const uint64_t*, const uint8_t*, size_t, const uint8_t*, uint8_t*, uint8_t*) { rt_set_error("rlc", "needs the CUDA build"); return BBS_E_CUDA; }
+int bbs_rlc_core_proof_verify_batch_hdr(bbs_ctx*, size_t, const uint8_t*, const uint8_t*, const uint64_t*, const uint32_t*, const uint8_t*, const uint64_t*, const uint8_t*, const uint64_t*, const uint8_t*, const uint64_t*, const uint8_t*, uint8_t*, uint8_t*) { rt_set_error("rlc", "needs the CUDA build"); return BBS_E_CUDA; }
+int bbs_rlc_proof_verify_batch_hdr(bbs_ctx*, size_t, const uint8_t*, const uint8_t*, const uint64_t*, const uint32_t*, const uint8_t*, const uint64_t*, const uint64_t*, const uint8_t*, const uint64_t*, const uint8_t*, const uint64_t*, const uint8_t*, uint8_t*, uint8_t*) { rt_set_error("rlc", "needs the CUDA build"); return BBS_E_CUDA; }
 #endif
 
 int bbs_msg_to_scalars_dev(bbs_ctx* p, size_t count, const uint8_t* d_msgs, const uint64_t* d_off, uint8_t* d_out, void* stream) {

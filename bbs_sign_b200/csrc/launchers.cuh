@@ -34,6 +34,10 @@ template <class C> int launch_msm_bucket(const MsmBucketArgs& a, rt_stream_t s);
 template <class C> int launch_msm_reduce(const MsmReduceArgs& a, rt_stream_t s);
 template <class C> int launch_rlc_msm_finish(const RlcMsmFinishArgs& a, rt_stream_t s);
 template <class C> int launch_rlc_combine(const RlcCombineArgs& a, rt_stream_t s);
+// the proof form of the mode: prep, buckets over the pairing records, acceptance of the undecided items
+template <class C> int launch_rlc_proof_prep(const RlcProofPrepArgs& a, rt_stream_t s);
+template <class C> int launch_msm_bucket_pair(const MsmBucketArgs& a, rt_stream_t s);
+template <class C> int launch_rlc_proof_accept(const uint32_t* flags, uint8_t* status, uint32_t n, rt_stream_t s);
 // cooperative pairing kernel; gscratch must hold coop_gscratch_size<C>(n) bytes
 template <class C> int launch_pairing_coop(const CoopArgs& a, rt_stream_t s);
 template <class C> size_t coop_gscratch_size(size_t n);

@@ -147,7 +147,9 @@ struct MsmBucketArgs { const uint32_t* offsets; const uint32_t* entries; const u
 // Persistent threads (grid = resident capacity): every lane takes the next unprocessed bucket from a global counter and
 // adds its points one per trip of ONE flat loop, so lanes whose bucket ends early fetch another bucket while the rest of
 // the warp keeps adding: bucket sizes (Poisson around n / 2^c) no longer cost max-over-lanes per warp.
-template <class C> __global__ void __launch_bounds__(128, 4) msm_bucket_kernel(const MsmBucketArgs a) {
+// PAIR = false: pts = n affine points, entry bit 31 = phi(point).  PAIR = true: pts = the proof pairing records
+// (PAIR_WORDS per item), entry bit 31 = the record's second point (-Bbar at word 3 FPN) instead of its first (Abar).
+template <class C, bool PAIR> __device__ __forceinline__ void msm_bucket_run(const MsmBucketArgs& a) {
     using F = typename C::Fp;
     BBS_A16 uint32_t acc[G1J];
     uint32_t b = 0, j = 0, end = 0;
@@ -167,11 +169,12 @@ template <class C> __global__ void __launch_bounds__(128, 4) msm_bucket_kernel(c
             continue;
         }
         const uint32_t e = a.entries[j++];
-        const uint4* src = (const uint4*)(a.pts + (size_t)(e & 0x7fffffffu) * G1A);
+        const uint4* src = PAIR ? (const uint4*)(a.pts + (size_t)(e & 0x7fffffffu) * PAIR_WORDS + ((e >> 31) ? 3 * FPN : 0))
+                                : (const uint4*)(a.pts + (size_t)(e & 0x7fffffffu) * G1A);
         BBS_A16 uint32_t p[G1A];
 #pragma unroll
         for (int q = 0; q < G1A / 4; q++) { uint4 v = __ldg(src + q); p[4 * q] = v.x; p[4 * q + 1] = v.y; p[4 * q + 2] = v.z; p[4 * q + 3] = v.w; }
-        if (e >> 31) {
+        if (!PAIR && (e >> 31)) {
             BBS_A16 uint32_t t[FPN];
             fe_mul<F>(t, p, C::GLV_BETA());            // phi(x, y) = (beta x, y)
             bn_copy<C::Fp::N>(p, t);
@@ -179,6 +182,8 @@ template <class C> __global__ void __launch_bounds__(128, 4) msm_bucket_kernel(c
         g1_add_mixed<C>(acc, acc, p);
     }
 }
+template <class C> __global__ void __launch_bounds__(128, 4) msm_bucket_kernel(const MsmBucketArgs a) { msm_bucket_run<C, false>(a); }
+template <class C> __global__ void __launch_bounds__(128, 4) msm_bucket_pair_kernel(const MsmBucketArgs a) { msm_bucket_run<C, true>(a); }
 
 struct MsmReduceArgs { MsmPlan plan; const uint32_t* buckets; uint32_t* row_part; };     // row_part[row][block][Jacobian]
 // grid (red_blocks, rows): thread t of a row owns the digits t*chunk + 1 .. t*chunk + chunk and produces
@@ -301,6 +306,52 @@ template <class C> __global__ void __launch_bounds__(RLC_TPB, 1) rlc_msm_finish_
         a.flags[0] = ((skip[0] || cx.w_inf) ? FL_SKIP0 : 0u) | (skip[1] ? FL_SKIP1 : 0u);
         a.status[0] = ST_REJECT;
     }
+}
+
+// ---- proof batches (bbs_rlc_*proof_verify_batch*) --------------------------------------------------------------
+// After the G1 half of proof verification, item i is accepted iff e(Abar_i, W) e(-Bbar_i, BP2) == 1, and its pairing
+// record holds exactly (Abar_i, -Bbar_i).  Every item without FL_DONE is checked at once by
+//     e( sum r_i Abar_i , W ) * e( sum r_i (-Bbar_i) , BP2 ) == 1
+// with the coefficients r_i of rlc_coeff (index = the item's position in the call).  Both sums share the scalar r_i: it is
+// value 0 of the item (rows [0, W), base Abar) and value 2 (rows [W, 2W), entry bit 31, base -Bbar) for the unchanged scan
+// and scatter kernels; msm_bucket_pair_kernel reads the bases straight from the pairing records.  FL_SKIP0 / FL_SKIP1
+// (identity Abar or W, identity Bbar) leave the value out, as the pairing kernels leave the factor out.
+struct RlcProofPrepArgs {
+    MsmPlan plan;
+    const uint32_t* flags;   // the G1 half's per-item flags
+    uint32_t* kv;            // n x 3 x 4 words (value 1 stays 0)
+    uint32_t* counts;        // rows << c, zeroed by the caller
+    uint32_t* live;          // set to 1 when some item reaches the pairing; zeroed by the caller
+    uint32_t n;
+    BBS_A16 uint32_t seed[8];    // the 32-byte seed as big-endian words
+};
+template <class C> __global__ void __launch_bounds__(RLC_TPB) rlc_proof_prep_kernel(const RlcProofPrepArgs a) {
+    const uint32_t i = blockIdx.x * RLC_TPB + threadIdx.x;
+    const uint32_t fl = i < a.n ? a.flags[i] : (uint32_t)FL_DONE;
+    const bool live = !(fl & FL_DONE);
+    if (__ballot_sync(0xffffffffu, live) && (threadIdx.x & 31) == 0) atomicOr(a.live, 1u);
+    if (i >= a.n) return;
+    BBS_A16 uint32_t r[8], kv[12];
+    for (int k = 0; k < 12; k++) kv[k] = 0;
+    if (live) {
+        rlc_coeff(r, a.seed, i);
+        if (!(fl & FL_SKIP0)) for (int k = 0; k < 4; k++) kv[k] = r[k];
+        if (!(fl & FL_SKIP1)) for (int k = 0; k < 4; k++) kv[8 + k] = r[k];
+    }
+    uint32_t* kd = a.kv + (size_t)i * 12;
+    for (int k = 0; k < 12; k++) kd[k] = kv[k];
+    if (!live) return;
+    const uint32_t c = a.plan.c, W = a.plan.W;
+    for (uint32_t s = 0; s < 3; s += 2)
+        for (uint32_t w = 0; w < W; w++) {
+            const uint32_t d = msm_digit(kd + 4 * s, w, W);
+            if (d) atomicAdd(a.counts + ((size_t)msm_row(s, w, W) << c) + d, 1u);
+        }
+}
+// the combined check held: every item that reached the pairing is accepted
+template <class C> __global__ void __launch_bounds__(RLC_TPB) rlc_proof_accept_kernel(const uint32_t* flags, uint8_t* status, uint32_t n) {
+    const uint32_t i = blockIdx.x * RLC_TPB + threadIdx.x;
+    if (i < n && !(flags[i] & FL_DONE)) status[i] = ST_ACCEPT;
 }
 
 }  // namespace bbs

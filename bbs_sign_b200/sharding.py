@@ -86,6 +86,24 @@ class ShardedVerifier:
         self._run_sharded(n, work)
         return out
 
+    def rlc_proof_verify_batch(self, proofs, ph, disclosed_messages, disclosed_indexes, *,
+                               headers: Optional[Sequence[bytes]] = None):
+        """`BatchContext.rlc_proof_verify_batch` split by proof index: every GPU checks its slice with one combined pairing
+        under its own library-drawn seed, so nothing is exchanged.  Returns (status, combined); `combined` is ST_ACCEPT
+        only if every shard's was."""
+        n = len(proofs)
+        out = np.full(n, 255, dtype=np.uint8)
+        combined = [1] * len(self.ctxs)
+        per_item_ph = _is_per_item(ph)
+
+        def work(ctx, g, lo, hi):
+            out[lo:hi], combined[g] = ctx.rlc_proof_verify_batch(
+                proofs[lo:hi], ph[lo:hi] if per_item_ph else ph, disclosed_messages[lo:hi], disclosed_indexes[lo:hi],
+                headers=None if headers is None else headers[lo:hi])
+
+        self._run_sharded(n, work)
+        return out, (1 if all(c == 1 for c in combined) else 0)
+
     def rlc_verify_batch(self, signatures: Sequence[bytes], messages: Sequence[Sequence[bytes]],
                          seed: Optional[bytes] = None) -> int:
         """Random-linear-combination verdict for the whole batch: every GPU reduces its slice to two compressed G1

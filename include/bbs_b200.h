@@ -296,6 +296,42 @@ int bbs_rlc_core_verify_batch(bbs_ctx* ctx, size_t n, const uint8_t* sigs, const
 int bbs_rlc_verify_batch(bbs_ctx* ctx, size_t n, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* offsets,
                          uint32_t n_msgs, const uint8_t* seed32_or_null, uint8_t* verdict);
 
+/* Proof verification with the pairing half by one random linear combination.  Arguments as bbs_[core_]proof_verify_batch
+ * and bbs_[core_]proof_verify_batch_hdr (per-item phs, NULL headers = the context's header), plus:
+ *   seed32_or_null : the coefficient seed; r_i = the first 16 bytes, as a big-endian integer, of SHA-256(seed || BE64(i))
+ *                    (1 if that is 0), i = the item's position in the call.  NULL: the library draws 32 bytes from the OS
+ *                    CSPRNG after it has received the batch.
+ *   status[i]      : what the call without rlc_ returns for item i.  An ACCEPT holds except with probability 2^-128 over
+ *                    the seed; every other status is exact.
+ *   combined       : (may be NULL) ACCEPT when the one combined check held for every item that reached the pairing, or
+ *                    when no item did; REJECT when it failed and the per-item pairing decided those items instead.
+ * After the G1 half (challenge comparison, Err variants, malformed input: exact per item, as in the call without rlc_),
+ * every proof that reaches the pairing is checked at once by
+ *     e( sum r_i Abar_i , W ) * e( sum r_i (-Bbar_i) , BP2 ) == 1
+ * one bucket MSM and one pairing for the batch.  If that fails, the per-item pairing kernel decides the same items, so
+ * the statuses stay exact at about the cost of the call without rlc_; `combined` tells a caller that this happened.
+ * THE SEED MUST BE UNPREDICTABLE TO WHOEVER SUBMITS THE BATCH: with a known seed, two proofs whose pairing checks fail
+ * can be built so that their failures cancel in the sum, and both are accepted.  Pass NULL; an explicit seed is for
+ * reproducible tests.  One issuer key per call (no issuer sets).  n must be below 2^31. */
+int bbs_rlc_core_proof_verify_batch(bbs_ctx* ctx, size_t n, const uint8_t* proofs_fixed, const uint8_t* commitments,
+                                    const uint64_t* commit_off, const uint32_t* disclosed_idx,
+                                    const uint8_t* disclosed_scalars, const uint64_t* dis_off, const uint8_t* ph,
+                                    size_t ph_len, const uint8_t* seed32_or_null, uint8_t* status, uint8_t* combined);
+int bbs_rlc_proof_verify_batch(bbs_ctx* ctx, size_t n, const uint8_t* proofs_fixed, const uint8_t* commitments,
+                               const uint64_t* commit_off, const uint32_t* disclosed_idx, const uint8_t* dis_msgs,
+                               const uint64_t* dis_msg_off, const uint64_t* dis_off, const uint8_t* ph, size_t ph_len,
+                               const uint8_t* seed32_or_null, uint8_t* status, uint8_t* combined);
+int bbs_rlc_core_proof_verify_batch_hdr(bbs_ctx* ctx, size_t n, const uint8_t* proofs_fixed, const uint8_t* commitments,
+                                        const uint64_t* commit_off, const uint32_t* disclosed_idx,
+                                        const uint8_t* disclosed_scalars, const uint64_t* dis_off, const uint8_t* headers,
+                                        const uint64_t* hdr_off, const uint8_t* phs, const uint64_t* ph_off,
+                                        const uint8_t* seed32_or_null, uint8_t* status, uint8_t* combined);
+int bbs_rlc_proof_verify_batch_hdr(bbs_ctx* ctx, size_t n, const uint8_t* proofs_fixed, const uint8_t* commitments,
+                                   const uint64_t* commit_off, const uint32_t* disclosed_idx, const uint8_t* dis_msgs,
+                                   const uint64_t* dis_msg_off, const uint64_t* dis_off, const uint8_t* headers,
+                                   const uint64_t* hdr_off, const uint8_t* phs, const uint64_t* ph_off,
+                                   const uint8_t* seed32_or_null, uint8_t* status, uint8_t* combined);
+
 /* ---- device-buffer entry points (no copies; all pointers are device pointers on the context's GPU;
  *      work is enqueued on `stream` (a cudaStream_t, NULL = default stream) and NOT synchronized) ------ */
 int bbs_msg_to_scalars_dev(bbs_ctx* ctx, size_t count, const uint8_t* d_msgs, const uint64_t* d_offsets,
@@ -347,7 +383,11 @@ int bbs_ctx_set_pairing_split(bbs_ctx* ctx, size_t max_items);
  * With profiling on, every *_dev batch call records CUDA events on its launching stream around each of its
  * kernels; bbs_ctx_kernel_times returns the durations (ms) of the last call in launch order:
  *   verify / proof verify: [msg_to_scalars (0 if absent), G1 kernel, pairing kernel];  sign: [h2s, sign].
- * The *_hdr calls with per-item headers append the per-item domain kernel: verify / proof verify slot 3, sign slot 2. */
+ * The *_hdr calls with per-item headers append the per-item domain kernel: verify / proof verify slot 3, sign slot 2.
+ * bbs_rlc_*proof_verify_batch*: [msg_to_scalars, G1 kernels, prep, scan + scatter, buckets, reduction, finish, combined
+ *   pairing, acceptance or per-item pairing]; the scan slot and the combined-pairing slot also hold the host's read of one
+ *   word (whether any item reached the pairing; the verdict).  Slots 3..8 are 0 when no item reached the pairing;
+ *   per-item headers: slot 9. */
 int bbs_ctx_set_profiling(bbs_ctx* ctx, int on);
 int bbs_ctx_kernel_times(bbs_ctx* ctx, float* ms, int n);
 /* Integer-multiply roofline probe: 8 independent multiply-accumulate chains per thread on every SM.

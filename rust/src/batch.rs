@@ -127,6 +127,21 @@ extern "C" {
                                  seed32_or_null: *const u8, verdict: *mut u8) -> i32;
     fn bbs_rlc_verify_batch(ctx: *mut BbsCtx, n: usize, sigs: *const u8, msgs: *const u8, offsets: *const u64, n_msgs: u32,
                             seed32_or_null: *const u8, verdict: *mut u8) -> i32;
+    fn bbs_rlc_core_proof_verify_batch(ctx: *mut BbsCtx, n: usize, proofs_fixed: *const u8, commitments: *const u8,
+                                       commit_off: *const u64, disclosed_idx: *const u32, disclosed_scalars: *const u8,
+                                       dis_off: *const u64, ph: *const u8, ph_len: usize, seed32_or_null: *const u8,
+                                       status: *mut u8, combined: *mut u8) -> i32;
+    fn bbs_rlc_proof_verify_batch(ctx: *mut BbsCtx, n: usize, proofs_fixed: *const u8, commitments: *const u8, commit_off: *const u64,
+                                  disclosed_idx: *const u32, dis_msgs: *const u8, dis_msg_off: *const u64, dis_off: *const u64,
+                                  ph: *const u8, ph_len: usize, seed32_or_null: *const u8, status: *mut u8, combined: *mut u8) -> i32;
+    fn bbs_rlc_core_proof_verify_batch_hdr(ctx: *mut BbsCtx, n: usize, proofs_fixed: *const u8, commitments: *const u8,
+                                           commit_off: *const u64, disclosed_idx: *const u32, disclosed_scalars: *const u8,
+                                           dis_off: *const u64, headers: *const u8, hdr_off: *const u64, phs: *const u8,
+                                           ph_off: *const u64, seed32_or_null: *const u8, status: *mut u8, combined: *mut u8) -> i32;
+    fn bbs_rlc_proof_verify_batch_hdr(ctx: *mut BbsCtx, n: usize, proofs_fixed: *const u8, commitments: *const u8,
+                                      commit_off: *const u64, disclosed_idx: *const u32, dis_msgs: *const u8, dis_msg_off: *const u64,
+                                      dis_off: *const u64, headers: *const u8, hdr_off: *const u64, phs: *const u8,
+                                      ph_off: *const u64, seed32_or_null: *const u8, status: *mut u8, combined: *mut u8) -> i32;
     fn bbs_msg_to_scalars_dev(ctx: *mut BbsCtx, count: usize, d_msgs: *const u8, d_offsets: *const u64, d_out: *mut u8,
                               stream: *mut c_void) -> i32;
     fn bbs_core_verify_batch_dev(ctx: *mut BbsCtx, n: usize, d_sigs: *const u8, d_msg_scalars: *const u8, n_msgs: u32,
@@ -504,12 +519,32 @@ pub fn proof_verify_batch_per_item<E: Pairing, F: Field>(ctx: &BatchCtx, proofs:
     proof_verify_on(ProofTarget::CtxPerItem(ctx.raw, headers, phs), proofs, &[], disclosed_messages, disclosed_indexes)
 }
 
+/// `proof_verify_batch` with the pairing checks of the batch folded into one random linear combination
+/// (`bbs_rlc_proof_verify_batch`): the same per-item results, where an accepted proof holds except with probability
+/// 2^-128 over a coefficient seed the library draws from the OS after it has the batch.  Fast when every proof's pairing
+/// holds; a batch in which some proof fails only its pairing costs about as much as `proof_verify_batch`.
+pub fn rlc_proof_verify_batch<E: Pairing, F: Field>(ctx: &BatchCtx, proofs: &[Proof<E, F>], ph: &[u8],
+    disclosed_messages: &[&[&[u8]]], disclosed_indexes: &[&[usize]])
+    -> Result<Vec<Result<bool, ItemError<ProofGenError>>>, BatchError> {
+    proof_verify_on(ProofTarget::RlcCtx(ctx.raw), proofs, ph, disclosed_messages, disclosed_indexes)
+}
+
+/// `proof_verify_batch_per_item` by one random linear combination, as `rlc_proof_verify_batch`.
+pub fn rlc_proof_verify_batch_per_item<E: Pairing, F: Field>(ctx: &BatchCtx, proofs: &[Proof<E, F>], headers: Option<&[&[u8]]>,
+    phs: &[&[u8]], disclosed_messages: &[&[&[u8]]], disclosed_indexes: &[&[usize]])
+    -> Result<Vec<Result<bool, ItemError<ProofGenError>>>, BatchError> {
+    assert!(phs.len() == proofs.len() && headers.map_or(true, |h| h.len() == proofs.len()), "one ph (and header) per proof");
+    proof_verify_on(ProofTarget::RlcCtxPerItem(ctx.raw, headers, phs), proofs, &[], disclosed_messages, disclosed_indexes)
+}
+
 /// Where a proof batch is verified: under the one key of a context, under a key per proof of an issuer set, or under the
-/// key of a context with a ph (and header) per proof.
+/// key of a context with a ph (and header) per proof; the Rlc forms check the pairings by one random linear combination.
 enum ProofTarget<'a> {
     Ctx(*mut BbsCtx),
     Set(*mut BbsIssuerSet, &'a [u32]),
     CtxPerItem(*mut BbsCtx, Option<&'a [&'a [u8]]>, &'a [&'a [u8]]),
+    RlcCtx(*mut BbsCtx),
+    RlcCtxPerItem(*mut BbsCtx, Option<&'a [&'a [u8]]>, &'a [&'a [u8]]),
 }
 
 fn proof_verify_on<E: Pairing, F: Field>(target: ProofTarget, proofs: &[Proof<E, F>], ph: &[u8],
@@ -565,17 +600,30 @@ fn proof_verify_on<E: Pairing, F: Field>(target: ProofTarget, proofs: &[Proof<E,
                                                  st.as_mut_ptr())
                 }
             }
-            ProofTarget::CtxPerItem(raw, headers, phs) => {
+            ProofTarget::CtxPerItem(raw, headers, phs) | ProofTarget::RlcCtxPerItem(raw, headers, phs) => {
                 // the items kept for the call, with their own ph / header
                 let (p, poff) = pack_items(&keep.iter().map(|&i| phs[i]).collect::<Vec<_>>());
                 let hs = headers.map(|h| pack_items(&keep.iter().map(|&i| h[i]).collect::<Vec<_>>()));
                 let (hp, hoff) = hs.as_ref().map_or((std::ptr::null(), std::ptr::null()), |(h, o)| (h.as_ptr(), o.as_ptr()));
-                unsafe {
-                    bbs_proof_verify_batch_hdr(raw, keep.len(), fixed.as_ptr(), commits.as_ptr(), coff.as_ptr(), idx.as_ptr(),
-                                               flat.as_ptr(), moffs.as_ptr(), doff.as_ptr(), hp, hoff, p.as_ptr(), poff.as_ptr(),
-                                               st.as_mut_ptr())
+                if matches!(target, ProofTarget::RlcCtxPerItem(..)) {
+                    unsafe {
+                        bbs_rlc_proof_verify_batch_hdr(raw, keep.len(), fixed.as_ptr(), commits.as_ptr(), coff.as_ptr(), idx.as_ptr(),
+                                                       flat.as_ptr(), moffs.as_ptr(), doff.as_ptr(), hp, hoff, p.as_ptr(), poff.as_ptr(),
+                                                       std::ptr::null(), st.as_mut_ptr(), std::ptr::null_mut())
+                    }
+                } else {
+                    unsafe {
+                        bbs_proof_verify_batch_hdr(raw, keep.len(), fixed.as_ptr(), commits.as_ptr(), coff.as_ptr(), idx.as_ptr(),
+                                                   flat.as_ptr(), moffs.as_ptr(), doff.as_ptr(), hp, hoff, p.as_ptr(), poff.as_ptr(),
+                                                   st.as_mut_ptr())
+                    }
                 }
             }
+            ProofTarget::RlcCtx(raw) => unsafe {
+                bbs_rlc_proof_verify_batch(raw, keep.len(), fixed.as_ptr(), commits.as_ptr(), coff.as_ptr(), idx.as_ptr(), flat.as_ptr(),
+                                           moffs.as_ptr(), doff.as_ptr(), ph.as_ptr(), ph.len(), std::ptr::null(), st.as_mut_ptr(),
+                                           std::ptr::null_mut())
+            },
         })?;
     }
     let mut out: Vec<Result<bool, ItemError<ProofGenError>>> =
@@ -751,6 +799,7 @@ fn _unused_bindings() {
         bbs_selftest_field as usize, bbs_selftest_g1_mul as usize, bbs_selftest_pairing as usize,
         bbs_core_verify_batch_hdr as usize, bbs_core_sign_batch_hdr as usize, bbs_core_proof_verify_batch_hdr as usize,
         bbs_core_proof_gen_batch_hdr as usize, bbs_proof_gen_batch_hdr as usize, bbs_core_verify_batch_hdr_dev as usize,
-        bbs_core_proof_verify_batch_hdr_dev as usize,
+        bbs_core_proof_verify_batch_hdr_dev as usize, bbs_rlc_core_proof_verify_batch as usize,
+        bbs_rlc_core_proof_verify_batch_hdr as usize,
     );
 }
