@@ -103,6 +103,7 @@ SYMBOLS = {
     "bbs_imad_peak": (C.c_int, [C.c_int, C.c_int, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_float)]),
     "bbs_selftest_field": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p]),
     "bbs_selftest_g1_mul": (C.c_int, [C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "bbs_selftest_g1": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "bbs_selftest_pairing": (C.c_int, [C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
 }
 

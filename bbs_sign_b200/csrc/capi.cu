@@ -1623,6 +1623,13 @@ int bbs_selftest_g1_mul(int curve, int device, size_t n, const uint8_t* pts, con
     if (curve == BBS_CURVE_BN254) return selftest_g1_mul<Bn>(n, pts, sc, out);
     return arg_error("unknown curve id");
 }
+int bbs_selftest_g1(int curve, int device, int op, size_t n, const uint8_t* p, const uint8_t* q, const uint8_t* sc,
+                    uint8_t* out) {
+    if (rt_set_device(device)) return BBS_E_CUDA;
+    if (curve == BBS_CURVE_BLS12_381) return selftest_g1<Bls>(op, n, p, q, sc, out);
+    if (curve == BBS_CURVE_BN254) return selftest_g1<Bn>(op, n, p, q, sc, out);
+    return arg_error("unknown curve id");
+}
 int bbs_selftest_pairing(int curve, int device, size_t n, const uint8_t* p_points, const uint8_t* r_points,
                          const uint8_t* q_point, uint8_t* status) {
     if (rt_set_device(device)) return BBS_E_CUDA;

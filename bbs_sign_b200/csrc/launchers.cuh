@@ -49,6 +49,7 @@ template <class C> int launch_proof_gen(const ProofGenArgs& a, uint32_t n, rt_st
 template <class C> int launch_proof_gen_per_item(const ProofGenArgs& a, uint32_t n, rt_stream_t s);
 template <class C> int launch_field_test(const FieldTestArgs& a, uint32_t n, rt_stream_t s);
 template <class C> int launch_g1_mul_test(const G1MulTestArgs& a, uint32_t n, rt_stream_t s);
+template <class C> int launch_g1_test(const G1TestArgs& a, uint32_t n, rt_stream_t s);
 template <class C> int launch_pair_test_prep(const PairTestPrepArgs& a, uint32_t n, rt_stream_t s);
 template <class C> int launch_pair_test(const PairTestArgs& a, uint32_t n, rt_stream_t s);
 

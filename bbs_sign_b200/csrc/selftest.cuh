@@ -68,6 +68,51 @@ template <class C> BBS_HD void g1_mul_test_item(const G1MulTestArgs& t, uint32_t
     g1_compress<C>(o, R);
 }
 
+// The G1 group law (bbs_selftest_g1): one operation per item on Jacobian operands, so the test can reach the rare-case
+// branches of the additions (P + P, P + (-P), identities) with one point under several Z.
+enum : int { G1_TEST_ADD = 0, G1_TEST_ADD_MIXED = 1, G1_TEST_DBL = 2, G1_TEST_MSM2 = 3, G1_TEST_MSM3 = 4 };
+constexpr int G1_TEST_LAST_OP = G1_TEST_MSM3;
+BBS_HD int g1_test_points(int op) { return op == G1_TEST_MSM2 ? 2 : op == G1_TEST_MSM3 ? 3 : 1; }
+
+struct G1TestArgs { int op; const uint8_t* p; const uint8_t* q; const uint8_t* sc; uint8_t* out; };
+// canonical little-endian (X, Y, Z) -> Montgomery Jacobian
+template <class C> BBS_HD void g1_test_load(uint32_t* r, const uint8_t* in) {
+    for (int k = 0; k < 3; k++) {
+        limbs_from_le<C::Fp::N>(r + k * FPN, in + k * 4 * C::Fp::N);
+        fe_to_mont<typename C::Fp>(r + k * FPN, r + k * FPN);
+    }
+}
+template <class C, int NP> BBS_HD void g1_test_msm(uint32_t* R, const uint8_t* p, const uint8_t* sc) {
+    BBS_A16 uint32_t P[NP][G1J], k[NP][8];
+    const uint32_t* pts[NP];
+    const uint32_t* ks[NP];
+    for (int j = 0; j < NP; j++) {
+        g1_test_load<C>(P[j], p + (size_t)j * 12 * C::Fp::N);
+        limbs_from_le<8>(k[j], sc + (size_t)j * 32);
+        pts[j] = g1_is_inf<C>(P[j]) ? nullptr : P[j];       // affine (x, y): Z only marks the identity
+        ks[j] = k[j];
+    }
+    g1_msm_scalar<C, NP>(R, pts, ks);
+}
+template <class C> BBS_HD void g1_test_item(const G1TestArgs& t, uint32_t i) {
+    constexpr size_t PB = 12 * C::Fp::N;         // bytes of one Jacobian operand
+    const int np = g1_test_points(t.op);
+    const uint8_t* p = t.p + (size_t)i * np * PB;
+    BBS_A16 uint32_t R[G1J];
+    if (t.op == G1_TEST_MSM2) g1_test_msm<C, 2>(R, p, t.sc + (size_t)i * 2 * 32);
+    else if (t.op == G1_TEST_MSM3) g1_test_msm<C, 3>(R, p, t.sc + (size_t)i * 3 * 32);
+    else {
+        BBS_A16 uint32_t P[G1J], Q[G1J];
+        g1_test_load<C>(P, p);
+        if (t.op == G1_TEST_DBL) g1_dbl<C>(R, P);
+        else {
+            g1_test_load<C>(Q, t.q + (size_t)i * PB);
+            if (t.op == G1_TEST_ADD) g1_add<C>(R, P, Q); else g1_add_mixed<C>(R, P, Q);
+        }
+    }
+    g1_compress<C>(t.out + (size_t)i * C::G1_BYTES, R);
+}
+
 struct PairTestPrepArgs { const uint8_t* q; uint32_t* W; uint32_t* lines; uint32_t* st; };
 template <class C> BBS_HD void pair_test_prep_item(const PairTestPrepArgs& t, uint32_t i) {
     if (i == 0) {

@@ -408,6 +408,14 @@ int bbs_selftest_field(int curve_id, int device, int op, size_t n, const uint8_t
 /* out[i] = comp(k_i * P_i) for compressed G1 points and LE32 scalars. */
 int bbs_selftest_g1_mul(int curve_id, int device, size_t n, const uint8_t* points, const uint8_t* scalars,
                         uint8_t* out);
+/* out[i] = comp(op(...)) on the G1 group law.  Operands are Jacobian points (X, Y, Z), three canonical little-endian Fp
+ * values each (48 / 32 bytes), Z = 0 the identity, so one point can be given under several Z: (l^2 x, l^3 y, l).
+ * op: 0 = g1_add(p_i, q_i); 1 = g1_add_mixed(p_i, q_i), q_i read as the affine (X, Y) of a finite point (its Z ignored);
+ *     2 = g1_dbl(p_i) (q ignored); 3 / 4 = the Straus product sum_j k_ij P_ij over 2 / 3 points (g1_msm_scalar):
+ *     p holds 2 / 3 operands per item, read as affine (X, Y) with Z = 0 for the identity (Z's value otherwise ignored),
+ *     scalars 2 / 3 canonical LE32 scalars per item (q ignored).  scalars is ignored by ops 0..2.  Other ops are refused. */
+int bbs_selftest_g1(int curve_id, int device, int op, size_t n, const uint8_t* p, const uint8_t* q, const uint8_t* scalars,
+                    uint8_t* out);
 /* status[i] = (e(P_i, Q) * e(R_i, BP2) == 1) for compressed G1 points P_i, R_i and one compressed G2 point Q. */
 int bbs_selftest_pairing(int curve_id, int device, size_t n, const uint8_t* p_points, const uint8_t* r_points,
                          const uint8_t* q_point, uint8_t* status);

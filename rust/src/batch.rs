@@ -171,6 +171,8 @@ extern "C" {
     fn bbs_imad_peak(device: i32, iters: i32, mode: i32, gprod_per_s: *mut f64, ms: *mut f32) -> i32;
     fn bbs_selftest_field(curve_id: i32, device: i32, op: i32, n: usize, a: *const u8, b: *const u8, out: *mut u8) -> i32;
     fn bbs_selftest_g1_mul(curve_id: i32, device: i32, n: usize, points: *const u8, scalars: *const u8, out: *mut u8) -> i32;
+    fn bbs_selftest_g1(curve_id: i32, device: i32, op: i32, n: usize, p: *const u8, q: *const u8, scalars: *const u8,
+                       out: *mut u8) -> i32;
     fn bbs_selftest_pairing(curve_id: i32, device: i32, n: usize, p_points: *const u8, r_points: *const u8, q_point: *const u8,
                             status: *mut u8) -> i32;
 }
@@ -796,7 +798,7 @@ fn _unused_bindings() {
         bbs_verify_batch_dev as usize, bbs_core_sign_batch_dev as usize, bbs_core_proof_verify_batch_dev as usize,
         bbs_ctx_launch_count as usize, bbs_ctx_memory_bytes as usize, bbs_core_verify_batch_multi as usize, bbs_core_proof_verify_batch_multi as usize, bbs_ctx_use_per_thread_pairing as usize,
         bbs_ctx_set_rlc_windows as usize, bbs_ctx_set_g1_split as usize, bbs_ctx_set_pairing_split as usize, bbs_ctx_set_profiling as usize, bbs_ctx_kernel_times as usize, bbs_imad_peak as usize,
-        bbs_selftest_field as usize, bbs_selftest_g1_mul as usize, bbs_selftest_pairing as usize,
+        bbs_selftest_field as usize, bbs_selftest_g1_mul as usize, bbs_selftest_g1 as usize, bbs_selftest_pairing as usize,
         bbs_core_verify_batch_hdr as usize, bbs_core_sign_batch_hdr as usize, bbs_core_proof_verify_batch_hdr as usize,
         bbs_core_proof_gen_batch_hdr as usize, bbs_proof_gen_batch_hdr as usize, bbs_core_verify_batch_hdr_dev as usize,
         bbs_core_proof_verify_batch_hdr_dev as usize, bbs_rlc_core_proof_verify_batch as usize,
