@@ -255,6 +255,55 @@ class BatchContext:
                                                   _ptr(_buf(seed)) if seed is not None else None, _ptr(v)), "bbs_rlc_verify_batch")
         return int(v[0])
 
+    def rlc_verify_batch_status(self, signatures, messages: Sequence[Sequence[bytes]], *,
+                                headers: Optional[Sequence[bytes]] = None, seed: Optional[bytes] = None):
+        """`verify_batch` with the pairings checked by one random linear combination (bbs_rlc_verify_batch_status*,
+        include/bbs_b200.h).  Returns (status, combined): the statuses are those of `verify_batch` (an ACCEPT holds except
+        with probability 2^-128 over the seed); `combined` is ST_ACCEPT when the one combined check held (or no item reached
+        it), ST_REJECT when it failed and the per-item path decided instead.  An item whose message count is not the
+        context's L gets ST_ERR_MSG_GEN_LEN and never reaches the library.  `seed=None` (the default) lets the library draw
+        the seed after it has the batch; pass a seed only for reproducible tests: a seed the submitter of the batch can
+        predict lets crafted signatures pass."""
+        sigs = _buf(b"".join(signatures) if isinstance(signatures, (list, tuple)) else signatures)
+        sb = self.suite.signature_bytes
+        n = sigs.size // sb
+        if len(messages) != n or (headers is not None and len(headers) != n):
+            raise BbsError("one message list (and header) per signature required")
+        keep = [i for i in range(n) if len(messages[i]) == self.L]
+        sel = sigs.reshape(n, sb)[keep].reshape(-1) if len(keep) < n else sigs
+        flat, offs = _pack_ragged([m for i in keep for m in messages[i]])
+        return self._verify_status(False, n, keep, sel, (flat, offs), headers, seed)
+
+    def rlc_core_verify_batch_status(self, signatures, msg_scalars, n_msgs: int, *,
+                                     headers: Optional[Sequence[bytes]] = None, seed: Optional[bytes] = None):
+        """`core_verify_batch` with the pairings checked by one random linear combination; returns (status, combined) as
+        `rlc_verify_batch_status`"""
+        sigs = _buf(signatures)
+        n = sigs.size // self.suite.signature_bytes
+        sc = _buf(msg_scalars)
+        if sc.size != n * n_msgs * 32 or (headers is not None and len(headers) != n):
+            raise BbsError("msg_scalars / headers have the wrong size")
+        keep = list(range(n)) if n_msgs == self.L else []
+        return self._verify_status(True, n, keep, sigs, (sc if sc.size else np.zeros(1, np.uint8),), headers, seed)
+
+    def _verify_status(self, core: bool, n: int, keep, sigs, msgs, headers, seed):
+        """(status, combined) of bbs_rlc_[core_]verify_batch_status[_hdr] over the items `keep` (those with L messages);
+        the others get ST_ERR_MSG_GEN_LEN here, and `combined` covers the kept items (ST_ACCEPT when there are none)"""
+        st = np.full(n, ST_ERR_MSG_GEN_LEN, dtype=np.uint8)
+        combined = np.full(1, ST_ACCEPT, dtype=np.uint8)
+        if keep:
+            out = np.full(len(keep), 255, dtype=np.uint8)
+            name = "bbs_rlc_" + ("core_" if core else "") + "verify_batch_status"
+            args = [self._h, len(keep), _ptr(sigs)] + [_ptr(m) for m in msgs] + [self.L]
+            if headers is not None:
+                name += "_hdr"
+                hb, hoff = _pack_items([headers[i] for i in keep], len(keep), "header")
+                args += [_ptr(hb), _ptr(hoff)]
+            args += [_ptr(_buf(seed)) if seed is not None else None, _ptr(out), _ptr(combined)]
+            self._check(getattr(self.lib, name)(*args), name)
+            st[keep] = out
+        return st, int(combined[0])
+
     # ---- test hooks (include/bbs_b200.h) ----
     def use_per_thread_pairing(self, on: bool = True):
         self._check(self.lib.bbs_ctx_use_per_thread_pairing(self._h, 1 if on else 0), "bbs_ctx_use_per_thread_pairing")

@@ -125,8 +125,8 @@ struct IssuerSet {
 // their scalars, 32 bytes each
 struct MsgIn { const uint8_t* scalars; const uint8_t* msgs; const uint64_t* off; };
 
-// The random-linear-combination form of a proof verify call (bbs_rlc_*proof_verify_batch*): the 32-byte coefficient seed
-// and where the combined check's verdict goes (may be null)
+// The random-linear-combination form of a call with per-item statuses (bbs_rlc_*proof_verify_batch*,
+// bbs_rlc_*verify_batch_status*): the 32-byte coefficient seed and where the combined check's verdict goes (may be null)
 struct RlcProofIn { const uint8_t* seed; uint8_t* combined; };
 
 #define TRY(expr) do { int rc_ = (expr); if (rc_) return rc_; } while (0)
@@ -646,18 +646,25 @@ struct Impl {
         p.red_blocks = (threads + RLC_TPB - 1) / RLC_TPB;
         return p;
     }
-    // shard -> comp(S1) || comp(S2) in c->s_rlc_parts (and the pairing record of the two sums); *bad != 0 when an item was
-    // malformed.  The host buffers of the shard are fed in up to 8 chunks: chunk k + 1 is uploaded on the copy stream while
-    // chunk k is hashed (byte messages) and prepared on the compute stream.
-    static int rlc_partial_dev(Ctx* c, size_t n, const uint8_t* sigs, const MsgIn& in, uint32_t n_msgs, const uint8_t* seed,
-                               uint64_t index_base, uint32_t* bad, rt_stream_t s) {
+    // The upload, hashing and prep stages of a shard: its host buffers are fed in up to 8 chunks, chunk k + 1 uploaded on
+    // the copy stream while chunk k is hashed (byte messages) and prepared on the compute stream.  `mode` (RLC_PREP_*):
+    // RLC_PREP_VERDICT sets the word s_rlc_bad when an item is malformed; the status modes write the malformed items'
+    // statuses and every item's flag word into s_status / s_flags and set s_rlc_bad when some item is well formed, and
+    // RLC_PREP_STATUS_HDR reads the items' domains from `item`.  Reserves the MSM scratch that rlc_msm_dev uses after it.
+    static int rlc_prep_dev(Ctx* c, size_t n, const uint8_t* sigs, const MsgIn& in, uint32_t n_msgs, const uint8_t* seed,
+                            uint64_t index_base, int mode, const ItemKeyView* item, MsmPlan& plan, rt_stream_t s) {
         if (n >= (1ull << 31)) return arg_error("rlc shard too large");
         const uint32_t blocks = (uint32_t)((n + RLC_TPB - 1) / RLC_TPB);
-        const MsmPlan plan = rlc_plan(n, c->rlc_windows);
+        const uint32_t sc_rows = n_msgs + 1 + (mode == RLC_PREP_STATUS_HDR ? 1u : 0u);
+        plan = rlc_plan(n, c->rlc_windows);
         const size_t nb = (size_t)plan.rows << plan.c, PT = 3 * C::Fp::N * 4;
-        TRY(c->s_rlc_sc.reserve((size_t)(blocks ? blocks : 1) * (n_msgs + 1) * 32));
+        TRY(c->s_rlc_sc.reserve((size_t)(blocks ? blocks : 1) * sc_rows * 32));
         TRY(c->s_rlc_parts.reserve(2 * C::G1_BYTES));
         TRY(c->s_rlc_bad.reserve(4));
+        if (mode != RLC_PREP_VERDICT) {
+            TRY(c->s_status.reserve(n));
+            TRY(c->s_flags.reserve(n * 4));
+        }
         TRY(c->s_msm_pts.reserve((n ? n : 1) * 2 * C::Fp::N * 4));
         TRY(c->s_msm_kv.reserve((n ? n : 1) * 48));
         TRY(c->s_msm_idx.reserve((3 * nb + 5) * 4));                        // next (4 words) | counts | offsets (nb + 1) | cursor
@@ -677,6 +684,7 @@ struct Impl {
             a.seed[i] = ((uint32_t)seed[4 * i] << 24) | ((uint32_t)seed[4 * i + 1] << 16) | ((uint32_t)seed[4 * i + 2] << 8) | seed[4 * i + 3];
         a.bad = (uint32_t*)c->s_rlc_bad.p;
         pa.plan = plan; pa.counts = counts;
+        pa.live = (uint32_t*)c->s_rlc_bad.p;
         // chunk = a whole number of waves of the prep kernel (4 blocks of RLC_TPB items per SM), at most 8 chunks; chunk
         // boundaries are multiples of the block size, so the blocks' partial sums keep their global index
         int sms = 0;
@@ -697,12 +705,28 @@ struct Impl {
             a.sigs = (const uint8_t*)c->s_sigs.p + i0 * SIG; a.scalars = (const uint8_t*)c->s_scalars.p + m0 * 32;
             a.n = (uint32_t)(i1 - i0);
             a.index_base = index_base + i0;
-            a.sc_part = (uint32_t*)c->s_rlc_sc.p + (i0 / RLC_TPB) * (n_msgs + 1) * 8;
+            a.sc_part = (uint32_t*)c->s_rlc_sc.p + (i0 / RLC_TPB) * sc_rows * 8;
             pa.pts = (uint32_t*)c->s_msm_pts.p + i0 * 2 * C::Fp::N; pa.kv = (uint32_t*)c->s_msm_kv.p + i0 * 12;
-            TRY((launch_rlc_prep<C>(pa, (uint32_t)((i1 - i0 + RLC_TPB - 1) / RLC_TPB), s)));
+            if (mode != RLC_PREP_VERDICT) {
+                pa.status = (uint8_t*)c->s_status.p + i0; pa.flags = (uint32_t*)c->s_flags.p + i0;
+                pa.domains = item ? item->domains + i0 * 8 : nullptr;
+            }
+            TRY((launch_rlc_prep<C>(pa, (uint32_t)((i1 - i0 + RLC_TPB - 1) / RLC_TPB), mode, s)));
             c->launches += 1;
         }
         PROF(c, 2, s);
+        return BBS_OK;
+    }
+    // scan, scatter, buckets, reduction and finish over the prepared shard: comp(S1) || comp(S2) in c->s_rlc_parts and the
+    // pairing record of the two sums, its flag word and status at pair / flags / status (index 0)
+    static int rlc_msm_dev(Ctx* c, size_t n, const MsmPlan& plan, uint32_t n_msgs, bool hdr, uint32_t* pair, uint32_t* flags,
+                           uint8_t* status, rt_stream_t s) {
+        const uint32_t blocks = (uint32_t)((n + RLC_TPB - 1) / RLC_TPB);
+        const size_t nb = (size_t)plan.rows << plan.c;
+        uint32_t* next = (uint32_t*)c->s_msm_idx.p;
+        uint32_t* counts = next + 4;
+        uint32_t* offsets = counts + nb;
+        uint32_t* cursor = offsets + nb + 1;
         TRY(launch_msm_scan(counts, offsets, cursor, (uint32_t)nb, s));
         MsmScatterArgs sa{plan, (const uint32_t*)c->s_msm_kv.p, cursor, (uint32_t*)c->s_msm_entries.p, (uint32_t)n};
         TRY((launch_msm_scatter<C>(sa, s)));
@@ -714,14 +738,23 @@ struct Impl {
         MsmReduceArgs ra{plan, (const uint32_t*)c->s_msm_buckets.p, (uint32_t*)c->s_rlc_pt.p};
         TRY((launch_msm_reduce<C>(ra, s)));
         PROF(c, 5, s);
+        RlcMsmFinishArgs f{c->view, plan, (const uint32_t*)c->s_rlc_pt.p, (const uint32_t*)c->s_rlc_sc.p, blocks, n_msgs,
+                           (uint8_t*)c->s_rlc_parts.p, pair, flags, status};
+        TRY((launch_rlc_msm_finish<C>(f, hdr, s)));
+        PROF(c, 6, s);
+        c->launches += (n ? 5 : 3);
+        return BBS_OK;
+    }
+    // shard -> comp(S1) || comp(S2) in c->s_rlc_parts (and the pairing record of the two sums in s_pair); *bad != 0 when an
+    // item was malformed
+    static int rlc_partial_dev(Ctx* c, size_t n, const uint8_t* sigs, const MsgIn& in, uint32_t n_msgs, const uint8_t* seed,
+                               uint64_t index_base, uint32_t* bad, rt_stream_t s) {
+        MsmPlan plan;
+        TRY(rlc_prep_dev(c, n, sigs, in, n_msgs, seed, index_base, RLC_PREP_VERDICT, nullptr, plan, s));
         TRY(c->s_pair.reserve(6 * C::Fp::N * 4));
         TRY(c->s_flags.reserve(4));
         TRY(c->s_status.reserve(1));
-        RlcMsmFinishArgs f{c->view, plan, (const uint32_t*)c->s_rlc_pt.p, (const uint32_t*)c->s_rlc_sc.p, blocks, n_msgs,
-                           (uint8_t*)c->s_rlc_parts.p, (uint32_t*)c->s_pair.p, (uint32_t*)c->s_flags.p, (uint8_t*)c->s_status.p};
-        TRY((launch_rlc_msm_finish<C>(f, s)));
-        PROF(c, 6, s);
-        c->launches += (n ? 5 : 3);
+        TRY(rlc_msm_dev(c, n, plan, n_msgs, false, (uint32_t*)c->s_pair.p, (uint32_t*)c->s_flags.p, (uint8_t*)c->s_status.p, s));
         TRY(rt_d2h(bad, c->s_rlc_bad.p, 4, s));
         return BBS_OK;
     }
@@ -748,6 +781,71 @@ struct Impl {
         TRY(finish_status(c, 1, verdict));             // synchronises: `bad` has arrived too
         if (bad) *verdict = ST_ERR_MALFORMED;
         return BBS_OK;
+    }
+    // Per-item statuses by one random linear combination (bbs_rlc_*verify_batch_status*; hdr_off != nullptr: a header per
+    // item).  The prep kernel decides the malformed items and leaves them out of the sums; if any item is left, ONE pairing
+    // checks the combination of all of them (its record, flag word and verdict in s_rlcp, apart from the items' arrays).
+    // If it holds, those items are accepted; if not, the per-item G1 half and pairing decide every item from the buffers
+    // already on the device.  Profiling slots: see include/bbs_b200.h.
+    static int rlc_verify_status(Ctx* c, size_t n, const uint8_t* sigs, const MsgIn& in, uint32_t n_msgs, const RlcProofIn& rlc,
+                                 uint8_t* status, const uint8_t* headers = nullptr, const uint64_t* hdr_off = nullptr) {
+        rt_stream_t s = c->stream;
+        uint8_t verdict = ST_ACCEPT;
+        if (n_msgs != c->L) {                                                // verify.rs:68-71, for every item
+            std::fill(status, status + n, (uint8_t)ST_ERR_MSG_GEN_LEN);
+            if (rlc.combined) *rlc.combined = verdict;
+            return BBS_OK;
+        }
+        constexpr size_t PW = 6 * C::Fp::N;
+        ItemKeyView item{};
+        if (hdr_off) TRY(item_keys(c, n, headers, hdr_off, item));
+        TRY(c->s_rlcp.reserve((PW + 2) * 4));                               // record | flags | status
+        MsmPlan plan;
+        TRY(rlc_prep_dev(c, n, sigs, in, n_msgs, rlc.seed, 0, hdr_off ? RLC_PREP_STATUS_HDR : RLC_PREP_STATUS,
+                         hdr_off ? &item : nullptr, plan, s));
+        uint32_t live = 0;
+        TRY(rt_d2h(&live, c->s_rlc_bad.p, 4, s));
+        TRY(rt_sync(s));
+        if (live) {                                                          // else every status is final already
+            uint32_t* pair = (uint32_t*)c->s_rlcp.p;
+            uint8_t* verdict_d = (uint8_t*)(pair + PW + 1);
+            TRY(rlc_msm_dev(c, n, plan, n_msgs, hdr_off != nullptr, pair, pair + PW, verdict_d, s));
+            TRY(pairing_dev(c, 1, verdict_d, s, nullptr, pair, pair + PW));
+            TRY(rt_d2h(&verdict, verdict_d, 1, s));
+            TRY(rt_sync(s));
+            PROF(c, 7, s);
+            if (verdict == ST_ACCEPT) {
+                TRY((launch_rlc_proof_accept<C>((const uint32_t*)c->s_flags.p, (uint8_t*)c->s_status.p, (uint32_t)n, s)));
+                c->launches += 1;
+                PROF(c, 8, s);
+            } else {
+                TRY(rlc_status_fallback(c, n, n_msgs, hdr_off ? &item : nullptr, s));
+            }
+            PROF(c, 9, s);
+        }
+        TRY(finish_status(c, n, status));
+        if (hdr_off) c->prof.xslot = 9;
+        if (rlc.combined) *rlc.combined = verdict;
+        return BBS_OK;
+    }
+    // the per-item path over the signatures and scalars that rlc_prep_dev left in s_sigs / s_scalars: the G1 half in the
+    // chunks of verify_chunked (its scratch reserved for the largest first), then one pairing launch
+    static int rlc_status_fallback(Ctx* c, size_t n, uint32_t n_msgs, const ItemKeyView* item, rt_stream_t s) {
+        size_t bounds[9];
+        const int n_chunks = plan_chunks(n, VERIFY_CHUNK, true, bounds);
+        size_t largest = 0;
+        for (int k = 0; k < n_chunks; k++) largest = std::max(largest, bounds[k + 1] - bounds[k]);
+        TRY(c->s_pair.reserve(n * 6 * C::Fp::N * 4));
+        if (largest <= c->split_max) {
+            TRY(c->s_g1v.reserve(largest * 3 * C::Fp::N * 4));
+            TRY(c->s_g1f.reserve(largest * 3 * C::Fp::N * 4));
+            TRY(c->s_g1st.reserve(2 * largest));
+        }
+        for (int k = 0; k < n_chunks; k++)
+            TRY(verify_g1_dev(c, bounds[k + 1] - bounds[k], bounds[k], (const uint8_t*)c->s_sigs.p, (const uint8_t*)c->s_scalars.p,
+                              n_msgs, (uint8_t*)c->s_status.p, s, nullptr, item));
+        PROF(c, 8, s);
+        return pairing_dev(c, n, (uint8_t*)c->s_status.p, s);
     }
     // n_parts x (comp(S1) || comp(S2)) -> one verdict byte
     static int rlc_combine(Ctx* c, size_t n_parts, const uint8_t* parts, uint8_t* verdict) {
@@ -816,7 +914,7 @@ struct Impl {
             // zero, so it yields S1 and S2 as they are
             RlcMsmFinishArgs f{c->view, plan, (const uint32_t*)c->s_rlc_pt.p, nullptr, 0u, 0u, (uint8_t*)c->s_rlc_parts.p,
                                pair, pair + PW, verdict_d};
-            TRY((launch_rlc_msm_finish<C>(f, s)));
+            TRY((launch_rlc_msm_finish<C>(f, false, s)));
             c->launches += 5;
             PROF(c, 7, s);
             TRY(pairing_dev(c, 1, verdict_d, s, nullptr, pair, pair + PW));
@@ -1544,6 +1642,44 @@ int bbs_rlc_proof_verify_batch_hdr(bbs_ctx* p, size_t n, const uint8_t* proofs, 
     DISPATCH(c, proof_verify(c, n, proofs, commit, commit_off, idx, MsgIn{nullptr, dis_msgs, dis_msg_off}, dis_off, phs, 0, status,
                              nullptr, nullptr, ph_off, headers, hdr_off, &rlc));
 }
+// signature verification with per-item statuses by one random linear combination: the arguments of the call without
+// rlc_ and _status, then the seed and the combined check's verdict, as the proof calls above
+int bbs_rlc_core_verify_batch_status(bbs_ctx* p, size_t n, const uint8_t* sigs, const uint8_t* scalars, uint32_t n_msgs,
+                                     const uint8_t* seed, uint8_t* status, uint8_t* combined) {
+    Ctx* c = as_ctx(p);
+    if (n && (!sigs || !status || (n_msgs && !scalars))) return arg_error("null");
+    CHECK_COUNTS(n, n_msgs);
+    RLC_PROOF_ARGS(seed, combined);
+    DISPATCH(c, rlc_verify_status(c, n, sigs, MsgIn{scalars, nullptr, nullptr}, n_msgs, rlc, status));
+}
+int bbs_rlc_verify_batch_status(bbs_ctx* p, size_t n, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* off,
+                                uint32_t n_msgs, const uint8_t* seed, uint8_t* status, uint8_t* combined) {
+    Ctx* c = as_ctx(p);
+    if (n && (!sigs || !status || !off)) return arg_error("null");
+    CHECK_COUNTS(n, n_msgs);
+    RLC_PROOF_ARGS(seed, combined);
+    DISPATCH(c, rlc_verify_status(c, n, sigs, MsgIn{nullptr, msgs, off}, n_msgs, rlc, status));
+}
+int bbs_rlc_core_verify_batch_status_hdr(bbs_ctx* p, size_t n, const uint8_t* sigs, const uint8_t* scalars, uint32_t n_msgs,
+                                         const uint8_t* headers, const uint64_t* hdr_off, const uint8_t* seed, uint8_t* status,
+                                         uint8_t* combined) {
+    Ctx* c = as_ctx(p);
+    if (n && (!sigs || !status || (n_msgs && !scalars))) return arg_error("null");
+    CHECK_COUNTS(n, n_msgs);
+    if (n) TRY(check_hdr_args(c, n, headers, hdr_off, true));
+    RLC_PROOF_ARGS(seed, combined);
+    DISPATCH(c, rlc_verify_status(c, n, sigs, MsgIn{scalars, nullptr, nullptr}, n_msgs, rlc, status, headers, hdr_off));
+}
+int bbs_rlc_verify_batch_status_hdr(bbs_ctx* p, size_t n, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* off,
+                                    uint32_t n_msgs, const uint8_t* headers, const uint64_t* hdr_off, const uint8_t* seed,
+                                    uint8_t* status, uint8_t* combined) {
+    Ctx* c = as_ctx(p);
+    if (n && (!sigs || !status || !off)) return arg_error("null");
+    CHECK_COUNTS(n, n_msgs);
+    if (n) TRY(check_hdr_args(c, n, headers, hdr_off, true));
+    RLC_PROOF_ARGS(seed, combined);
+    DISPATCH(c, rlc_verify_status(c, n, sigs, MsgIn{nullptr, msgs, off}, n_msgs, rlc, status, headers, hdr_off));
+}
 #else
 int bbs_rlc_partial_core(bbs_ctx*, size_t, const uint8_t*, const uint8_t*, uint32_t, const uint8_t*, uint64_t, uint8_t*, uint8_t*) { rt_set_error("rlc", "needs the CUDA build"); return BBS_E_CUDA; }
 int bbs_rlc_partial(bbs_ctx*, size_t, const uint8_t*, const uint8_t*, const uint64_t*, uint32_t, const uint8_t*, uint64_t, uint8_t*, uint8_t*) { rt_set_error("rlc", "needs the CUDA build"); return BBS_E_CUDA; }
@@ -1554,6 +1690,10 @@ int bbs_rlc_core_proof_verify_batch(bbs_ctx*, size_t, const uint8_t*, const uint
 int bbs_rlc_proof_verify_batch(bbs_ctx*, size_t, const uint8_t*, const uint8_t*, const uint64_t*, const uint32_t*, const uint8_t*, const uint64_t*, const uint64_t*, const uint8_t*, size_t, const uint8_t*, uint8_t*, uint8_t*) { rt_set_error("rlc", "needs the CUDA build"); return BBS_E_CUDA; }
 int bbs_rlc_core_proof_verify_batch_hdr(bbs_ctx*, size_t, const uint8_t*, const uint8_t*, const uint64_t*, const uint32_t*, const uint8_t*, const uint64_t*, const uint8_t*, const uint64_t*, const uint8_t*, const uint64_t*, const uint8_t*, uint8_t*, uint8_t*) { rt_set_error("rlc", "needs the CUDA build"); return BBS_E_CUDA; }
 int bbs_rlc_proof_verify_batch_hdr(bbs_ctx*, size_t, const uint8_t*, const uint8_t*, const uint64_t*, const uint32_t*, const uint8_t*, const uint64_t*, const uint64_t*, const uint8_t*, const uint64_t*, const uint8_t*, const uint64_t*, const uint8_t*, uint8_t*, uint8_t*) { rt_set_error("rlc", "needs the CUDA build"); return BBS_E_CUDA; }
+int bbs_rlc_core_verify_batch_status(bbs_ctx*, size_t, const uint8_t*, const uint8_t*, uint32_t, const uint8_t*, uint8_t*, uint8_t*) { rt_set_error("rlc", "needs the CUDA build"); return BBS_E_CUDA; }
+int bbs_rlc_verify_batch_status(bbs_ctx*, size_t, const uint8_t*, const uint8_t*, const uint64_t*, uint32_t, const uint8_t*, uint8_t*, uint8_t*) { rt_set_error("rlc", "needs the CUDA build"); return BBS_E_CUDA; }
+int bbs_rlc_core_verify_batch_status_hdr(bbs_ctx*, size_t, const uint8_t*, const uint8_t*, uint32_t, const uint8_t*, const uint64_t*, const uint8_t*, uint8_t*, uint8_t*) { rt_set_error("rlc", "needs the CUDA build"); return BBS_E_CUDA; }
+int bbs_rlc_verify_batch_status_hdr(bbs_ctx*, size_t, const uint8_t*, const uint8_t*, const uint64_t*, uint32_t, const uint8_t*, const uint64_t*, const uint8_t*, uint8_t*, uint8_t*) { rt_set_error("rlc", "needs the CUDA build"); return BBS_E_CUDA; }
 #endif
 
 int bbs_msg_to_scalars_dev(bbs_ctx* p, size_t count, const uint8_t* d_msgs, const uint64_t* d_off, uint8_t* d_out, void* stream) {

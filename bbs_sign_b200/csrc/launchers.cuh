@@ -27,12 +27,12 @@ template <class C> int launch_verify_g1(const VerifyG1Args& a, uint32_t n, rt_st
 template <class C> int launch_pairing(const PairingArgs& a, uint32_t n, rt_stream_t s);
 #ifndef BBS_HOSTSIM
 // random-linear-combination batch mode (rlc.cuh)
-template <class C> int launch_rlc_prep(const RlcPrepArgs& a, uint32_t n_blocks, rt_stream_t s);
+template <class C> int launch_rlc_prep(const RlcPrepArgs& a, uint32_t n_blocks, int mode, rt_stream_t s);   // mode: RLC_PREP_*
 int launch_msm_scan(const uint32_t* counts, uint32_t* offsets, uint32_t* cursor, uint32_t nb, rt_stream_t s);
 template <class C> int launch_msm_scatter(const MsmScatterArgs& a, rt_stream_t s);
 template <class C> int launch_msm_bucket(const MsmBucketArgs& a, rt_stream_t s);
 template <class C> int launch_msm_reduce(const MsmReduceArgs& a, rt_stream_t s);
-template <class C> int launch_rlc_msm_finish(const RlcMsmFinishArgs& a, rt_stream_t s);
+template <class C> int launch_rlc_msm_finish(const RlcMsmFinishArgs& a, bool hdr, rt_stream_t s);
 template <class C> int launch_rlc_combine(const RlcCombineArgs& a, rt_stream_t s);
 // the proof form of the mode: prep, buckets over the pairing records, acceptance of the undecided items
 template <class C> int launch_rlc_proof_prep(const RlcProofPrepArgs& a, rt_stream_t s);

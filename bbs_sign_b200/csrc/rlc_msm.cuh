@@ -41,9 +41,23 @@ struct RlcPrepArgs {
     uint32_t* pts;           // n x affine Montgomery
     uint32_t* kv;            // n x 3 x 4 words
     uint32_t* counts;        // rows << c, zeroed by the caller
+    // status modes (RLC_PREP_STATUS*) only:
+    uint8_t* status;         // n: ERR_MALFORMED for a malformed item, untouched otherwise
+    uint32_t* flags;         // n: FL_DONE for a malformed item, 0 otherwise
+    uint32_t* live;          // set to 1 when some item is well formed; zeroed by the caller
+    const uint32_t* domains; // RLC_PREP_STATUS_HDR: n x 8 words, the items' domains d_i (canonical limbs)
 };
-template <class C> __global__ void __launch_bounds__(RLC_TPB, 4) rlc_prep_kernel(const RlcPrepArgs pa) {
+// RLC_PREP_VERDICT: one verdict per batch (bbs_rlc_partial*, bbs_rlc_[core_]verify_batch); a malformed item sets `bad`.
+// RLC_PREP_STATUS: per-item statuses (bbs_rlc_[core_]verify_batch_status): an item is checked completely (A with its
+// subgroup test, e < r, every m_ij < r) before it contributes; a malformed one gets r_i = 0, so it adds nothing to any sum,
+// and its status is final (FL_DONE).  RLC_PREP_STATUS_HDR: also one header per item, with K_i = K + (d_i - d) Q1, so
+//     sum r_i B_i = (sum r_i) K + (sum r_i (d_i - d)) Q1 + sum_j (sum r_i m_ij) H_j
+// and the prep adds the Fr row sum r_i (d_i - d) after the message rows.
+enum : int { RLC_PREP_VERDICT = 0, RLC_PREP_STATUS = 1, RLC_PREP_STATUS_HDR = 2 };
+template <class C, int MODE = RLC_PREP_VERDICT> __global__ void __launch_bounds__(RLC_TPB, 4) rlc_prep_kernel(const RlcPrepArgs pa) {
     using Fr = typename C::Fr;
+    constexpr bool STATUS = MODE != RLC_PREP_VERDICT;
+    constexpr uint32_t HDR = MODE == RLC_PREP_STATUS_HDR ? 1u : 0u;
     __shared__ BBS_A16 uint32_t ss[RLC_TPB][8];
     const RlcArgs& a = pa.base;
     const uint32_t i = blockIdx.x * RLC_TPB + threadIdx.x;
@@ -59,8 +73,15 @@ template <class C> __global__ void __launch_bounds__(RLC_TPB, 4) rlc_prep_kernel
         for (int k = 0; k < 12; k++) kv[k] = 0;
         int st = g1_decompress<C>(A, sig);
         ok = st != PT_BAD && fr_from_le32<C>(e, sig + C::G1_BYTES);
-        rlc_coeff(r, a.seed, a.index_base + i);
-        fe_to_mont<Fr>(rm, r);
+        if (STATUS)
+            for (uint32_t j = 0; j < a.n_msgs && ok; j++) {
+                BBS_A16 uint32_t m[8];
+                ok = fr_from_le32<C>(m, sc + j * 32);
+            }
+        if (!STATUS || ok) {
+            rlc_coeff(r, a.seed, a.index_base + i);
+            fe_to_mont<Fr>(rm, r);
+        }
         if (ok && st == PT_OK) {
             BBS_A16 uint32_t ae[8];
             fe_mul<Fr>(ae, rm, e);                  // r_i e_i mod r, canonical
@@ -82,8 +103,8 @@ template <class C> __global__ void __launch_bounds__(RLC_TPB, 4) rlc_prep_kernel
                 }
         }
     }
-    // scalars: sum r_i, sum r_i m_ij
-    uint32_t* scp = a.sc_part + (size_t)blockIdx.x * (a.n_msgs + 1) * 8;
+    // scalars: sum r_i, sum r_i m_ij (, sum r_i (d_i - d))
+    uint32_t* scp = a.sc_part + (size_t)blockIdx.x * (a.n_msgs + 1 + HDR) * 8;
     rlc_block_sum_fr<C>(ss, r);
     if (threadIdx.x == 0) bn_copy<8>(scp, ss[0]);
     __syncthreads();
@@ -98,7 +119,26 @@ template <class C> __global__ void __launch_bounds__(RLC_TPB, 4) rlc_prep_kernel
         if (threadIdx.x == 0) bn_copy<8>(scp + (j + 1) * 8, ss[0]);
         __syncthreads();
     }
-    if (valid && !ok) atomicOr(a.bad, 1u);
+    if (HDR) {
+        BBS_A16 uint32_t t[8];
+        bn_zero<8>(t);
+        if (valid && ok) {
+            BBS_A16 uint32_t dd[8];
+            fe_sub<Fr>(dd, pa.domains + (size_t)i * 8, a.ctx.domain);
+            fe_mul<Fr>(t, rm, dd);
+        }
+        rlc_block_sum_fr<C>(ss, t);
+        if (threadIdx.x == 0) bn_copy<8>(scp + (a.n_msgs + 1) * 8, ss[0]);
+    }
+    if (STATUS) {
+        if (valid) {
+            pa.flags[i] = ok ? 0u : (uint32_t)FL_DONE;
+            if (!ok) pa.status[i] = ST_ERR_MALFORMED;
+        }
+        if (__ballot_sync(0xffffffffu, valid && ok) && (threadIdx.x & 31) == 0) atomicOr(pa.live, 1u);
+    } else if (valid && !ok) {
+        atomicOr(a.bad, 1u);
+    }
 }
 
 constexpr int MSM_SCAN_TPB = 1024;
@@ -229,22 +269,25 @@ struct RlcMsmFinishArgs {
 // the fixed-base term F = (sum r_i) K + sum_j (sum_i r_i m_ij) H_j, one generator per lane; then S2 = S2' - F, and the two
 // points are normalised in two warps: compressed for the host-combined multi-GPU path (rlc_combine) and written as the
 // pairing record (x, y, 1) that the single-shard verdict feeds straight to the pairing kernel.
-template <class C> __global__ void __launch_bounds__(RLC_TPB, 1) rlc_msm_finish_kernel(const RlcMsmFinishArgs a) {
+// HDR (per-item headers, RLC_PREP_STATUS_HDR): the prep blocks' rows end with sum r_i (d_i - d), and F gains that multiple
+// of Q1, whose window table is slot L + 1 of a per-item-header context (n_msgs == L).
+template <class C, bool HDR = false> __global__ void __launch_bounds__(RLC_TPB, 1) rlc_msm_finish_kernel(const RlcMsmFinishArgs a) {
     using Fr = typename C::Fr;
     using F = typename C::Fp;
+    constexpr uint32_t X = HDR ? 1u : 0u;
     __shared__ BBS_A16 uint32_t sp[RLC_TPB][3 * C::Fp::N];
     __shared__ BBS_A16 uint32_t ss[RLC_TPB][8];
-    __shared__ BBS_A16 uint32_t sums[MAX_L + 1][8];
+    __shared__ BBS_A16 uint32_t sums[MAX_L + 1 + X][8];
     __shared__ BBS_A16 uint32_t res[3][3 * C::Fp::N];        // S1, S2', F
     __shared__ BBS_A16 uint32_t sf[32][3 * C::Fp::N];        // warp 3: partial sums of F
     __shared__ uint32_t skip[2];
     const CtxView& cx = a.ctx;
     const uint32_t t = threadIdx.x, W = a.plan.W, rows = a.plan.rows;
     // Fr sums over the prep blocks
-    for (uint32_t j = 0; j <= a.n_msgs; j++) {
+    for (uint32_t j = 0; j <= a.n_msgs + X; j++) {
         BBS_A16 uint32_t v[8];
         bn_zero<8>(v);
-        for (uint32_t b = t; b < a.n_blocks; b += RLC_TPB) fe_add<Fr>(v, v, a.sc_part + ((size_t)b * (a.n_msgs + 1) + j) * 8);
+        for (uint32_t b = t; b < a.n_blocks; b += RLC_TPB) fe_add<Fr>(v, v, a.sc_part + ((size_t)b * (a.n_msgs + 1 + X) + j) * 8);
         rlc_block_sum_fr<C>(ss, v);
         if (t == 0) bn_copy<8>(sums[j], ss[0]);
         __syncthreads();
@@ -275,7 +318,7 @@ template <class C> __global__ void __launch_bounds__(RLC_TPB, 1) rlc_msm_finish_
             g1_copy<C>(res[job], acc);
         }
     } else if (job == 3) {
-        for (uint32_t j = lane; j <= a.n_msgs; j += 32)
+        for (uint32_t j = lane; j <= a.n_msgs + X; j += 32)
             if (!(j == 0 && cx.k_inf)) tab_accumulate<C>(acc, cx, j, sums[j]);
         g1_copy<C>(sf[lane], acc);                           // warp 3 only
         __syncwarp();

@@ -4,9 +4,11 @@
 #ifndef BBS_HOSTSIM
 namespace bbs {
 
-template <class C> int launch_rlc_prep(const RlcPrepArgs& a, uint32_t n_blocks, rt_stream_t s) {
+template <class C> int launch_rlc_prep(const RlcPrepArgs& a, uint32_t n_blocks, int mode, rt_stream_t s) {
     if (n_blocks == 0) return 0;
-    rlc_prep_kernel<C><<<n_blocks, RLC_TPB, 0, s>>>(a);
+    if (mode == RLC_PREP_STATUS_HDR) rlc_prep_kernel<C, RLC_PREP_STATUS_HDR><<<n_blocks, RLC_TPB, 0, s>>>(a);
+    else if (mode == RLC_PREP_STATUS) rlc_prep_kernel<C, RLC_PREP_STATUS><<<n_blocks, RLC_TPB, 0, s>>>(a);
+    else rlc_prep_kernel<C><<<n_blocks, RLC_TPB, 0, s>>>(a);
     RT_CHECK(cudaGetLastError());
     return 0;
 }
@@ -54,8 +56,9 @@ template <class C> int launch_msm_reduce(const MsmReduceArgs& a, rt_stream_t s) 
     RT_CHECK(cudaGetLastError());
     return 0;
 }
-template <class C> int launch_rlc_msm_finish(const RlcMsmFinishArgs& a, rt_stream_t s) {
-    rlc_msm_finish_kernel<C><<<1, RLC_TPB, 0, s>>>(a);
+template <class C> int launch_rlc_msm_finish(const RlcMsmFinishArgs& a, bool hdr, rt_stream_t s) {
+    if (hdr) rlc_msm_finish_kernel<C, true><<<1, RLC_TPB, 0, s>>>(a);
+    else rlc_msm_finish_kernel<C><<<1, RLC_TPB, 0, s>>>(a);
     RT_CHECK(cudaGetLastError());
     return 0;
 }
@@ -78,22 +81,22 @@ template <class C> int launch_rlc_proof_accept(const uint32_t* flags, uint8_t* s
 }
 
 #if defined(BBS_TU_BLS) || !defined(BBS_TU_BN)
-template int launch_rlc_prep<Bls>(const RlcPrepArgs&, uint32_t, rt_stream_t);
+template int launch_rlc_prep<Bls>(const RlcPrepArgs&, uint32_t, int, rt_stream_t);
 template int launch_msm_scatter<Bls>(const MsmScatterArgs&, rt_stream_t);
 template int launch_msm_bucket<Bls>(const MsmBucketArgs&, rt_stream_t);
 template int launch_msm_reduce<Bls>(const MsmReduceArgs&, rt_stream_t);
-template int launch_rlc_msm_finish<Bls>(const RlcMsmFinishArgs&, rt_stream_t);
+template int launch_rlc_msm_finish<Bls>(const RlcMsmFinishArgs&, bool, rt_stream_t);
 template int launch_rlc_combine<Bls>(const RlcCombineArgs&, rt_stream_t);
 template int launch_msm_bucket_pair<Bls>(const MsmBucketArgs&, rt_stream_t);
 template int launch_rlc_proof_prep<Bls>(const RlcProofPrepArgs&, rt_stream_t);
 template int launch_rlc_proof_accept<Bls>(const uint32_t*, uint8_t*, uint32_t, rt_stream_t);
 #endif
 #if defined(BBS_TU_BN) || !defined(BBS_TU_BLS)
-template int launch_rlc_prep<Bn>(const RlcPrepArgs&, uint32_t, rt_stream_t);
+template int launch_rlc_prep<Bn>(const RlcPrepArgs&, uint32_t, int, rt_stream_t);
 template int launch_msm_scatter<Bn>(const MsmScatterArgs&, rt_stream_t);
 template int launch_msm_bucket<Bn>(const MsmBucketArgs&, rt_stream_t);
 template int launch_msm_reduce<Bn>(const MsmReduceArgs&, rt_stream_t);
-template int launch_rlc_msm_finish<Bn>(const RlcMsmFinishArgs&, rt_stream_t);
+template int launch_rlc_msm_finish<Bn>(const RlcMsmFinishArgs&, bool, rt_stream_t);
 template int launch_rlc_combine<Bn>(const RlcCombineArgs&, rt_stream_t);
 template int launch_msm_bucket_pair<Bn>(const MsmBucketArgs&, rt_stream_t);
 template int launch_rlc_proof_prep<Bn>(const RlcProofPrepArgs&, rt_stream_t);

@@ -104,6 +104,25 @@ class ShardedVerifier:
         self._run_sharded(n, work)
         return out, (1 if all(c == 1 for c in combined) else 0)
 
+    def rlc_verify_batch_status(self, signatures, messages: Sequence[Sequence[bytes]], *,
+                                headers: Optional[Sequence[bytes]] = None):
+        """`BatchContext.rlc_verify_batch_status` split by signature index: every GPU checks its slice with one combined
+        pairing under its own library-drawn seed, so nothing is exchanged.  Returns (status, combined); `combined` is
+        ST_ACCEPT only if every shard's was."""
+        sigs = np.frombuffer(b"".join(signatures) if isinstance(signatures, (list, tuple)) else signatures, dtype=np.uint8) \
+            if not isinstance(signatures, np.ndarray) else signatures.reshape(-1)
+        sb = self.suite.signature_bytes
+        n = sigs.size // sb
+        out = np.full(n, 255, dtype=np.uint8)
+        combined = [1] * len(self.ctxs)
+
+        def work(ctx, g, lo, hi):
+            out[lo:hi], combined[g] = ctx.rlc_verify_batch_status(sigs[lo * sb: hi * sb], messages[lo:hi],
+                                                                  headers=None if headers is None else headers[lo:hi])
+
+        self._run_sharded(n, work)
+        return out, (1 if all(c == 1 for c in combined) else 0)
+
     def rlc_verify_batch(self, signatures: Sequence[bytes], messages: Sequence[Sequence[bytes]],
                          seed: Optional[bytes] = None) -> int:
         """Random-linear-combination verdict for the whole batch: every GPU reduces its slice to two compressed G1

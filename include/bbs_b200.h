@@ -332,6 +332,39 @@ int bbs_rlc_proof_verify_batch_hdr(bbs_ctx* ctx, size_t n, const uint8_t* proofs
                                    const uint64_t* hdr_off, const uint8_t* phs, const uint64_t* ph_off,
                                    const uint8_t* seed32_or_null, uint8_t* status, uint8_t* combined);
 
+/* Signature verification with per-item statuses by one random linear combination.  Arguments as
+ * bbs_[core_]verify_batch and bbs_[core_]verify_batch_hdr, plus:
+ *   seed32_or_null : the coefficient seed; r_i = the first 16 bytes, as a big-endian integer, of SHA-256(seed || BE64(i))
+ *                    (1 if that is 0), i = the item's position in the call.  NULL: the library draws 32 bytes from the OS
+ *                    CSPRNG after it has received the batch.
+ *   status[i]      : what bbs_[core_]verify_batch[_hdr] returns for item i.  An ACCEPT holds except with probability
+ *                    2^-128 over the seed; every other status is exact.
+ *   combined       : (may be NULL) ACCEPT when the one combined check held, or when no item reached it; REJECT when it
+ *                    failed and the per-item path decided every item instead.
+ * Every item is first checked for malformed input (A decodes and lies in the subgroup, e < r, every message scalar < r):
+ * a malformed item gets ERR_MALFORMED and stays out of the sums.  The others are checked at once by
+ *     e( sum r_i A_i , W ) * e( sum r_i (e_i A_i - B_i) , BP2 ) == 1
+ * two bucket MSMs and one pairing for the batch, as bbs_rlc_[core_]verify_batch.  If that fails, the per-item G1 half and
+ * pairing of bbs_verify_batch decide every item from the buffers already on the GPU, so the statuses stay exact at about
+ * the cost of the per-item call plus the combined check; `combined` tells a caller that this happened.  n_msgs != L gives
+ * ERR_MSG_GEN_LEN for every item and launches nothing.  The _hdr forms take one header per item (headers[hdr_off[i] ..
+ * hdr_off[i+1]), checked as in bbs_verify_batch_hdr) and need a context created with BBS_CTX_PER_ITEM_HEADER; with domain_i
+ * of item i and d of the context, K_i = K + (domain_i - d) Q1 and one more fixed-base term enters the sum.
+ * THE SEED MUST BE UNPREDICTABLE TO WHOEVER SUBMITS THE BATCH.  With a known seed, two items whose message scalars are
+ * shifted by +r_1 and -r_0 (r_0, r_1 the coefficients of their positions, the same H_j) cancel in the sum, and both are
+ * accepted although neither verifies.  Pass NULL; an explicit seed is for reproducible tests.  One issuer key per call
+ * (no issuer sets).  n must be below 2^31. */
+int bbs_rlc_core_verify_batch_status(bbs_ctx* ctx, size_t n, const uint8_t* sigs, const uint8_t* msg_scalars, uint32_t n_msgs,
+                                     const uint8_t* seed32_or_null, uint8_t* status, uint8_t* combined);
+int bbs_rlc_verify_batch_status(bbs_ctx* ctx, size_t n, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* offsets,
+                                uint32_t n_msgs, const uint8_t* seed32_or_null, uint8_t* status, uint8_t* combined);
+int bbs_rlc_core_verify_batch_status_hdr(bbs_ctx* ctx, size_t n, const uint8_t* sigs, const uint8_t* msg_scalars,
+                                         uint32_t n_msgs, const uint8_t* headers, const uint64_t* hdr_off,
+                                         const uint8_t* seed32_or_null, uint8_t* status, uint8_t* combined);
+int bbs_rlc_verify_batch_status_hdr(bbs_ctx* ctx, size_t n, const uint8_t* sigs, const uint8_t* msgs, const uint64_t* offsets,
+                                    uint32_t n_msgs, const uint8_t* headers, const uint64_t* hdr_off,
+                                    const uint8_t* seed32_or_null, uint8_t* status, uint8_t* combined);
+
 /* ---- device-buffer entry points (no copies; all pointers are device pointers on the context's GPU;
  *      work is enqueued on `stream` (a cudaStream_t, NULL = default stream) and NOT synchronized) ------ */
 int bbs_msg_to_scalars_dev(bbs_ctx* ctx, size_t count, const uint8_t* d_msgs, const uint64_t* d_offsets,
@@ -387,6 +420,11 @@ int bbs_ctx_set_pairing_split(bbs_ctx* ctx, size_t max_items);
  * bbs_rlc_*proof_verify_batch*: [msg_to_scalars, G1 kernels, prep, scan + scatter, buckets, reduction, finish, combined
  *   pairing, acceptance or per-item pairing]; the scan slot and the combined-pairing slot also hold the host's read of one
  *   word (whether any item reached the pairing; the verdict).  Slots 3..8 are 0 when no item reached the pairing;
+ *   per-item headers: slot 9.
+ * bbs_rlc_*verify_batch_status*: [first chunk's upload wait and msg_to_scalars, the other chunks' msg_to_scalars and the
+ *   prep kernels, scan + scatter, buckets, reduction, finish, combined pairing, acceptance or per-item G1 half, per-item
+ *   pairing]; the scan slot and the combined-pairing slot also hold the host's read of one word (whether any item is well
+ *   formed; the verdict).  Slots 2..8 are 0 when no item is well formed, slot 8 is 0 when the combined check held;
  *   per-item headers: slot 9. */
 int bbs_ctx_set_profiling(bbs_ctx* ctx, int on);
 int bbs_ctx_kernel_times(bbs_ctx* ctx, float* ms, int n);

@@ -142,6 +142,16 @@ extern "C" {
                                       commit_off: *const u64, disclosed_idx: *const u32, dis_msgs: *const u8, dis_msg_off: *const u64,
                                       dis_off: *const u64, headers: *const u8, hdr_off: *const u64, phs: *const u8,
                                       ph_off: *const u64, seed32_or_null: *const u8, status: *mut u8, combined: *mut u8) -> i32;
+    fn bbs_rlc_core_verify_batch_status(ctx: *mut BbsCtx, n: usize, sigs: *const u8, msg_scalars: *const u8, n_msgs: u32,
+                                        seed32_or_null: *const u8, status: *mut u8, combined: *mut u8) -> i32;
+    fn bbs_rlc_verify_batch_status(ctx: *mut BbsCtx, n: usize, sigs: *const u8, msgs: *const u8, offsets: *const u64, n_msgs: u32,
+                                   seed32_or_null: *const u8, status: *mut u8, combined: *mut u8) -> i32;
+    fn bbs_rlc_core_verify_batch_status_hdr(ctx: *mut BbsCtx, n: usize, sigs: *const u8, msg_scalars: *const u8, n_msgs: u32,
+                                            headers: *const u8, hdr_off: *const u64, seed32_or_null: *const u8, status: *mut u8,
+                                            combined: *mut u8) -> i32;
+    fn bbs_rlc_verify_batch_status_hdr(ctx: *mut BbsCtx, n: usize, sigs: *const u8, msgs: *const u8, offsets: *const u64,
+                                       n_msgs: u32, headers: *const u8, hdr_off: *const u64, seed32_or_null: *const u8,
+                                       status: *mut u8, combined: *mut u8) -> i32;
     fn bbs_msg_to_scalars_dev(ctx: *mut BbsCtx, count: usize, d_msgs: *const u8, d_offsets: *const u64, d_out: *mut u8,
                               stream: *mut c_void) -> i32;
     fn bbs_core_verify_batch_dev(ctx: *mut BbsCtx, n: usize, d_sigs: *const u8, d_msg_scalars: *const u8, n_msgs: u32,
@@ -779,6 +789,48 @@ pub fn rlc_verify_batch<E: Pairing, F: Field>(ctx: &BatchCtx, sigs: &[Signature<
     Ok(signature_status(verdict))
 }
 
+/// `verify_batch_with` with the pairings checked by one random linear combination (`bbs_rlc_verify_batch_status`, not
+/// in the reference): the same per-item results, where an accepted signature holds except with probability 2^-128 over
+/// the coefficient seed, which the library draws from the OS CSPRNG after it has received the batch.  When the combined
+/// check fails, the library decides every item with the per-item path, so the results stay exact.
+pub fn rlc_verify_batch_items<E: Pairing, F: Field>(ctx: &BatchCtx, sigs: &[Signature<E, F>], messages: &[&[&[u8]]])
+    -> Result<Vec<Result<bool, ItemError<SignatureError>>>, BatchError> {
+    rlc_verify_status(ctx, sigs, None, messages)
+}
+
+/// `verify_batch_per_header` by one random linear combination, as `rlc_verify_batch_items`; `ctx` comes from
+/// `PublicKey::batch_ctx_per_item_header`.
+pub fn rlc_verify_batch_per_header<E: Pairing, F: Field>(ctx: &BatchCtx, sigs: &[Signature<E, F>], headers: &[&[u8]],
+    messages: &[&[&[u8]]]) -> Result<Vec<Result<bool, ItemError<SignatureError>>>, BatchError> {
+    rlc_verify_status(ctx, sigs, Some(headers), messages)
+}
+
+fn rlc_verify_status<E: Pairing, F: Field>(ctx: &BatchCtx, sigs: &[Signature<E, F>], headers: Option<&[&[u8]]>,
+    messages: &[&[&[u8]]]) -> Result<Vec<Result<bool, ItemError<SignatureError>>>, BatchError> {
+    assert_eq!(sigs.len(), messages.len(), "one message list per signature");
+    assert!(headers.map_or(true, |h| h.len() == sigs.len()), "one header per signature");
+    let l = uniform_len(messages)?;
+    let mut sb = Vec::new();
+    for s in sigs {
+        ser(s, &mut sb);
+    }
+    let (flat, offs) = pack(messages);
+    let mut st = vec![0u8; sigs.len()];
+    let mut combined = 0u8;
+    check(unsafe {
+        match headers {
+            Some(h) => {
+                let (hdr, hoff) = pack_items(h);
+                bbs_rlc_verify_batch_status_hdr(ctx.raw, sigs.len(), sb.as_ptr(), flat.as_ptr(), offs.as_ptr(), l as u32, hdr.as_ptr(),
+                                                hoff.as_ptr(), std::ptr::null(), st.as_mut_ptr(), &mut combined)
+            }
+            None => bbs_rlc_verify_batch_status(ctx.raw, sigs.len(), sb.as_ptr(), flat.as_ptr(), offs.as_ptr(), l as u32,
+                                                std::ptr::null(), st.as_mut_ptr(), &mut combined),
+        }
+    })?;
+    Ok(st.into_iter().map(signature_status).collect())
+}
+
 /// Refuses anything but the CUDA build of the library (the host simulation the engine's tests build from the same
 /// sources must never be linked into a product).
 pub fn assert_cuda_build() {
@@ -802,6 +854,7 @@ fn _unused_bindings() {
         bbs_core_verify_batch_hdr as usize, bbs_core_sign_batch_hdr as usize, bbs_core_proof_verify_batch_hdr as usize,
         bbs_core_proof_gen_batch_hdr as usize, bbs_proof_gen_batch_hdr as usize, bbs_core_verify_batch_hdr_dev as usize,
         bbs_core_proof_verify_batch_hdr_dev as usize, bbs_rlc_core_proof_verify_batch as usize,
-        bbs_rlc_core_proof_verify_batch_hdr as usize,
+        bbs_rlc_core_proof_verify_batch_hdr as usize, bbs_rlc_core_verify_batch_status as usize,
+        bbs_rlc_core_verify_batch_status_hdr as usize,
     );
 }
